@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path
+    python bench.py ... --dump-outputs DIR     # + the rows of the last timed step as DIR/*.npy
 
 Workload at N=1 = BASELINE.json configs[1] ("c2"): E. coli-sized 4.6 Mbp synthetic reference,
 20 000 simulated reads (R9.4 6-mer model, noise 1.0), full-read mapping (every chunk of every
@@ -61,7 +62,7 @@ def parse_args():
                     help="--impl reference: reads per step (0 = max(50 x host cores, min(1500, 20000 / steps)))")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config3", action="store_true", help="N=1: skip the config 3 leg")
-    ap.add_argument("--c3-steps", type=int, default=2)
+    ap.add_argument("--c3-steps", type=int, default=None, help="N=1: timed steps of the config 3 leg (default: --steps)")
     ap.add_argument("--channels", type=int, default=512, help="read-until leg: concurrent channels")
     ap.add_argument("--stream-rounds", type=int, default=24, help="read-until leg: timed rounds (0 = skip)")
     ap.add_argument("--shard", default="reads", choices=["reads", "contigs"],
@@ -69,7 +70,12 @@ def parse_args():
                          "(default, weak scaling); contigs = the index is partitioned by contig, every "
                          "rank maps every read, NCCL merges the chains (SURVEY 8e mode 2, strong scaling)")
     ap.add_argument("--seed", type=int, default=20251017)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rows the last timed step returned as DIR/<field>.npy (config 3 leg: "
+                         "DIR/config3_<field>.npy), rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1 or (args.c3_steps is not None and args.c3_steps < 1):
+        ap.error("--steps and --c3-steps must be at least 1")
     return resolve_workload(args, int(os.environ.get("WORLD_SIZE", "1")))
 
 
@@ -380,6 +386,31 @@ def stream_latency(mapper, reads, n_channels, rounds, warm=3):
             "timed": "smb_stream_round call, host buffers in -> decisions out (host clock)"}
 
 
+# ------------------------------------------------------------------ output dump
+DUMP_BYTES_PER_LEG = 32 << 20   # two legs at N=1: at most 64 MB in all
+
+
+def dump_rows(rows, directory, prefix, seed):
+    """The smb_mapping rows of a mapping call, one DIR/<prefix><field>.npy per field (float32 for
+    the float fields, float64 for the integer ones: exact) and <prefix>read_index.npy, the read
+    each row belongs to.  Above DUMP_BYTES_PER_LEG a fixed sample of the rows, drawn from --seed."""
+    import ctypes as C
+    from sigmap_b200 import _ffi as F
+    fields = [(n, t is C.c_float) for n, t in F.Mapping._fields_]
+    dt = np.dtype([(n, "<f4" if flt else "<u4") for n, flt in fields])
+    assert dt.itemsize == C.sizeof(F.Mapping)
+    n = len(rows)
+    row_bytes = 8 + sum(4 if flt else 8 for _, flt in fields)
+    keep = np.arange(n)
+    if n * row_bytes > DUMP_BYTES_PER_LEG:
+        keep = np.sort(np.random.default_rng(seed).choice(n, DUMP_BYTES_PER_LEG // row_bytes, replace=False))
+    a = np.frombuffer(b"".join(bytes(rows[int(i)]) for i in keep), dt)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, prefix + "read_index.npy"), keep.astype(np.float64))
+    for name, flt in fields:
+        np.save(os.path.join(directory, prefix + name + ".npy"), a[name].astype(np.float32 if flt else np.float64))
+
+
 # ------------------------------------------------------------------ our arm
 def measure(args, rank, world, local, dist, light=False):
     """One workload on this rank's GPU: device-resident leg, end-to-end leg, (read-until leg),
@@ -388,7 +419,7 @@ def measure(args, rank, world, local, dist, light=False):
     import torch
     from sigmap_b200.mapper import Mapper, default_params, full_read_params
 
-    steps = args.c3_steps if light else args.steps
+    steps = (args.c3_steps or args.steps) if light else args.steps
     warmup = min(args.warmup, 1) if light else args.warmup
     t_setup = time.time()
     by_contig = args.shard == "contigs" and world > 1
@@ -568,6 +599,8 @@ def measure(args, rank, world, local, dist, light=False):
         if world == 1:
             out["cpu_baseline"] = cpu
         out["concordance"] = conc
+    if rank == 0 and args.dump_outputs:
+        dump_rows(rows, args.dump_outputs, "config3_" if light else "", args.seed)
     mapper.close()
     del pinned
     return out

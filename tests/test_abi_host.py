@@ -36,11 +36,11 @@ def test_every_declared_symbol_is_exported_and_bound():
         ["ldd", _ffi.LIB_PATH], capture_output=True, text=True).stdout
 
 
-def test_struct_sizes_match_header():
+def test_struct_sizes_match_header(tmp_path):
     from sigmap_b200 import _ffi
     src = '#include "sigmap_b200.h"\n#include <stdio.h>\nint main(){printf("%zu %zu %zu %zu %zu\\n",' \
           'sizeof(smb_params),sizeof(smb_mapping),sizeof(smb_chain),sizeof(smb_anchor),sizeof(smb_stats));}'
-    exe = "/tmp/smb_sizes"
+    exe = str(tmp_path / "smb_sizes")
     subprocess.run(["gcc", "-x", "c", "-", "-I", os.path.join(ROOT, "include"), "-o", exe],
                    input=src, text=True, check=True)
     got = [int(x) for x in subprocess.run([exe], capture_output=True, text=True).stdout.split()]

@@ -110,11 +110,30 @@ def test_paf_rows_golden_default_and_full(gmapper, golden, host):
             assert paf_cols(line) == golden.paf[mode][name], f"{mode} {name}"
 
 
-def test_cli_dropin_matches_reference_cli(ref, small, tmp_path):
+def test_cli_dropin_matches_reference_cli(ref, small, golden, host, tmp_path):
     """`sigmap -i` writes the reference's .pt byte for byte; `sigmap -m` on the reference-built
-    index prints the reference's PAF rows (all columns and tags except the wall-clock mt)."""
+    index prints the reference's PAF rows (all columns and tags except the wall-clock mt): on the
+    golden genome and reads against the stored rows of the reference CLI, and, where oracle/_ref
+    was built, on fresh inputs against the live reference."""
+    import hashlib
     from sigmap_b200.host import MODEL_PATH
     exe = os.path.join(ROOT, "sigmap_b200", "bin", "sigmap")
+    gdir = tmp_path / "golden"
+    (gdir / "sig").mkdir(parents=True)
+    fasta, gidx = str(gdir / "ref.fa"), str(gdir / "idx")
+    golden.genome(host).write_fasta(fasta)
+    golden.reads(host).write_blow5(str(gdir / "sig" / "reads.blow5"))
+    r = subprocess.run([exe, "-i", "-r", fasta, "-p", MODEL_PATH, "-o", gidx], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-400:]
+    assert hashlib.sha256(open(gidx + ".pt", "rb").read()).hexdigest() == str(golden["pt_sha256"])
+    full_read = ["--max-num-chunks", "100000", "--stop-mapping", "1e30", "--stop-mapping-mean", "1e30",
+                 "--min-num-anchors", "2000000000"]
+    for mode, extra in (("default", []), ("full", full_read)):
+        out = str(gdir / f"{mode}.paf")
+        r = subprocess.run([exe, "-m", "-r", fasta, "-p", MODEL_PATH, "-x", gidx, "-s", str(gdir / "sig"),
+                            "-o", out, "-t", "2"] + extra, capture_output=True, text=True)
+        assert r.returncode == 0, r.stderr[-400:]
+        assert {l.split("\t")[0]: paf_cols(l) for l in open(out)} == golden.paf[mode], mode
     ours_idx = str(tmp_path / "ours")
     r = subprocess.run([exe, "-i", "-r", small.fasta, "-p", MODEL_PATH, "-o", ours_idx],
                        capture_output=True, text=True)
@@ -127,8 +146,8 @@ def test_cli_dropin_matches_reference_cli(ref, small, tmp_path):
     assert "Finished mapping in" in r.stderr
     ours = {l.split("\t")[0]: paf_cols(l) for l in open(out)}
     assert len(ours) == small.reads.n
-    if ref is None:
-        pytest.skip("oracle/_ref not built: compared the .pt only")
+    if ref is None:  # the stored rows above are the comparison with the reference
+        return
     rout = str(tmp_path / "ref.paf")
     rr = ref.cli(["-i", "-r", small.fasta, "-p", MODEL_PATH, "-o", str(tmp_path / "refidx")])
     assert rr.returncode == 0
