@@ -187,6 +187,45 @@ uint32_t smb_index_num_contigs(const smb_ctx *ctx);
  * follow are independent per rank (no collective on the data path). */
 int smb_index_broadcast(smb_ctx *ctx, int root);
 
+/* ------------------------------------------------------- device index build */
+/* Sigmap::ConstructIndex (sigmap.cc:999-1046) on this context's GPU: the point cloud of
+ * smbh_build_point_cloud_alloc, bit for bit (same pos, val, order), built from the sequences
+ * without a host pass.  seqs[i] holds lengths[i] bases followed by a NUL.  *pos / *val are
+ * allocated by the library (release with smbh_free). */
+int smb_point_cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
+                          const float *level_mean, uint64_t **pos, float **val, size_t *count);
+/* One rank's part of that cloud, field for field what smbh_build_point_cloud_part fills (free
+ * with smbh_cloud_part_free).  Needs no shard group. */
+int smb_point_cloud_build_part(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
+                               const float *level_mean, const uint32_t *owner, uint32_t rank,
+                               struct smbh_cloud_part *out);
+/* The device index straight from the sequences; no point cloud passes through host memory.
+ * contig_owner == NULL: the whole index, as smb_index_set_points builds it from the same cloud.
+ * Otherwise this context's shard of a contig-sharded index, as smb_index_set_points_sharded builds
+ * it (join a shard group first); the device keeps only the rank's part.  Set the contig lengths
+ * with smb_index_set_contigs as usual.  SMB_ERR_CAPACITY when the device memory does not hold the
+ * build (about 6 bytes per base of the reference and 12 per point of the whole cloud, then the
+ * index itself). */
+int smb_index_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
+                    const float *level_mean, const uint32_t *contig_owner);
+/* The last device cloud build of this context.  The `last kept value` selection walks tiles of
+ * `tile` window starts (option "cloud_tile") speculatively, then re-walks the tiles whose incoming
+ * state it guessed wrong (DESIGN.md, device index build). */
+typedef struct smb_build_stats {
+  uint64_t points;             /* points of the whole cloud */
+  uint64_t tiles;              /* selection tiles */
+  uint64_t tiles_rewalked;     /* tiles whose first decisions differed from the speculative walk */
+  uint64_t tiles_unconverged;  /* tiles that passed their incoming state on (all masked, or never
+                                  met the speculative walk: a run of equal z) */
+  uint64_t tiles_redone;       /* tiles re-walked a second time, behind an unconverged one */
+  uint64_t tile;               /* window starts per tile */
+  uint32_t strands;            /* strands with a window (2 per contig of >= 11 bases) */
+  uint32_t strands_serial_mean; /* of those, strands whose level sum could not be taken as an exact
+                                   integer sum and was added sequentially (DESIGN.md) */
+  double ms_upload, ms_census, ms_levels, ms_zsums, ms_select, ms_scatter, ms_index; /* CUDA-event ms */
+} smb_build_stats;
+int smb_index_build_stats(smb_ctx *ctx, smb_build_stats *out);
+
 /* ------------------------------------------------------------ whole hot path */
 /* Replaces the per-read body of Sigmap::StreamingMap (sigmap.cc:630-866) for n_reads
  * reads at once: raw int16 samples of read r are raw[read_off[r] .. read_off[r+1]);

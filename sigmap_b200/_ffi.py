@@ -149,6 +149,19 @@ class CloudPart(C.Structure):
     ]
 
 
+class BuildStats(C.Structure):
+    _fields_ = [
+        ("points", C.c_uint64),
+        ("tiles", C.c_uint64),
+        ("tiles_rewalked", C.c_uint64),
+        ("tiles_unconverged", C.c_uint64),
+        ("tiles_redone", C.c_uint64),
+        ("tile", C.c_uint64),
+        ("strands", C.c_uint32),
+        ("strands_serial_mean", C.c_uint32),
+    ] + [(f"ms_{k}", C.c_double) for k in ("upload", "census", "levels", "zsums", "select", "scatter", "index")]
+
+
 # name -> (restype, argtypes); every symbol include/sigmap_b200.h declares
 PROTOTYPES = {
     "smb_default_params": (None, [C.POINTER(Params)]),
@@ -180,6 +193,12 @@ PROTOTYPES = {
     "smbh_cloud_part_free": (None, [C.POINTER(CloudPart)]),
     "smb_index_num_contigs": (C.c_uint32, [C.c_void_p]),
     "smb_index_broadcast": (C.c_int, [C.c_void_p, C.c_int]),
+    "smb_point_cloud_build": (C.c_int, [C.c_void_p, charpp, u32p, C.c_uint32, f32p, C.POINTER(u64p),
+                                        C.POINTER(f32p), C.POINTER(C.c_size_t)]),
+    "smb_point_cloud_build_part": (C.c_int, [C.c_void_p, charpp, u32p, C.c_uint32, f32p, u32p, C.c_uint32,
+                                             C.POINTER(CloudPart)]),
+    "smb_index_build": (C.c_int, [C.c_void_p, charpp, u32p, C.c_uint32, f32p, u32p]),
+    "smb_index_build_stats": (C.c_int, [C.c_void_p, C.POINTER(BuildStats)]),
     "smb_map_reads": (C.c_int, [C.c_void_p, i16p, u64p, f32p, f32p, f32p, C.c_size_t,
                                 C.POINTER(Params), C.POINTER(Mapping)]),
     "smb_reads_upload": (C.c_int, [C.c_void_p, i16p, u64p, f32p, f32p, f32p, C.c_size_t]),

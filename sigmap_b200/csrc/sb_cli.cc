@@ -8,9 +8,13 @@
 // collectives -- for references whose index exceeds one GPU).  `-t` is accepted for
 // compatibility (the GPU path does not use host mapping threads).
 //
-// Differences kept on purpose and documented in DESIGN.md: `-i` writes <prefix>.pt only (the
-// device index is rebuilt from the point cloud at load time; nanoflann's <prefix>.si is
-// neither needed nor produced); FAST5 input is not supported (BLOW5 only).
+// `-i` writes <prefix>.pt and <prefix>.si (a KD-tree in nanoflann's layout, for the reference's own
+// `sigmap -m`; this program never reads it: the device index is rebuilt from the point cloud at
+// load time).  The point cloud is built on the host, or on device N with an explicit --gpu N; the
+// files are the same byte for byte.  `-m --index-from-ref` builds the device index(es) from -r on
+// the devices instead of reading -x (with --shard contigs every device builds only its own part):
+// the way to map against a reference whose point cloud would not fit in host memory.
+// Difference kept on purpose and documented in DESIGN.md: FAST5 input is not supported (BLOW5 only).
 #include <dirent.h>
 #include <sys/stat.h>
 #include <sys/time.h>
@@ -67,6 +71,8 @@ struct Args {
   bool index = false, map = false, help = false;
   std::string ref, model, ref_index, sig_dir, output;
   int dimension = 6, max_leaf = 20, threads = 1, gpu = 0;
+  bool gpu_given = false;       // --gpu N given: `-i` builds the point cloud on device N
+  bool index_from_ref = false;  // --index-from-ref: `-m` builds the index from -r, no -x
   std::vector<int> gpus;       // --gpus 0,1,2,...: empty = the single device --gpu
   bool shard_contigs = false;  // --shard contigs
   smb_params prm;
@@ -80,12 +86,13 @@ const char *kHelp =
     " Mapping options:\n  -m, --map              Map signal data\n"
     "      --step-size INT    Seeding step size in reads [2]\n"
     "  -t, --num-threads INT  # threads for mapping [1] (accepted, unused on GPU)\n"
-    "      --gpu INT          CUDA device ordinal [0]\n"
+    "      --gpu INT          CUDA device ordinal [0]; with -i: build the point cloud on it\n"
     "      --gpus LIST        several devices, e.g. 0,1,2,3 (one context per entry)\n"
     "      --shard MODE       with --gpus: reads (split the reads, index replicated; default)\n"
     "                         or contigs (split the index by contig, chains merged)\n\n"
     " Input options:\n  -r, --ref FILE         Reference file\n  -p, --pore-model FILE  Pore model file\n"
-    "  -x, --ref-index FILE   Reference index file\n  -s, --sig-dir DIR      Signal data directory\n\n"
+    "  -x, --ref-index FILE   Reference index file\n"
+    "      --index-from-ref   with -m: build the index on the device(s) from -r instead of -x\n  -s, --sig-dir DIR      Signal data directory\n\n"
     " Output options:\n  -o, --output arg       Output file\n\n"
     " Development options:\n      --search-radius FLT            Search radius for each seed [0.08]\n"
     "      --max-num-chunks INT           Max # chunks before stop trying to map a read [30]\n"
@@ -120,7 +127,10 @@ Args parse(int argc, char **argv) {
     else if (o == "-d" || o == "--dimension") a.dimension = atoi(val().c_str());
     else if (o == "-l" || o == "--max-leaf") a.max_leaf = atoi(val().c_str());
     else if (o == "-t" || o == "--num-threads") a.threads = atoi(val().c_str());
-    else if (o == "--gpu") a.gpu = atoi(val().c_str());
+    else if (o == "--gpu") {
+      a.gpu = atoi(val().c_str());
+      a.gpu_given = true;
+    } else if (o == "--index-from-ref") a.index_from_ref = true;
     else if (o == "--gpus") {
       const std::string list = val();
       for (size_t at = 0; at <= list.size();) {
@@ -169,8 +179,15 @@ int build_index(const Args &a) {
   uint64_t *pos = nullptr;
   float *val = nullptr;
   size_t n = 0;
-  if (smbh_build_point_cloud_alloc(fa.seqs, fa.lengths, fa.n, mean.data(), &pos, &val, &n))
+  if (a.gpu_given) {
+    smb_ctx *ctx = nullptr;
+    if (smb_create(&ctx, a.gpu)) die(std::string("smb_create: ") + smb_last_error(nullptr));
+    if (smb_point_cloud_build(ctx, fa.seqs, fa.lengths, fa.n, mean.data(), &pos, &val, &n))
+      die(std::string("smb_point_cloud_build: ") + smb_last_error(ctx));
+    smb_destroy(ctx);
+  } else if (smbh_build_point_cloud_alloc(fa.seqs, fa.lengths, fa.n, mean.data(), &pos, &val, &n)) {
     die("Out of memory while collecting points!");
+  }
   fprintf(stderr, "Collected %zu points.\n", n);
   if (smbh_pt_write(a.output.c_str(), pos, val, n, a.dimension, a.max_leaf))
     die("Cannot write index file!");
@@ -189,11 +206,15 @@ int map_reads(const Args &a) {
   fprintf(stderr, "Number of threads: %d\n", a.threads);
   if (a.ref.empty()) die("No reference file specified!");
   if (a.model.empty()) die("No pore model file specified!");
-  if (a.ref_index.empty()) die("No reference index file specified!");
+  if (a.ref_index.empty() && !a.index_from_ref) die("No reference index file specified!");
   if (a.sig_dir.empty()) die("No signal data directory specified!");
   if (a.output.empty()) die("No output file specified!");
   fprintf(stderr, "Reference file: %s\nPore model file: %s\nReference index file: %s\nSignal directory: %s\nOutput file: %s\n",
-          a.ref.c_str(), a.model.c_str(), a.ref_index.c_str(), a.sig_dir.c_str(), a.output.c_str());
+          a.ref.c_str(), a.model.c_str(), a.index_from_ref ? "(built from the reference)" : a.ref_index.c_str(),
+          a.sig_dir.c_str(), a.output.c_str());
+  std::vector<float> level_mean(4096), level_stdv(4096);
+  if (a.index_from_ref && smbh_pore_model_load(a.model.c_str(), level_mean.data(), level_stdv.data()))
+    die("Cannot load pore model!");
   if (!is_dir(a.sig_dir)) die("Signal directory is in valid!");
   double t0 = now();
   std::vector<std::string> files;
@@ -218,7 +239,8 @@ int map_reads(const Args &a) {
     float *val = nullptr;
     size_t n_points = 0;
     int dim = 0, max_leaf = 0;
-    if (smbh_pt_read(a.ref_index.c_str(), &pos, &val, &n_points, &dim, &max_leaf)) die("Cannot read index file!");
+    if (!a.index_from_ref && smbh_pt_read(a.ref_index.c_str(), &pos, &val, &n_points, &dim, &max_leaf))
+      die("Cannot read index file!");
     std::vector<uint32_t> owner(std::max(fa.n, 1u), 0);
     smbh_assign_contigs(fa.lengths, fa.n, (uint32_t)G, owner.data());
     if (smb_shard_local_group(ctxs.data(), (uint32_t)G)) die(std::string("smb_shard_local_group: ") + smb_last_error(ctxs[0]));
@@ -226,7 +248,8 @@ int map_reads(const Args &a) {
     std::vector<std::thread> th;
     for (size_t g = 0; g < G; ++g)
       th.emplace_back([&, g] {
-        if (smb_index_set_points_sharded(ctxs[g], pos, val, n_points, owner.data(), fa.n) ||
+        if ((a.index_from_ref ? smb_index_build(ctxs[g], fa.seqs, fa.lengths, fa.n, level_mean.data(), owner.data())
+                              : smb_index_set_points_sharded(ctxs[g], pos, val, n_points, owner.data(), fa.n)) ||
             smb_index_set_contigs(ctxs[g], fa.lengths, fa.n))
           err[g] = smb_last_error(ctxs[g]);
       });
@@ -237,7 +260,12 @@ int map_reads(const Args &a) {
     smbh_free(val);
   } else {
     for (size_t g = 0; g < G; ++g) {
-      if (smb_index_load(ctxs[g], a.ref_index.c_str())) die(std::string("smb_index_load: ") + smb_last_error(ctxs[g]));
+      if (a.index_from_ref) {
+        if (smb_index_build(ctxs[g], fa.seqs, fa.lengths, fa.n, level_mean.data(), nullptr))
+          die(std::string("smb_index_build: ") + smb_last_error(ctxs[g]));
+      } else if (smb_index_load(ctxs[g], a.ref_index.c_str())) {
+        die(std::string("smb_index_load: ") + smb_last_error(ctxs[g]));
+      }
       if (smb_index_set_contigs(ctxs[g], fa.lengths, fa.n)) die(std::string("smb_index_set_contigs: ") + smb_last_error(ctxs[g]));
     }
   }

@@ -28,6 +28,7 @@
 #include "k_sort.cuh"
 #include "k_events.cuh"
 #include "k_index.cuh"
+#include "k_cloud.cuh"
 #include "sb_device.cuh"
 #include "sb_exchange.cuh"
 
@@ -258,6 +259,9 @@ struct smb_ctx {
   int pipeline_mode = 0;          // SMB_PIPELINE=auto|on|off: wave-pipelined ticks (see map_uploaded_impl)
   bool stage_big = true;          // SMB_STAGE=small: 128 staged hits per warp of the lean search kernel whatever the room
   bool index_kd = true;           // SMB_INDEX=morton: points in Morton order instead of the aligned KD order
+  uint32_t cloud_tile = 16384;    // SMB_CLOUD_TILE=n: window starts per tile of the device cloud's point selection
+  smb_build_stats build_stats{};  // the last device cloud build (smb_index_build_stats)
+  unsigned char *h_cloud_stage = nullptr;  // pinned: two upload slices of the device cloud build
   uint32_t sort_queries_min = 200000;  // SMB_SORT_QUERIES_MIN=n: batches with fewer queries keep their natural order
   bool dp_dynamic = true;         // SMB_DP=static: warp w of the DP grid handles segment w
   unsigned dp_grid = 148 * 8;     // persistent DP grid: every block that fits on the device
@@ -453,6 +457,19 @@ static int launch_search(smb_ctx *ctx, SearchArgs sa, uint32_t nq_max, cudaStrea
 }
 
 // ------------------------------------------------------------------ index build
+// What the KD-order build takes: device arrays plus the extent of the points the index sees.
+struct IndexInput {
+  const float *val;              // values the windows read (whole cloud, or a shard's runs)
+  const uint64_t *pos;           // position of every window (whole cloud: of every point)
+  const uint32_t *wsrc, *worig;  // shard: value index / whole-cloud index of each window (else null)
+  uint64_t W;                    // windows
+  size_t n_points;               // points of the whole cloud
+  float vmin, vmax;
+  uint32_t max_tpos, max_bucket;
+  std::vector<uint64_t> bucket_span;  // 1 + largest target per bucket (contig << 1 | strand)
+};
+static int build_index_core(smb_ctx *ctx, IndexInput &in);
+
 // owner == nullptr: every window of the cloud.  Otherwise (contig-sharded index) only the
 // windows whose first point lies on a contig with owner[contig] == rank; a window keeps its six
 // values even where it runs into the next contig / strand (Q2), so the shard holds exactly the
@@ -531,7 +548,6 @@ static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size
   const float *u_val = subset ? h_val.data() : val;
   const uint64_t *u_pos = subset ? h_pos.data() : pos;
   const size_t n_val = subset ? h_val.size() : n, n_pos = subset ? h_pos.size() : n;
-  const uint32_t n_leaves = (uint32_t)((W + kLeaf - 1) / kLeaf);
   const size_t n_seen = part ? part->n_values : n;  // points this rank can look at
   float vmin = n_seen ? val[0] : 0.0f, vmax = vmin;
   uint32_t max_tpos = 0, max_bucket = 0;
@@ -550,18 +566,12 @@ static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size
     if (b >= bucket_span.size()) bucket_span.resize((size_t)b + 1, 0);
     bucket_span[b] = std::max<uint64_t>(bucket_span[b], (uint64_t)t + 1);
   }
-  const float span = std::max(vmax - vmin, 1e-6f);
   cudaStream_t s = ctx->stream;
   DevBuf<float> d_val;
-  DevBuf<uint64_t> d_pos, code_a, code_b;
-  DevBuf<uint32_t> w_a, w_b, d_wsrc, d_worig;
-  DevBuf<unsigned char> tmp;
+  DevBuf<uint64_t> d_pos;
+  DevBuf<uint32_t> d_wsrc, d_worig;
   CK(d_val.ensure(n_val));
   CK(d_pos.ensure(n_pos));
-  CK(code_a.ensure(W));
-  CK(code_b.ensure(W));
-  CK(w_a.ensure(W));
-  CK(w_b.ensure(W));
   CK(cudaMemcpyAsync(d_val.p, u_val, n_val * sizeof(float), cudaMemcpyHostToDevice, s));
   CK(cudaMemcpyAsync(d_pos.p, u_pos, n_pos * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
   if (subset) {
@@ -570,6 +580,35 @@ static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size
     CK(cudaMemcpyAsync(d_wsrc.p, h_wsrc.data(), W * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(d_worig.p, h_worig.data(), W * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
   }
+  IndexInput in{d_val.p, d_pos.p, d_wsrc.p, d_worig.p, W, n, vmin, vmax, max_tpos, max_bucket, std::move(bucket_span)};
+  const int rc = build_index_core(ctx, in);
+  cudaStreamSynchronize(s);
+  d_val.release();
+  d_pos.release();
+  d_wsrc.release();
+  d_worig.release();
+  return rc;
+}
+
+// The KD-order build from device arrays, wherever they came from (host_index.cc's cloud uploaded
+// by build_index, or the device-built cloud of k_cloud.cuh).  Window w starts at value
+// wsrc[w] (w itself when wsrc is null) and is point worig[w] of the whole cloud.
+static int build_index_core(smb_ctx *ctx, IndexInput &in) {
+  const uint64_t W = in.W;
+  const uint32_t n_leaves = (uint32_t)((W + kLeaf - 1) / kLeaf);
+  const float vmin = in.vmin, span = std::max(in.vmax - in.vmin, 1e-6f);
+  const std::vector<uint64_t> &bucket_span = in.bucket_span;
+  const float *d_val = in.val;
+  const uint64_t *d_pos = in.pos;
+  const uint32_t *d_wsrc = in.wsrc, *d_worig = in.worig;
+  cudaStream_t s = ctx->stream;
+  DevBuf<uint64_t> code_a, code_b;
+  DevBuf<uint32_t> w_a, w_b;
+  DevBuf<unsigned char> tmp;
+  CK(code_a.ensure(W));
+  CK(code_b.ensure(W));
+  CK(w_a.ensure(W));
+  CK(w_b.ensure(W));
   DevBuf<uint32_t> ext_min, ext_max;
   const uint32_t *d_order = nullptr;
   if (ctx->index_kd && W > (uint64_t)kLeaf) {
@@ -589,9 +628,9 @@ static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size
       const uint64_t n_seg = (W + (1ull << log2s) - 1) >> log2s;
       CK(cudaMemsetAsync(ext_min.p, 0xFF, n_seg * kDim * sizeof(uint32_t), s));
       CK(cudaMemsetAsync(ext_max.p, 0x00, n_seg * kDim * sizeof(uint32_t), s));
-      k_kd_extent<<<blocks, kKdThreads, 0, s>>>(d_val.p, first ? nullptr : ia, d_wsrc.p, W, log2s, ext_min.p, ext_max.p);
+      k_kd_extent<<<blocks, kKdThreads, 0, s>>>(d_val, first ? nullptr : ia, d_wsrc, W, log2s, ext_min.p, ext_max.p);
       LAUNCH_CHECK();
-      k_kd_keys<<<blocks, kKdThreads, 0, s>>>(d_val.p, first ? nullptr : ia, d_wsrc.p, W, log2s, ext_min.p, ext_max.p,
+      k_kd_keys<<<blocks, kKdThreads, 0, s>>>(d_val, first ? nullptr : ia, d_wsrc, W, log2s, ext_min.p, ext_max.p,
                                               code_a.p, ia);
       LAUNCH_CHECK();
       int seg_bits = 0;
@@ -603,7 +642,7 @@ static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size
     }
     d_order = ia;
   } else {
-    k_morton<<<(unsigned)((W + 255) / 256), 256, 0, s>>>(d_val.p, W, vmin, 1.0f / span, code_a.p, w_a.p, d_wsrc.p);
+    k_morton<<<(unsigned)((W + 255) / 256), 256, 0, s>>>(d_val, W, vmin, 1.0f / span, code_a.p, w_a.p, d_wsrc);
     LAUNCH_CHECK();
     size_t tb = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, tb, code_a.p, code_b.p, w_a.p, w_b.p, (uint64_t)W, 0, 60, s);
@@ -615,10 +654,10 @@ static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size
   CK(ctx->leaves.ensure((size_t)n_leaves * kLeafRec));
   CK(ctx->leaf_widx.ensure((size_t)n_leaves * kLeaf));
   k_build_leaves<<<(unsigned)(((uint64_t)n_leaves * kLeaf + 255) / 256), 256, 0, s>>>(
-      d_val.p, d_pos.p, d_order, W, n_leaves, ctx->leaves.p, ctx->leaf_widx.p, d_wsrc.p, d_worig.p);
+      d_val, d_pos, d_order, W, n_leaves, ctx->leaves.p, ctx->leaf_widx.p, d_wsrc, d_worig);
   LAUNCH_CHECK();
   IndexView ix{};
-  ix.n_points = n;
+  ix.n_points = in.n_points;
   ix.n_windows = W;
   ix.n_leaves = n_leaves;
   ix.vmin = vmin;
@@ -662,14 +701,10 @@ static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size
   ix.leaves = ctx->leaves.p;
   ix.leaf_widx = ctx->leaf_widx.p;
   CK(cudaStreamSynchronize(s));
-  d_val.release();
-  d_pos.release();
   code_a.release();
   code_b.release();
   w_a.release();
   w_b.release();
-  d_wsrc.release();
-  d_worig.release();
   tmp.release();
   ext_min.release();
   ext_max.release();
@@ -687,8 +722,8 @@ static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size
   }
   ctx->ix = ix;
   ctx->search_grid_main = search_grid<false>(ctx);
-  ctx->max_tpos = max_tpos;
-  ctx->max_bucket = max_bucket;
+  ctx->max_tpos = in.max_tpos;
+  ctx->max_bucket = in.max_bucket;
   ctx->has_index = true;
   return SMB_OK;
 }
@@ -1513,6 +1548,8 @@ static bool apply_option(smb_ctx *ctx, const char *name_in, const char *value) {
     ctx->part_small = strcmp(value, "small") == 0;
   } else if (name == "DP") {
     ctx->dp_dynamic = strcmp(value, "static") != 0;
+  } else if (name == "CLOUD_TILE") {  // takes effect at the next device cloud build
+    ctx->cloud_tile = (uint32_t)std::min(std::max(atoi(value), 1), 1 << 30);
   } else if (name == "INDEX") {  // kd (default) | morton; takes effect at the next index build
     ctx->index_kd = strcmp(value, "morton") != 0;
   } else if (name == "DP_TILES") {
@@ -1627,7 +1664,8 @@ int smb_create(smb_ctx **out, int device) {
                                 (int)part_sort_smem_bytes(kPartSortCapSmall, 2304))) != cudaSuccess)
     return bail("cudaFuncSetAttribute(k_part_sort)", e);
   for (const char *name : {"SORT", "SEARCH", "FRONT_CAP", "RUNS_CAP", "GRAB", "PART_FILL", "PART", "DP", "DP_PASSES",
-                           "DP_TILES", "SORT_QUERIES_MIN", "INDEX", "PREP_ROUNDS", "PREP_BOUND", "PIPELINE", "STAGE", "EVENTS_OVERLAP", "EVENTS", "UPLOAD_SLICE_MB"})
+                           "DP_TILES", "SORT_QUERIES_MIN", "INDEX", "PREP_ROUNDS", "PREP_BOUND", "PIPELINE", "STAGE", "EVENTS_OVERLAP", "EVENTS", "UPLOAD_SLICE_MB",
+                           "CLOUD_TILE"})
     if (const char *env = getenv((std::string("SMB_") + name).c_str())) apply_option(ctx, name, env);
   {
     int per_sm = 0, n_sm = 148;
@@ -1689,6 +1727,7 @@ void smb_destroy(smb_ctx *ctx) {
   if (ctx->d_ctr) cudaFree(ctx->d_ctr);
   if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
   if (ctx->h_ctl) cudaFreeHost(ctx->h_ctl);
+  if (ctx->h_cloud_stage) cudaFreeHost(ctx->h_cloud_stage);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
 }
@@ -3008,6 +3047,519 @@ int smb_stream_round(smb_ctx *ctx, const uint32_t *channels, uint32_t n, const i
       make_row(ctx, st[ch], ctx->stream_kept[ch] + (uint32_t)ctx->stream_pending[ch].size(), used, &maps[i]);
     }
   }
+  return SMB_OK;
+}
+
+}  // extern "C"
+
+// ================================================================== device index build
+// The point cloud of host_index.cc's build_cloud, built on the device (k_cloud.cuh), and the
+// index built from it without a host copy.  DESIGN.md, "device index build".
+namespace {
+
+template <class T>
+struct DevArr {  // exact-size device array, freed with its owner
+  T *p = nullptr;
+  size_t n = 0;
+  DevArr() = default;
+  DevArr(const DevArr &) = delete;
+  DevArr &operator=(const DevArr &) = delete;
+  ~DevArr() { reset(); }
+  void reset() {
+    if (p) cudaFree(p);
+    p = nullptr;
+    n = 0;
+  }
+  cudaError_t alloc(size_t k) {
+    reset();
+    const cudaError_t e = cudaMalloc((void **)&p, std::max<size_t>(k, 1) * sizeof(T));
+    if (e != cudaSuccess) {
+      p = nullptr;
+      cudaGetLastError();  // an out-of-memory return is not sticky; clear it
+      return e;
+    }
+    n = k;
+    return e;
+  }
+};
+
+struct StageTimer {  // CUDA events between the stages of one build
+  cudaEvent_t ev[9] = {};
+  int n = 0;
+  ~StageTimer() {
+    for (cudaEvent_t e : ev)
+      if (e) cudaEventDestroy(e);
+  }
+  cudaError_t mark(cudaStream_t s) {
+    if (!ev[n]) {
+      const cudaError_t e = cudaEventCreate(&ev[n]);
+      if (e != cudaSuccess) return e;
+    }
+    return cudaEventRecord(ev[n++], s);
+  }
+  double ms(int a, int b) const {
+    float f = 0.0f;
+    if (a < n && b < n) cudaEventElapsedTime(&f, ev[a], ev[b]);
+    return f;
+  }
+};
+
+constexpr size_t kCloudSlice = 16u << 20;  // bytes per pinned upload slice
+
+}  // namespace
+
+#define CLOUD_ALLOC(arr, k, what)                                                                             \
+  do {                                                                                                        \
+    if ((arr).alloc(k) != cudaSuccess)                                                                        \
+      return fail(ctx, SMB_ERR_CAPACITY,                                                                      \
+                  std::string("device index build: out of device memory for ") + (what) + " (" +            \
+                      std::to_string(((size_t)(k) * sizeof(*(arr).p)) >> 20) + " MiB more)");              \
+  } while (0)
+
+// The whole cloud in device memory (*pos / *val, *count points).  Stage times go to
+// ctx->build_stats (ms_index is left to the caller).
+static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
+                       const float *level_mean, DevArr<uint64_t> &pos, DevArr<float> &val, uint64_t *count) {
+  using namespace cloud;
+  if (n && (!seqs || !lengths)) return fail(ctx, SMB_ERR_ARG, "device index build: null sequences / lengths");
+  if (!level_mean) return fail(ctx, SMB_ERR_ARG, "device index build: null level table");
+  CK(cudaSetDevice(ctx->device));
+  cudaStream_t s = ctx->stream;
+  smb_build_stats &bs = ctx->build_stats;
+  memset(&bs, 0, sizeof bs);
+  bs.tile = ctx->cloud_tile;
+  *count = 0;
+  // segments: + strands by contig, then - strands (contigs under 11 bases have no window)
+  std::vector<Seg> segs;
+  std::vector<uint64_t> plus_off(n, 0);
+  uint64_t n_bases = 0, n_pos = 0;
+  for (uint32_t c = 0; c < n; ++c) {
+    if (lengths[c] < (uint32_t)kMaskK) continue;
+    if (!seqs[c]) return fail(ctx, SMB_ERR_ARG, "device index build: null sequence");
+    plus_off[c] = n_bases;
+    n_bases += lengths[c];
+  }
+  for (uint32_t strand = 0; strand < 2; ++strand)
+    for (uint32_t c = 0; c < n; ++c) {
+      if (lengths[c] < (uint32_t)kMaskK) continue;
+      segs.push_back(Seg{plus_off[c], n_pos, lengths[c], c, strand, 0});
+      n_pos += lengths[c] - kK + 1;
+    }
+  if (segs.empty()) {
+    CLOUD_ALLOC(pos, 0, "the point cloud");
+    CLOUD_ALLOC(val, 0, "the point cloud");
+    return SMB_OK;
+  }
+  const uint32_t n_segs = (uint32_t)segs.size(), n_plus = n_segs / 2;
+  bs.strands = n_segs;
+  StageTimer tm;
+  CK(tm.mark(s));
+  // ---- upload the + strands through two pinned slices
+  DevArr<unsigned char> d_seq;
+  CLOUD_ALLOC(d_seq, n_bases, "the reference sequences");
+  {
+    const size_t slice = kCloudSlice;
+    cudaEvent_t done[2] = {};
+    if (!ctx->h_cloud_stage) CK(cudaHostAlloc((void **)&ctx->h_cloud_stage, 2 * slice, cudaHostAllocDefault));
+    CK(cudaEventCreateWithFlags(&done[0], cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&done[1], cudaEventDisableTiming));
+    int k = 0;
+    cudaError_t e = cudaSuccess;
+    for (uint32_t c = 0; c < n && e == cudaSuccess; ++c) {
+      if (lengths[c] < (uint32_t)kMaskK) continue;
+      for (uint64_t a = 0; a < lengths[c] && e == cudaSuccess; a += slice) {
+        const size_t len = (size_t)std::min<uint64_t>(slice, lengths[c] - a);
+        unsigned char *h = ctx->h_cloud_stage + (size_t)k * slice;
+        if ((e = cudaEventSynchronize(done[k])) != cudaSuccess) break;
+        memcpy(h, seqs[c] + a, len);
+        if ((e = cudaMemcpyAsync(d_seq.p + plus_off[c] + a, h, len, cudaMemcpyHostToDevice, s)) != cudaSuccess) break;
+        e = cudaEventRecord(done[k], s);
+        k ^= 1;
+      }
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    cudaEventDestroy(done[0]);
+    cudaEventDestroy(done[1]);
+    if (e != cudaSuccess) return fail(ctx, SMB_ERR_CUDA, std::string("device index build: upload: ") + cudaGetErrorString(e));
+  }
+  ctx->stats.h2d_bytes += n_bases;
+  DevArr<Seg> d_segs;
+  CLOUD_ALLOC(d_segs, n_segs, "the segment table");
+  CK(cudaMemcpyAsync(d_segs.p, segs.data(), n_segs * sizeof(Seg), cudaMemcpyHostToDevice, s));
+  CK(tm.mark(s));
+  // ---- 11-mer census over the + strands
+  std::vector<Chunk> chunks;
+  for (uint32_t i = 0; i < n_plus; ++i)
+    for (uint32_t p = 0; p < segs[i].len - kMaskK + 1; p += kChunkPos) chunks.push_back(Chunk{i, p});
+  const size_t n_census = chunks.size();
+  for (uint32_t i = 0; i < n_segs; ++i)
+    for (uint32_t p = 0; p < segs[i].len - kK + 1; p += kChunkPos) chunks.push_back(Chunk{i, p});
+  DevArr<Chunk> d_chunks;
+  DevArr<uint32_t> d_hist;
+  DevArr<unsigned long long> d_total;
+  CLOUD_ALLOC(d_chunks, chunks.size(), "the chunk table");
+  CLOUD_ALLOC(d_hist, (size_t)1 << (2 * kMaskK), "the 11-mer histogram");
+  CLOUD_ALLOC(d_total, 1, "the 11-mer histogram");
+  CK(cudaMemcpyAsync(d_chunks.p, chunks.data(), chunks.size() * sizeof(Chunk), cudaMemcpyHostToDevice, s));
+  CK(cudaMemsetAsync(d_hist.p, 0, d_hist.n * sizeof(uint32_t), s));
+  CK(cudaMemsetAsync(d_total.p, 0, sizeof(unsigned long long), s));
+  k_cloud_census<<<(unsigned)n_census, 256, 0, s>>>(d_seq.p, d_segs.p, d_chunks.p, d_hist.p, d_total.p);
+  LAUNCH_CHECK();
+  CK(tm.mark(s));
+  // ---- level hashes and mask, both strands
+  DevArr<uint16_t> d_hm;
+  CLOUD_ALLOC(d_hm, n_pos, "the per-position level hashes");
+  k_cloud_hm<<<(unsigned)(chunks.size() - n_census), 256, 0, s>>>(d_seq.p, d_segs.p, d_chunks.p + n_census, d_hist.p,
+                                                                   d_total.p, d_hm.p);
+  LAUNCH_CHECK();
+  CK(tm.mark(s));
+  CK(cudaStreamSynchronize(s));
+  d_seq.reset();
+  d_hist.reset();
+  d_chunks.reset();
+  // ---- z-normalisation: sequential double sums per strand -> z table per segment
+  DevArr<float> d_lv, d_ztab;
+  CLOUD_ALLOC(d_lv, kTable, "the level table");
+  CLOUD_ALLOC(d_ztab, (size_t)n_segs * kTable, "the z tables");
+  CK(cudaMemcpyAsync(d_lv.p, level_mean, kTable * sizeof(float), cudaMemcpyHostToDevice, s));
+  // the mean as an exact integer sum in units of the smallest ulp of the table (k_cloud_zsums):
+  // possible when every level is finite and a strand's sum of |level| / unit stays in an int64
+  int unit_exp = 0, int_ok = 1;
+  {
+    int lo = 1 << 30;
+    double q_max = 0.0;
+    for (int i = 0; i < kTable; ++i) {
+      const float x = level_mean[i];
+      if (!std::isfinite(x)) int_ok = 0;
+      else if (x != 0.0f) lo = std::min(lo, std::max(std::ilogb(x), -126) - 23);
+    }
+    if (lo == 1 << 30) lo = 0;
+    for (int i = 0; i < kTable && int_ok; ++i) q_max = std::max(q_max, std::ldexp(std::fabs((double)level_mean[i]), -lo));
+    uint32_t max_len = 0;
+    for (const Seg &g : segs) max_len = std::max(max_len, g.len);
+    if (!int_ok || q_max * (double)max_len >= 9.0e18) int_ok = 0;
+    unit_exp = lo;
+  }
+  DevArr<unsigned int> d_serial;
+  CLOUD_ALLOC(d_serial, 1, "the z sums");
+  CK(cudaMemsetAsync(d_serial.p, 0, sizeof(unsigned int), s));
+  k_cloud_zsums<<<(n_segs + kZWarps - 1) / kZWarps, kZWarps * 32, 0, s>>>(d_segs.p, n_segs, d_hm.p, d_lv.p, int_ok,
+                                                                           unit_exp, d_ztab.p, d_serial.p);
+  LAUNCH_CHECK();
+  CK(cudaMemcpyAsync(&bs.strands_serial_mean, d_serial.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, s));
+  CK(tm.mark(s));
+  // ---- point selection: speculative tiles, fix-up, chain
+  std::vector<Tile> tiles;
+  const uint32_t T = std::max<uint32_t>(ctx->cloud_tile, 1);
+  uint64_t n_tiles64 = 0;
+  for (const Seg &g : segs) n_tiles64 += (g.len - kMaskK + 1 + (uint64_t)T - 1) / T;
+  if (n_tiles64 >= 0xFFFFFFFFull) return fail(ctx, SMB_ERR_ARG, "device index build: more than 2^32 tiles: raise cloud_tile");
+  tiles.reserve(n_tiles64);
+  for (uint32_t i = 0; i < n_segs; ++i) {
+    const uint32_t nw = segs[i].len - kMaskK + 1;
+    for (uint32_t p = 0; p < nw; p += std::min(T, nw - p)) tiles.push_back(Tile{i, p, p + std::min(T, nw - p), 0});
+  }
+  const uint32_t n_tiles = (uint32_t)tiles.size();
+  DevArr<Tile> d_tiles;
+  DevArr<TileState> d_ts;
+  DevArr<uint8_t> d_flags;
+  DevArr<ChainStats> d_cs;
+  DevArr<unsigned long long> d_cnt, d_off;
+  CLOUD_ALLOC(d_tiles, n_tiles, "the tile table");
+  CLOUD_ALLOC(d_ts, n_tiles, "the tile states");
+  CLOUD_ALLOC(d_flags, n_pos, "the keep flags");
+  CLOUD_ALLOC(d_cs, 1, "the tile states");
+  CLOUD_ALLOC(d_cnt, n_tiles, "the tile counts");
+  CLOUD_ALLOC(d_off, n_tiles, "the tile counts");
+  CK(cudaMemcpyAsync(d_tiles.p, tiles.data(), n_tiles * sizeof(Tile), cudaMemcpyHostToDevice, s));
+  const unsigned tb = 128, tg = (n_tiles + tb - 1) / tb;
+  k_cloud_spec<<<tg, tb, 0, s>>>(d_segs.p, d_tiles.p, n_tiles, d_hm.p, d_ztab.p, d_flags.p, d_ts.p);
+  LAUNCH_CHECK();
+  k_cloud_assume<<<1, 1, 0, s>>>(d_ts.p, n_tiles);
+  LAUNCH_CHECK();
+  k_cloud_fix<<<tg, tb, 0, s>>>(d_segs.p, d_tiles.p, n_tiles, d_hm.p, d_ztab.p, d_flags.p, d_ts.p);
+  LAUNCH_CHECK();
+  k_cloud_chain<<<1, 1, 0, s>>>(d_segs.p, d_tiles.p, n_tiles, d_hm.p, d_ztab.p, d_flags.p, d_ts.p, d_cs.p);
+  LAUNCH_CHECK();
+  k_cloud_counts<<<tg, tb, 0, s>>>(d_ts.p, n_tiles, d_cnt.p);
+  LAUNCH_CHECK();
+  {
+    size_t tmp_bytes = 0;
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_cnt.p, d_off.p, (int64_t)n_tiles, s));
+    DevArr<unsigned char> tmp;
+    CLOUD_ALLOC(tmp, tmp_bytes, "the tile scan");
+    CK(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, d_cnt.p, d_off.p, (int64_t)n_tiles, s));
+    ctx->stats.launches += 2;
+    unsigned long long last_off = 0, last_cnt = 0;
+    ChainStats cs{};
+    CK(cudaMemcpyAsync(&last_off, d_off.p + n_tiles - 1, sizeof last_off, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(&last_cnt, d_cnt.p + n_tiles - 1, sizeof last_cnt, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(&cs, d_cs.p, sizeof cs, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    *count = last_off + last_cnt;
+    bs.tiles = n_tiles;
+    bs.tiles_rewalked = cs.rewalked;
+    bs.tiles_unconverged = cs.unconverged;
+    bs.tiles_redone = cs.redone;
+  }
+  CK(tm.mark(s));
+  // ---- scatter
+  CLOUD_ALLOC(pos, *count, "the point cloud");
+  CLOUD_ALLOC(val, *count, "the point cloud");
+  k_cloud_scatter<<<(unsigned)(((uint64_t)n_tiles * 32 + 255) / 256), 256, 0, s>>>(d_segs.p, d_tiles.p, n_tiles, d_hm.p,
+                                                                                     d_ztab.p, d_flags.p, d_off.p, pos.p, val.p);
+  LAUNCH_CHECK();
+  CK(tm.mark(s));
+  CK(cudaStreamSynchronize(s));
+  bs.points = *count;
+  bs.ms_upload = tm.ms(0, 1);
+  bs.ms_census = tm.ms(1, 2);
+  bs.ms_levels = tm.ms(2, 3);
+  bs.ms_zsums = tm.ms(3, 4);
+  bs.ms_select = tm.ms(4, 5);
+  bs.ms_scatter = tm.ms(5, 6);
+  return SMB_OK;
+}
+
+namespace {
+struct DevPart {  // one rank's part of the cloud in device memory (host_index.cc PartSink)
+  DevArr<uint64_t> pos, run_off, run_first, w_pos;
+  DevArr<float> val;
+  DevArr<uint8_t> own;
+  DevArr<uint32_t> w_src, w_orig;
+  uint64_t n_values = 0, n_runs = 0, n_windows = 0;
+};
+}  // namespace
+
+// The rank's part of the device cloud; with windows, also the window table of its shard.
+static int part_build(smb_ctx *ctx, const DevArr<uint64_t> &pos, const DevArr<float> &val, uint64_t n,
+                      const uint32_t *owner, uint32_t n_contigs, uint32_t rank, bool windows, DevPart &out) {
+  using namespace cloud;
+  cudaStream_t s = ctx->stream;
+  DevArr<uint32_t> d_owner;
+  CLOUD_ALLOC(d_owner, n_contigs, "the owner table");
+  CK(cudaMemcpyAsync(d_owner.p, owner, n_contigs * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+  const uint64_t nb64 = (n + kPartBlock - 1) / kPartBlock;
+  if (nb64 >= 0x7FFFFFFFull) return fail(ctx, SMB_ERR_CAPACITY, "device index build: cloud too large for one part pass");
+  const uint32_t nb = (uint32_t)std::max<uint64_t>(nb64, 1);
+  DevArr<unsigned long long> blk, cnt3, off3;
+  CLOUD_ALLOC(blk, nb, "the part counters");
+  CLOUD_ALLOC(cnt3, 3 * (size_t)nb, "the part counters");
+  CLOUD_ALLOC(off3, 3 * (size_t)nb + 3, "the part counters");
+  CK(cudaMemsetAsync(blk.p, 0, nb * sizeof(unsigned long long), s));
+  if (n) {
+    k_part_count<<<nb, kPartThreads, 0, s>>>(pos.p, n, d_owner.p, rank, blk.p);
+    LAUNCH_CHECK();
+  }
+  k_part_unpack<<<(nb + 255) / 256, 256, 0, s>>>(blk.p, nb, cnt3.p);
+  LAUNCH_CHECK();
+  size_t tmp_bytes = 0;
+  CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, cnt3.p, off3.p, (int64_t)nb, s));
+  DevArr<unsigned char> tmp;
+  CLOUD_ALLOC(tmp, tmp_bytes, "the part scan");
+  for (int k = 0; k < 3; ++k)
+    CK(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, cnt3.p + (size_t)k * nb, off3.p + (size_t)k * nb, (int64_t)nb, s));
+  ctx->stats.launches += 3;
+  unsigned long long last[6];
+  for (int k = 0; k < 3; ++k) {
+    CK(cudaMemcpyAsync(last + 2 * k, off3.p + (size_t)k * nb + nb - 1, 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(last + 2 * k + 1, cnt3.p + (size_t)k * nb + nb - 1, 8, cudaMemcpyDeviceToHost, s));
+  }
+  CK(cudaStreamSynchronize(s));
+  out.n_values = last[0] + last[1];
+  out.n_runs = last[2] + last[3];
+  out.n_windows = last[4] + last[5];
+  CLOUD_ALLOC(out.pos, out.n_values, "the rank's part");
+  CLOUD_ALLOC(out.val, out.n_values, "the rank's part");
+  CLOUD_ALLOC(out.own, out.n_values, "the rank's part");
+  CLOUD_ALLOC(out.run_off, out.n_runs + 1, "the rank's part");
+  CLOUD_ALLOC(out.run_first, out.n_runs, "the rank's part");
+  if (windows) {
+    CLOUD_ALLOC(out.w_pos, out.n_windows, "the shard's windows");
+    CLOUD_ALLOC(out.w_src, out.n_windows, "the shard's windows");
+    CLOUD_ALLOC(out.w_orig, out.n_windows, "the shard's windows");
+  }
+  if (n) {
+    k_part_emit<<<nb, kPartThreads, 0, s>>>(pos.p, val.p, n, d_owner.p, rank, off3.p, nb, out.pos.p, out.val.p,
+                                            out.own.p, out.run_off.p, out.run_first.p, windows ? out.w_pos.p : nullptr,
+                                            out.w_src.p, out.w_orig.p);
+    LAUNCH_CHECK();
+  }
+  const uint64_t end = out.n_values;
+  CK(cudaMemcpyAsync(out.run_off.p + out.n_runs, &end, sizeof end, cudaMemcpyHostToDevice, s));
+  CK(cudaStreamSynchronize(s));
+  return SMB_OK;
+}
+
+// Extent of the points the index sees (build_index's host loop, as device reductions).
+static int cloud_extent(smb_ctx *ctx, const uint64_t *pos, const float *val, uint64_t n, uint32_t n_buckets,
+                        bool fixed_buckets, IndexInput &in) {
+  using namespace cloud;
+  cudaStream_t s = ctx->stream;
+  DevArr<CloudExtent> d_ext;
+  DevArr<unsigned long long> d_span;
+  CLOUD_ALLOC(d_ext, 1, "the cloud extent");
+  CLOUD_ALLOC(d_span, n_buckets, "the cloud extent");
+  const CloudExtent init{0xFFFFFFFFu, 0u, 0u, 0u};
+  CK(cudaMemcpyAsync(d_ext.p, &init, sizeof init, cudaMemcpyHostToDevice, s));
+  CK(cudaMemsetAsync(d_span.p, 0, n_buckets * sizeof(unsigned long long), s));
+  if (n) {
+    const unsigned grid = (unsigned)std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->n_sm * 8);
+    k_cloud_extent<<<grid, 256, 0, s>>>(pos, val, n, d_ext.p, d_span.p);
+    LAUNCH_CHECK();
+  }
+  CloudExtent ext{};
+  std::vector<uint64_t> span(n_buckets);
+  CK(cudaMemcpyAsync(&ext, d_ext.p, sizeof ext, cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(span.data(), d_span.p, n_buckets * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  in.vmin = n ? ord_val(ext.vmin_ord) : 0.0f;
+  in.vmax = n ? ord_val(ext.vmax_ord) : 0.0f;
+  in.max_tpos = ext.max_tpos;
+  // the host loop sizes the bucket table by the largest bucket seen (a shard: every bucket)
+  in.max_bucket = fixed_buckets ? n_buckets - 1 : ext.max_bucket;
+  span.resize(fixed_buckets ? n_buckets : (n ? (size_t)ext.max_bucket + 1 : 0));
+  in.bucket_span = std::move(span);
+  return SMB_OK;
+}
+
+extern "C" {
+
+int smb_point_cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
+                          const float *level_mean, uint64_t **pos, float **val, size_t *count) {
+  if (!pos || !val || !count) return fail(ctx, SMB_ERR_ARG, "smb_point_cloud_build: null output");
+  *pos = nullptr;
+  *val = nullptr;
+  *count = 0;
+  DevArr<uint64_t> d_pos;
+  DevArr<float> d_val;
+  uint64_t c = 0;
+  int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &c);
+  if (rc) return rc;
+  uint64_t *P = (uint64_t *)malloc(std::max<uint64_t>(c, 1) * sizeof(uint64_t));
+  float *V = (float *)malloc(std::max<uint64_t>(c, 1) * sizeof(float));
+  if (!P || !V) {
+    free(P);
+    free(V);
+    return fail(ctx, SMB_ERR_IO, "smb_point_cloud_build: out of host memory");
+  }
+  cudaError_t e = cudaMemcpy(P, d_pos.p, c * sizeof(uint64_t), cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess) e = cudaMemcpy(V, d_val.p, c * sizeof(float), cudaMemcpyDeviceToHost);
+  if (e != cudaSuccess) {
+    free(P);
+    free(V);
+    return fail(ctx, SMB_ERR_CUDA, std::string("smb_point_cloud_build: ") + cudaGetErrorString(e));
+  }
+  ctx->stats.d2h_bytes += c * 12;
+  *pos = P;
+  *val = V;
+  *count = c;
+  return SMB_OK;
+}
+
+int smb_point_cloud_build_part(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
+                               const float *level_mean, const uint32_t *owner, uint32_t rank, smbh_cloud_part *out) {
+  if (!out) return fail(ctx, SMB_ERR_ARG, "smb_point_cloud_build_part: null output");
+  memset(out, 0, sizeof *out);
+  if (!owner) return fail(ctx, SMB_ERR_ARG, "smb_point_cloud_build_part: null owner table");
+  DevPart part;
+  {
+    DevArr<uint64_t> d_pos;
+    DevArr<float> d_val;
+    uint64_t c = 0;
+    int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &c);
+    if (rc) return rc;
+    rc = part_build(ctx, d_pos, d_val, c, owner, n, rank, false, part);
+    if (rc) return rc;
+    out->n_points_total = c;
+  }
+  out->n_values = part.n_values;
+  out->n_runs = part.n_runs;
+  auto take = [](const void *src, size_t bytes, cudaError_t &e) -> void * {
+    void *p = malloc(bytes ? bytes : 1);
+    if (p && bytes && e == cudaSuccess) e = cudaMemcpy(p, src, bytes, cudaMemcpyDeviceToHost);
+    return p;
+  };
+  cudaError_t e = cudaSuccess;
+  out->pos = (uint64_t *)take(part.pos.p, part.n_values * sizeof(uint64_t), e);
+  out->val = (float *)take(part.val.p, part.n_values * sizeof(float), e);
+  out->own = (uint8_t *)take(part.own.p, part.n_values, e);
+  out->run_off = (uint64_t *)take(part.run_off.p, (part.n_runs + 1) * sizeof(uint64_t), e);
+  out->run_first = (uint64_t *)take(part.run_first.p, part.n_runs * sizeof(uint64_t), e);
+  if (!out->pos || !out->val || !out->own || !out->run_off || !out->run_first || e != cudaSuccess) {
+    smbh_cloud_part_free(out);
+    return e != cudaSuccess ? fail(ctx, SMB_ERR_CUDA, std::string("smb_point_cloud_build_part: ") + cudaGetErrorString(e))
+                            : fail(ctx, SMB_ERR_IO, "smb_point_cloud_build_part: out of host memory");
+  }
+  return SMB_OK;
+}
+
+int smb_index_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
+                    const float *level_mean, const uint32_t *contig_owner) {
+  CK(cudaSetDevice(ctx->device));
+  if (contig_owner) {
+    if (!ctx->ex) return fail(ctx, SMB_ERR_STATE, "join a shard group first (smb_shard_local_group / smb_shard_nccl_init)");
+    if (!n) return fail(ctx, SMB_ERR_ARG, "smb_index_build: no contigs");
+    for (uint32_t c = 0; c < n; ++c)
+      if (contig_owner[c] >= (uint32_t)ctx->ex->world) return fail(ctx, SMB_ERR_ARG, "contig owner out of range");
+  }
+  DevArr<uint64_t> d_pos;
+  DevArr<float> d_val;
+  uint64_t N = 0;
+  int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &N);
+  if (rc) return rc;
+  if (N < (uint64_t)kDim) return fail(ctx, SMB_ERR_ARG, "point cloud smaller than the index dimension");
+  StageTimer tm;
+  CK(tm.mark(ctx->stream));
+  const uint64_t W_all = N - (kDim - 1);
+  if (!contig_owner) {
+    if (W_all > 0xFFFFFFF0ull) return fail(ctx, SMB_ERR_CAPACITY, "more than 2^32 window points: shard the index by contig");
+    IndexInput in{d_val.p, d_pos.p, nullptr, nullptr, W_all, (size_t)N, 0.0f, 0.0f, 0u, 0u, {}};
+    rc = cloud_extent(ctx, d_pos.p, d_val.p, N, 2 * n, false, in);
+    if (!rc) rc = build_index_core(ctx, in);
+    ctx->index_sharded = false;
+  } else {
+    const uint32_t rank = (uint32_t)ctx->ex->rank;
+    DevPart part;
+    rc = part_build(ctx, d_pos, d_val, N, contig_owner, n, rank, true, part);
+    if (rc) return rc;
+    d_pos.reset();  // the rank keeps its part only
+    d_val.reset();
+    if (part.n_values > 0xFFFFFFF0ull)
+      return fail(ctx, SMB_ERR_CAPACITY, "more than 2^32 window points on one shard: use more ranks");
+    IndexInput in{part.val.p, part.w_pos.p, part.w_src.p, part.w_orig.p, part.n_windows, (size_t)N, 0.0f, 0.0f, 0u, 0u, {}};
+    rc = cloud_extent(ctx, part.pos.p, part.val.p, part.n_values, 2 * n, true, in);
+    if (rc) return rc;
+    if (part.n_windows == 0) {  // a rank may own nothing (more ranks than contigs): one padding leaf
+      const float pad[kDim] = {kPadValue, kPadValue, kPadValue, kPadValue, kPadValue, kPadValue};
+      const uint64_t pad_pos = ~0ull;
+      const uint32_t zero = 0, none = 0xFFFFFFFFu;
+      CLOUD_ALLOC(part.val, kDim, "the padding leaf");
+      CLOUD_ALLOC(part.w_pos, 1, "the padding leaf");
+      CLOUD_ALLOC(part.w_src, 1, "the padding leaf");
+      CLOUD_ALLOC(part.w_orig, 1, "the padding leaf");
+      CK(cudaMemcpy(part.val.p, pad, sizeof pad, cudaMemcpyHostToDevice));
+      CK(cudaMemcpy(part.w_pos.p, &pad_pos, 8, cudaMemcpyHostToDevice));
+      CK(cudaMemcpy(part.w_src.p, &zero, 4, cudaMemcpyHostToDevice));
+      CK(cudaMemcpy(part.w_orig.p, &none, 4, cudaMemcpyHostToDevice));
+      in.val = part.val.p;
+      in.pos = part.w_pos.p;
+      in.wsrc = part.w_src.p;
+      in.worig = part.w_orig.p;
+      in.W = 1;
+    }
+    rc = build_index_core(ctx, in);
+    ctx->index_sharded = rc == SMB_OK;
+  }
+  CK(tm.mark(ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  ctx->build_stats.ms_index = tm.ms(0, 1);
+  return rc;
+}
+
+int smb_index_build_stats(smb_ctx *ctx, smb_build_stats *out) {
+  if (!out) return fail(ctx, SMB_ERR_ARG, "smb_index_build_stats: null output");
+  *out = ctx->build_stats;
   return SMB_OK;
 }
 

@@ -120,6 +120,50 @@ class Mapper:
         self._check(F.lib.smb_index_set_points_part(self._ctx, C.byref(part.c), n_contigs),
                     "smb_index_set_points_part")
 
+    def build_index(self, ref, level_mean, owner=None):
+        """Build the device index from the reference sequences on this GPU (smb_index_build): the
+        index set_index builds from host.build_point_cloud, with no point cloud in host memory.
+        owner: contig -> shard rank table; this context's shard only (join a group first).
+        Sets the contig lengths too."""
+        level_mean = np.ascontiguousarray(level_mean, np.float32)
+        own = None if owner is None else np.ascontiguousarray(owner, np.uint32)
+        self._check(F.lib.smb_index_build(self._ctx, ref.seq_ptrs, F.ptr(ref.lengths, F.u32p), ref.n,
+                                          F.ptr(level_mean, F.f32p), F.ptr(own, F.u32p)), "smb_index_build")
+        self.set_contigs(ref.lengths)
+
+    def point_cloud(self, ref, level_mean):
+        """(pos uint64[n], val float32[n]) built on this GPU: equal to host.build_point_cloud."""
+        level_mean = np.ascontiguousarray(level_mean, np.float32)
+        pp, vp, n = F.u64p(), F.f32p(), C.c_size_t()
+        self._check(F.lib.smb_point_cloud_build(self._ctx, ref.seq_ptrs, F.ptr(ref.lengths, F.u32p), ref.n,
+                                                F.ptr(level_mean, F.f32p), C.byref(pp), C.byref(vp),
+                                                C.byref(n)), "smb_point_cloud_build")
+        try:
+            pos = np.ctypeslib.as_array(pp, (max(n.value, 1),))[:n.value].copy()
+            val = np.ctypeslib.as_array(vp, (max(n.value, 1),))[:n.value].copy()
+        finally:
+            F.lib.smbh_free(pp)
+            F.lib.smbh_free(vp)
+        return pos, val
+
+    def point_cloud_part(self, ref, level_mean, owner, rank):
+        """Shard `rank`'s part of the point cloud built on this GPU: equal to
+        host.build_point_cloud_part (a host.CloudPart)."""
+        from .host import CloudPart
+        level_mean = np.ascontiguousarray(level_mean, np.float32)
+        owner = np.ascontiguousarray(owner, np.uint32)
+        c = F.CloudPart()
+        self._check(F.lib.smb_point_cloud_build_part(self._ctx, ref.seq_ptrs, F.ptr(ref.lengths, F.u32p), ref.n,
+                                                     F.ptr(level_mean, F.f32p), F.ptr(owner, F.u32p), rank,
+                                                     C.byref(c)), "smb_point_cloud_build_part")
+        return CloudPart(c)
+
+    def build_stats(self):
+        """Tiles and per-stage device milliseconds of the last device cloud build."""
+        s = F.BuildStats()
+        self._check(F.lib.smb_index_build_stats(self._ctx, C.byref(s)), "smb_index_build_stats")
+        return {k: getattr(s, k) for k, _ in F.BuildStats._fields_}
+
     def broadcast_index(self, root=0):
         """Read-sharded runs: receive (or, on `root`, send) the device index over NVLink instead of
         building it on every rank.  Collective over the joined group; contig lengths travel too."""

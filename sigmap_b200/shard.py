@@ -177,6 +177,13 @@ class ContigShardGroup:
                 part.close()
             m.set_contigs(ref.lengths)
 
+    def build_index(self, ref, level_mean, owner=None):
+        """Contig-sharded index built on the devices from the reference sequences
+        (smb_index_build): each member builds the cloud on its GPU and keeps only its own part."""
+        owner = assign_contigs(ref.lengths, self.world) if owner is None else owner
+        self.owner = np.ascontiguousarray(owner, np.uint32)
+        self._each(lambda m: m.build_index(ref, level_mean, self.owner))
+
     def replicate_index(self, pos, val, contig_lengths, root=0):
         """Read-sharded mode: the index is built on `root` only and broadcast to the other members
         over NVLink / peer copies (smb_index_broadcast); every member then maps its own reads."""
