@@ -130,8 +130,8 @@ int smb_set_limits(smb_ctx *ctx, uint32_t max_batch_chunks, uint64_t max_batch_a
 
 /* Run-time switches for A/B measurements and for tests that have to reach the fallback paths:
  * name = an SMB_<NAME> environment variable without the prefix (smb_create reads those once),
- * e.g. ("sort", "part|entry|small|global"), ("search", "lean|general"), ("front_cap", "72"),
- * ("runs_cap", "64"), ("dp", "dynamic|static"), ("events", "auto|thread|warp").  Results never
+ * e.g. ("sort", "part|entry|global"), ("search", "lean|general"), ("front_cap", "72"),
+ * ("runs_cap", "64"), ("dp_passes", "3"), ("events", "auto|thread|warp").  Results never
  * depend on them (every path is held to the same parity tests); only speed does. */
 int smb_set_option(smb_ctx *ctx, const char *name, const char *value);
 

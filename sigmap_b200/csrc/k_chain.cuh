@@ -306,7 +306,7 @@ __global__ void __launch_bounds__(kPrepThreads, 8) k_chain_prep(ChainArgs a) {
       }
       // position-only link test over the maximal lookback range, cut where the target gap alone
       // rules every further predecessor out: 3 dt >= 4 (q_i - qmin) >= 4 dq
-      const int32_t qlim = (a.seg_qmin && sg < a.n_slots) ? 4 * (qi - (int32_t)a.seg_qmin[sg]) : 0x7FFFFFFF;
+      const int32_t qlim = sg < a.n_slots ? 4 * (qi - (int32_t)a.seg_qmin[sg]) : 0x7FFFFFFF;
       const int depth = (int)min(i, (uint32_t)kBand);
       const int in_smem = min(depth, me);
       int d = 1;
@@ -390,7 +390,7 @@ __global__ void __launch_bounds__(kPrepThreads, 8) k_chain_prep(ChainArgs a) {
       const float ci = a.coef[i];
       // no predecessor at or beyond 3 dt >= 4 (q_i - qmin) can be gap-compatible: whatever the
       // reference's loop still does there (count skips, break) leaves score and predecessor as they are
-      const int32_t qlim = (a.seg_qmin && (uint32_t)mine.x < a.n_slots) ? 4 * (qi - (int32_t)a.seg_qmin[mine.x]) : 0x7FFFFFFF;
+      const int32_t qlim = (uint32_t)mine.x < a.n_slots ? 4 * (qi - (int32_t)a.seg_qmin[mine.x]) : 0x7FFFFFFF;
       float M = __int_as_float(mine.w);  // 6 * coef = chaining_scores[anchor_index]
       uint32_t best = i;
       int S = 0;  // num_skips
@@ -810,15 +810,10 @@ __global__ void __launch_bounds__(kDpPassThreads, 6) k_dp_pass(ChainArgs a) {
 
 // Segments differ a lot in how many linked anchors they hold, so a fixed warp <-> segment
 // assignment leaves most warps of a block idle behind its slowest one: persistent warps take
-// segments from a work cursor instead (dynamic = 0: warp w handles segment w).
-__global__ void __launch_bounds__(kDpThreads) k_chain_dp(ChainArgs a, int dynamic) {
+// segments from a work cursor instead.
+__global__ void __launch_bounds__(kDpThreads) k_chain_dp(ChainArgs a) {
   const int lane = threadIdx.x & 31;
   if (a.ctr->abort) return;
-  if (!dynamic) {
-    const uint32_t slot = (blockIdx.x * kDpThreads + threadIdx.x) / 32;
-    if (slot < a.n_slots) dp_segment(a, slot, lane);
-    return;
-  }
   for (;;) {
     uint32_t slot = 0;
     if (lane == 0) slot = atomicAdd(&a.ctr->dp_cursor, 1u);

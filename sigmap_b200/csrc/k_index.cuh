@@ -2,9 +2,8 @@
 // KD-tree (nanoflann.hpp:858-1004 build, :1278-1410 radius search), and its build kernels.
 //
 // Layout (see IndexView in sb_device.cuh): the N-5 window points value[w..w+5]
-// (sigmap_adaptor.h:89-97) are put into the aligned KD order (below; or sorted by a 60-bit Morton
-// code, 6 dims x 10 bits) and cut into 8-point leaves; 8 consecutive leaves / nodes form the next
-// level's node, pointer-free.  A query is handled by ONE WARP that advances EIGHT tree nodes (or
+// (sigmap_adaptor.h:89-97) are put into the aligned KD order (below) and cut into 8-point leaves;
+// 8 consecutive leaves / nodes form the next level's node, pointer-free.  A query is handled by ONE WARP that advances EIGHT tree nodes (or
 // eight leaves) per step, two per 8-lane group: every lane tests two child boxes (three 8-byte
 // loads each) or evaluates two points, so each step keeps six independent loads per lane in
 // flight and the whole warp stays busy at fan-out 8 -- where a 6-D hierarchy prunes far better
@@ -30,33 +29,6 @@ constexpr float kPadValue = 1.0e18f;  // padding points: never inside any ball
 constexpr float kPadExtent = -1.0e18f;  // padding boxes: negative half extent, never met
 
 // ------------------------------------------------------------------ build
-__device__ __forceinline__ uint64_t spread10(uint32_t v) {
-  // bit i of v -> bit 6*i
-  uint64_t r = 0;
-#pragma unroll
-  for (int i = 0; i < 10; ++i) r |= (uint64_t)((v >> i) & 1u) << (6 * i);
-  return r;
-}
-
-// wsrc (contig-sharded index): offset of local window w's first value in val[]; nullptr = w
-__global__ void k_morton(const float *__restrict__ val, uint64_t n_windows, float vmin, float inv_span,
-                         uint64_t *__restrict__ code, uint32_t *__restrict__ widx,
-                         const uint32_t *__restrict__ wsrc) {
-  uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (w >= n_windows) return;
-  const uint64_t v0 = wsrc ? (uint64_t)wsrc[w] : w;
-  uint64_t c = 0;
-#pragma unroll
-  for (int d = 0; d < kDim; ++d) {
-    float t = (val[v0 + d] - vmin) * inv_span * 1024.0f;
-    int qv = (int)t;
-    qv = qv < 0 ? 0 : (qv > 1023 ? 1023 : qv);
-    c |= spread10((uint32_t)qv) << (kDim - 1 - d);
-  }
-  code[w] = c;
-  widx[w] = (uint32_t)w;
-}
-
 // ---- aligned KD order (the default point order).  The pointer-free hierarchy puts node k of level
 // l over the points [k * 8^(l+1), (k+1) * 8^(l+1)) of the order, so any order works; what the search
 // pays for is how tight those groups are.  Morton order cuts space at fixed midpoints and a group of
@@ -156,7 +128,8 @@ k_kd_keys(const float *__restrict__ val, const uint32_t *__restrict__ idx, const
   if (!idx) idx_out[i] = w;
 }
 
-// sorted rank i -> leaf records; one thread per slot of the padded leaf array
+// sorted rank i -> leaf records; one thread per slot of the padded leaf array.  order == nullptr:
+// rank i is window i (an index of one leaf)
 __global__ void k_build_leaves(const float *__restrict__ val, const uint64_t *__restrict__ pos,
                                const uint32_t *__restrict__ order, uint64_t n_windows,
                                uint32_t n_leaves, uint2 *__restrict__ leaves,
@@ -168,7 +141,7 @@ __global__ void k_build_leaves(const float *__restrict__ val, const uint64_t *__
   uint2 *rec = leaves + (size_t)leaf * kLeafRec + sub;
   float2 *v = reinterpret_cast<float2 *>(rec);
   if (i < n_windows) {
-    const uint32_t w = order[i];
+    const uint32_t w = order ? order[i] : (uint32_t)i;
     const uint64_t v0 = wsrc ? (uint64_t)wsrc[w] : (uint64_t)w;
 #pragma unroll
     for (int k = 0; k < 3; ++k) v[k * kLeaf] = make_float2(val[v0 + 2 * k], val[v0 + 2 * k + 1]);
@@ -369,7 +342,6 @@ struct SearchArgs {
   float inv_span;              // 1 / coordinates per part
   const uint64_t *bucket_base;
   uint32_t n_buckets;
-  uint32_t grab;               // queries per grab of the work counter (0 = default)
   unsigned int *work;          // the work counter of this launch
   // lean kernel: queries in Morton order.  order[k] = payload of the k-th query (pipeline:
   // entry << kQueryBits | query number; stage: query id); nullptr = natural order.
@@ -696,7 +668,7 @@ k_search_lean(const __grid_constant__ IndexView ix, const __grid_constant__ Sear
   const int top_level = ix.n_levels - 1;
   const int n_top = (int)ix.level_count[top_level];  // <= 8
   const int front_cap = (int)a.front_cap;
-  const uint32_t grab = a.grab ? a.grab : (uint32_t)kLeanGrab;
+  const uint32_t grab = (uint32_t)kLeanGrab;
   const bool routed = !STAGE && a.runs;
   int staged = 0;
   uint32_t staged_entry = 0;
@@ -860,7 +832,7 @@ k_radius_search(const __grid_constant__ IndexView ix, const __grid_constant__ Se
   const uint32_t nq = a.qlist ? *a.qlist_n : (STAGE ? a.n_queries : a.q_off[a.B]);
   const float r2 = a.radius;
   const float r2_prune = r2 * 1.0001f + 1e-12f;
-  const uint32_t grab = a.qlist ? 1u : (a.grab ? a.grab : (uint32_t)kSearchGrab);
+  const uint32_t grab = a.qlist ? 1u : (uint32_t)kSearchGrab;
   const int top_level = n_levels - 1;
   const uint32_t n_top = ix.level_count[top_level];  // <= 8
   const bool routed = !STAGE && a.runs;

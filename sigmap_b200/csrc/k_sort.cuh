@@ -29,15 +29,12 @@ namespace sb {
 
 constexpr int kRunsCap = 512;        // run records a k_part_sort CTA holds in shared memory at a time (one tile of a
                                      // list); the lists themselves hold runs_cap records, sized per step by the host
-// Two shapes of the kernel (template parameters CAP = anchors of one part held in shared memory,
-// THREADS, BINS = fine bins per part):
-//   <10240, 1024, 8192>  one 200 KB CTA per SM: fewest passes over an entry's runs
-//   < 5120,  512, 4096>  two 100 KB CTAs per SM: one CTA's barrier / DRAM waits overlap the
-//                        other's work, at the price of twice the parts per entry
-constexpr int kSortCapBig = 10240, kSortCapSmall = 5120;
-// k_part_sort shapes: <5120, 512, 4096> two 105 KB CTAs per SM; <2304, 256, 2304> four 52 KB CTAs
+// k_seg_sort runs as <10240, 1024, 8192> (template parameters CAP = anchors of one part held in
+// shared memory, THREADS, BINS = fine bins per part): one 200 KB CTA per SM, the fewest passes
+// over an entry's runs
+constexpr int kSortCapBig = 10240;
+// k_part_sort runs as <5120, 512, 4096>: two 105 KB CTAs per SM
 constexpr int kPartSortCap = 5120;   // anchors of one (entry, part) held by a k_part_sort CTA
-constexpr int kPartSortCapSmall = 2304;
 constexpr int kCoarseBins = 256;
 constexpr int kSmallBin = 24;        // bins up to this size: insertion sort by one thread
 constexpr int kBigBinCap = 512;      // dense bins queued for the warp-wide rank sort

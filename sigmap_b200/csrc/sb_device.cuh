@@ -65,9 +65,9 @@ struct DevBuf {
 };
 
 // ---- flat device index over the ordered window points (replaces nanoflann) ----
-// Leaves hold 8 consecutive points of the point order (aligned KD order, k_index.cuh; Morton order
-// with SMB_INDEX=morton); a node holds the boxes of its 8
-// children (level 0: leaves 8n..8n+7, level l: nodes 8n..8n+7 of level l-1), pointer-free.
+// Leaves hold 8 consecutive points of the point order (aligned KD order, k_index.cuh); a node
+// holds the boxes of its 8 children (level 0: leaves 8n..8n+7, level l: nodes 8n..8n+7 of level
+// l-1), pointer-free.
 // A warp works on FOUR nodes (or leaves) per half step, one 8-lane group each, so records are
 // laid out for 8 lanes:
 //   node  = [3][8 children] x four binary16: (lo0 lo1 lo2 lo3) (lo4 lo5 hi0 hi1) (hi2 hi3 hi4 hi5),

@@ -251,25 +251,17 @@ struct smb_ctx {
   int gshift = 0;
   uint32_t n_coarse = 1;
   uint64_t g_total = 1;           // linear coordinates of the whole index (sum of the bucket spans)
-  double part_fill = 0.70;        // share of a k_part_sort CTA's capacity an average part should fill
   int dp_passes = kDpFreePasses;  // SMB_DP_PASSES=n
-  bool prep_bound = true;         // SMB_PREP_BOUND=0: link test over the whole 5 000-position range
   int prep_rounds = kPrepRounds;  // SMB_PREP_ROUNDS=n: settle rounds inside k_chain_prep (0 = none)
   uint32_t dp_pass_max_entries = kDpPassMaxEntries;  // SMB_DP_TILES=n: per-tile DP pass up to n chunks per step (0 = never)
   int pipeline_mode = 0;          // SMB_PIPELINE=auto|on|off: wave-pipelined ticks (see map_uploaded_impl)
-  bool stage_big = true;          // SMB_STAGE=small: 128 staged hits per warp of the lean search kernel whatever the room
-  bool index_kd = true;           // SMB_INDEX=morton: points in Morton order instead of the aligned KD order
   uint32_t cloud_tile = 16384;    // SMB_CLOUD_TILE=n: window starts per tile of the device cloud's point selection
   smb_build_stats build_stats{};  // the last device cloud build (smb_index_build_stats)
   unsigned char *h_cloud_stage = nullptr;  // pinned: two upload slices of the device cloud build
   uint32_t sort_queries_min = 200000;  // SMB_SORT_QUERIES_MIN=n: batches with fewer queries keep their natural order
-  bool dp_dynamic = true;         // SMB_DP=static: warp w of the DP grid handles segment w
   unsigned dp_grid = 148 * 8;     // persistent DP grid: every block that fits on the device
-  bool part_small = false;        // SMB_PART=small: four 52 KB k_part_sort CTAs per SM instead of two 105 KB ones
   bool part_sort = true;          // SMB_SORT=entry: always the one-CTA-per-entry sort (k_seg_sort)
   bool seg_sort = true;           // per-entry shared-memory sort; SMB_SORT=global forces the radix sort
-  uint32_t search_grab = 0;       // SMB_GRAB=n: queries per grab of the search work counter (0 = default)
-  bool sort_small = false;        // SMB_SORT=small: two 100 KB sort CTAs per SM instead of one 200 KB CTA
   cudaStream_t stream_cp = nullptr;  // smb_map_reads: upload slices (copy + K1 filter) run here, under the mapping
   std::vector<cudaEvent_t> slice_events;
   size_t upload_slice_bytes = 64u << 20;  // SMB_UPLOAD_SLICE_MB=n
@@ -387,62 +379,46 @@ static int launch_search(smb_ctx *ctx, SearchArgs sa, uint32_t nq_max, cudaStrea
     return SMB_OK;
   }
   CK(w.ovf_list.ensure(nq_max));
+  if (!STAGE) CK(w.entry_info.ensure(sa.B));
   if (nq_max < ctx->sort_queries_min) {
     // a small batch (a read-until round) fits the caches whatever the order: the queries keep their
     // natural order (consecutive queries share an entry, so a flush serves several of them) and the
     // round saves the key kernel and the five launches of the radix sort
     if (!STAGE) {
-      CK(w.entry_info.ensure(sa.B));
       k_entry_info<<<(sa.B + 255) / 256, 256, 0, s>>>(sa.feat_row, sa.entry_slot, sa.slots, sa.B, w.entry_info.p);
       LAUNCH_CHECK();
     }
     sa.order = nullptr;
-    sa.stage_cap = ctx->stage_big ? lean_stage_cap(ctx->ix.smem_bytes) : (uint32_t)kLeanStage;
     sa.nq_cap = 0xFFFFFFFFu;
-    sa.entry_info = w.entry_info.p;
-    sa.front_cap = std::min<uint32_t>(std::max<uint32_t>(ctx->front_cap, 72u), (uint32_t)kFrontCap);
-    sa.ovf_list = w.ovf_list.p;
-    sa.work = &ctx->d_ctr->work;
-    sa.grab = ctx->search_grab;
-    k_search_lean<STAGE><<<ctx->n_sm, kLeanWarps * 32, lean_smem(ctx->ix.smem_bytes, sa.stage_cap), s>>>(ctx->ix, sa);
-    LAUNCH_CHECK();
-    sa.qlist = w.ovf_list.p;
-    sa.qlist_n = &ctx->d_ctr->n_overflow;
-    sa.work = &ctx->d_ctr->work2;
-    sa.grab = 0;
-    k_radius_search<STAGE><<<STAGE ? search_grid<true>(ctx) : ctx->search_grid_main, kSearchWarps * 32, gsm, s>>>(ctx->ix, sa);
-    LAUNCH_CHECK();
-    return SMB_OK;
-  }
-  CK(w.qkey_a.ensure(nq_max));
-  CK(w.qkey_b.ensure(nq_max));
-  CK(w.qpay_a.ensure(nq_max));
-  CK(w.qpay_b.ensure(nq_max));
-  if (STAGE) {
-    k_query_keys_stage<<<(nq_max + 255) / 256, 256, 0, s>>>(sa.features, nq_max, ctx->ix.vmin, ctx->ix.inv_span,
-                                                            w.qkey_a.p, w.qpay_a.p);
   } else {
-    CK(w.entry_info.ensure(sa.B));
-    // entries without queries write nothing; the sort only looks at the first q_off[B] keys,
-    // but it is sized on the host: pad the tail with the largest key so it stays at the end
-    CK(cudaMemsetAsync(w.qkey_a.p, 0xFF, (size_t)nq_max * sizeof(uint32_t), s));
-    k_query_keys<<<sa.B, 128, 0, s>>>(sa.features, sa.feat_row, sa.q_off, sa.entry_slot, sa.slots, sa.B, sa.step,
-                                      ctx->ix.vmin, ctx->ix.inv_span, w.qkey_a.p, w.qpay_a.p, w.entry_info.p, nq_max);
+    CK(w.qkey_a.ensure(nq_max));
+    CK(w.qkey_b.ensure(nq_max));
+    CK(w.qpay_a.ensure(nq_max));
+    CK(w.qpay_b.ensure(nq_max));
+    if (STAGE) {
+      k_query_keys_stage<<<(nq_max + 255) / 256, 256, 0, s>>>(sa.features, nq_max, ctx->ix.vmin, ctx->ix.inv_span,
+                                                              w.qkey_a.p, w.qpay_a.p);
+    } else {
+      // entries without queries write nothing; the sort only looks at the first q_off[B] keys,
+      // but it is sized on the host: pad the tail with the largest key so it stays at the end
+      CK(cudaMemsetAsync(w.qkey_a.p, 0xFF, (size_t)nq_max * sizeof(uint32_t), s));
+      k_query_keys<<<sa.B, 128, 0, s>>>(sa.features, sa.feat_row, sa.q_off, sa.entry_slot, sa.slots, sa.B, sa.step,
+                                        ctx->ix.vmin, ctx->ix.inv_span, w.qkey_a.p, w.qpay_a.p, w.entry_info.p, nq_max);
+    }
+    LAUNCH_CHECK();
+    size_t tb = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, tb, w.qkey_a.p, w.qkey_b.p, w.qpay_a.p, w.qpay_b.p, (int)nq_max, 0, 24, s);
+    CK(w.qsort_temp.ensure(tb));
+    CK(cub::DeviceRadixSort::SortPairs(w.qsort_temp.p, tb, w.qkey_a.p, w.qkey_b.p, w.qpay_a.p, w.qpay_b.p, (int)nq_max,
+                                       0, 24, s));
+    ctx->stats.launches += 5;
+    sa.order = w.qpay_b.p;
   }
-  LAUNCH_CHECK();
-  size_t tb = 0;
-  cub::DeviceRadixSort::SortPairs(nullptr, tb, w.qkey_a.p, w.qkey_b.p, w.qpay_a.p, w.qpay_b.p, (int)nq_max, 0, 24, s);
-  CK(w.qsort_temp.ensure(tb));
-  CK(cub::DeviceRadixSort::SortPairs(w.qsort_temp.p, tb, w.qkey_a.p, w.qkey_b.p, w.qpay_a.p, w.qpay_b.p, (int)nq_max,
-                                     0, 24, s));
-  ctx->stats.launches += 5;
-  sa.order = w.qpay_b.p;
-  sa.stage_cap = ctx->stage_big ? lean_stage_cap(ctx->ix.smem_bytes) : (uint32_t)kLeanStage;
+  sa.stage_cap = lean_stage_cap(ctx->ix.smem_bytes);
   sa.entry_info = w.entry_info.p;
   sa.front_cap = std::min<uint32_t>(std::max<uint32_t>(ctx->front_cap, 72u), (uint32_t)kFrontCap);
   sa.ovf_list = w.ovf_list.p;
   sa.work = &ctx->d_ctr->work;
-  sa.grab = ctx->search_grab;
   k_search_lean<STAGE><<<ctx->n_sm, kLeanWarps * 32, lean_smem(ctx->ix.smem_bytes, sa.stage_cap), s>>>(ctx->ix, sa);
   LAUNCH_CHECK();
   // the queries whose frontier outgrew the lean kernel's slots (none, mostly: the launch then
@@ -450,7 +426,6 @@ static int launch_search(smb_ctx *ctx, SearchArgs sa, uint32_t nq_max, cudaStrea
   sa.qlist = w.ovf_list.p;
   sa.qlist_n = &ctx->d_ctr->n_overflow;
   sa.work = &ctx->d_ctr->work2;
-  sa.grab = 0;
   k_radius_search<STAGE><<<STAGE ? search_grid<true>(ctx) : ctx->search_grid_main, kSearchWarps * 32, gsm, s>>>(ctx->ix, sa);
   LAUNCH_CHECK();
   return SMB_OK;
@@ -462,7 +437,7 @@ struct IndexInput {
   const float *val;              // values the windows read (whole cloud, or a shard's runs)
   const uint64_t *pos;           // position of every window (whole cloud: of every point)
   const uint32_t *wsrc, *worig;  // shard: value index / whole-cloud index of each window (else null)
-  uint64_t W;                    // windows
+  uint64_t W;                    // windows, >= 1 (a rank that owns none passes one padding window)
   size_t n_points;               // points of the whole cloud
   float vmin, vmax;
   uint32_t max_tpos, max_bucket;
@@ -605,14 +580,14 @@ static int build_index_core(smb_ctx *ctx, IndexInput &in) {
   DevBuf<uint64_t> code_a, code_b;
   DevBuf<uint32_t> w_a, w_b;
   DevBuf<unsigned char> tmp;
-  CK(code_a.ensure(W));
-  CK(code_b.ensure(W));
-  CK(w_a.ensure(W));
-  CK(w_b.ensure(W));
   DevBuf<uint32_t> ext_min, ext_max;
-  const uint32_t *d_order = nullptr;
-  if (ctx->index_kd && W > (uint64_t)kLeaf) {
+  const uint32_t *d_order = nullptr;  // null: the windows' own order (one leaf holds them all)
+  if (W > (uint64_t)kLeaf) {
     // aligned KD order (k_index.cuh): one pass per power-of-two segment size, top down
+    CK(code_a.ensure(W));
+    CK(code_b.ensure(W));
+    CK(w_a.ensure(W));
+    CK(w_b.ensure(W));
     int log2s = 4;
     while ((1ull << log2s) < W) ++log2s;
     const unsigned blocks = (unsigned)((W + kKdThreads - 1) / kKdThreads);
@@ -641,15 +616,6 @@ static int build_index_core(smb_ctx *ctx, IndexInput &in) {
       ctx->stats.launches += 9;
     }
     d_order = ia;
-  } else {
-    k_morton<<<(unsigned)((W + 255) / 256), 256, 0, s>>>(d_val, W, vmin, 1.0f / span, code_a.p, w_a.p, d_wsrc);
-    LAUNCH_CHECK();
-    size_t tb = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, tb, code_a.p, code_b.p, w_a.p, w_b.p, (uint64_t)W, 0, 60, s);
-    CK(tmp.ensure(tb));
-    CK(cub::DeviceRadixSort::SortPairs(tmp.p, tb, code_a.p, code_b.p, w_a.p, w_b.p, (uint64_t)W, 0, 60, s));
-    ctx->stats.launches += 8;
-    d_order = w_b.p;
   }
   CK(ctx->leaves.ensure((size_t)n_leaves * kLeafRec));
   CK(ctx->leaf_widx.ensure((size_t)n_leaves * kLeaf));
@@ -956,13 +922,13 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   int mode = std::max(*sort_mode, !ctx->seg_sort ? (int)SORT_GLOBAL : (!ctx->part_sort ? (int)SORT_SEG : (int)SORT_PART));
   const bool want_seg = mode != SORT_GLOBAL;
   // parts per entry (k_sort.cuh): equal coordinate ranges sized so that a part of an average
-  // entry fills part_fill (70 %) of one k_part_sort CTA; more than kMaxParts -> one list, k_seg_sort
+  // entry fills kPartFill (70 %) of one k_part_sort CTA; more than kMaxParts -> one list, k_seg_sort
+  constexpr double kPartFill = 0.70;
   uint32_t n_parts = 1;
   uint64_t span = std::max<uint64_t>(ctx->g_total, 1);
-  const int part_cap = ctx->part_small ? kPartSortCapSmall : kPartSortCap;
   if (mode == SORT_PART) {
     const double per_coord = std::max(ctx->est_anchors_per_chunk, 1.0) / (double)std::max<uint64_t>(ctx->g_total, 1);
-    const double want = ctx->part_fill * (double)part_cap / per_coord;
+    const double want = kPartFill * (double)kPartSortCap / per_coord;
     if (want < (double)ctx->g_total) {
       const uint64_t sp2 = std::max<uint64_t>((uint64_t)want, 1);
       const uint64_t np = (ctx->g_total + sp2 - 1) / sp2;
@@ -1021,7 +987,6 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   sa.n_parts = n_parts;
   sa.inv_span = inv_span;
   sa.bucket_base = ctx->bucket_base.p;
-  sa.grab = ctx->search_grab;
   sa.n_buckets = ctx->max_bucket + 1u;
   // query-order buffers are sized from a running estimate (the exact count is on the device)
   const uint32_t q_per_chunk_max = (uint32_t)(kFeatCap - kDim) / (uint32_t)prm.step_size;
@@ -1066,8 +1031,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     }
     if (ctx->h_ctl[0] > 0.0) return 1;  // nothing has been committed to the slots yet
   }
-  k_step_check<<<1, 1, 0, s>>>(ctx->d_ctr, cap, mode, 8u * (unsigned)part_cap,
-                               8ull * (unsigned)(ctx->sort_small ? kSortCapSmall : kSortCapBig), n_parts);
+  k_step_check<<<1, 1, 0, s>>>(ctx->d_ctr, cap, mode, 8u * (unsigned)kPartSortCap, 8ull * (unsigned)kSortCapBig, n_parts);
   LAUNCH_CHECK();
 
   // ---- sort by (entry, bucket, target, query)
@@ -1097,10 +1061,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     ps.bucket_base = ctx->bucket_base.p;
     ps.n_buckets = ctx->max_bucket + 1u;
     ps.ctr = ctx->d_ctr;
-    if (ctx->part_small)
-      k_part_sort<kPartSortCapSmall, 256, 2304><<<(unsigned)n_lists, 256, part_sort_smem_bytes(kPartSortCapSmall, 2304), s>>>(ps);
-    else
-      k_part_sort<kPartSortCap, 512, 4096><<<(unsigned)n_lists, 512, part_sort_smem_bytes(kPartSortCap, 4096), s>>>(ps);
+    k_part_sort<kPartSortCap, 512, 4096><<<(unsigned)n_lists, 512, part_sort_smem_bytes(kPartSortCap, 4096), s>>>(ps);
     LAUNCH_CHECK();
   } else if (mode == SORT_SEG) {
     // one CTA per entry working through the entry in several passes
@@ -1119,10 +1080,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     ss.gshift = ctx->gshift;
     ss.n_coarse = ctx->n_coarse;
     ss.ctr = ctx->d_ctr;
-    if (ctx->sort_small)
-      k_seg_sort<kSortCapSmall, 512, 4096><<<B, 512, sort_smem_bytes(kSortCapSmall, 4096), s>>>(ss);
-    else
-      k_seg_sort<kSortCapBig, 1024, 8192><<<B, 1024, sort_smem_bytes(kSortCapBig, 8192), s>>>(ss);
+    k_seg_sort<kSortCapBig, 1024, 8192><<<B, 1024, sort_smem_bytes(kSortCapBig, 8192), s>>>(ss);
     LAUNCH_CHECK();
   } else {
     // radix sort on (entry, bucket, target) only; k_fix_ties orders equal-target runs by query.
@@ -1153,7 +1111,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   ca.coef = w.coef.p;
   ca.pred = w.pred.p;
   ca.n_slots = (uint32_t)n_slots64;
-  ca.seg_qmin = ctx->prep_bound ? w.seg_qmin.p : nullptr;
+  ca.seg_qmin = w.seg_qmin.p;
   CK(w.seg.ensure(ca.n_slots));
   CK(w.seg_max.ensure(ca.n_slots));
   ca.seg = w.seg.p;
@@ -1180,10 +1138,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   }
   {
     const unsigned dp_blocks = (unsigned)(((uint64_t)ca.n_slots * 32 + kDpThreads - 1) / kDpThreads);
-    if (ctx->dp_dynamic)
-      k_chain_dp<<<std::min(dp_blocks, ctx->dp_grid), kDpThreads, 0, s>>>(ca, 1);
-    else
-      k_chain_dp<<<dp_blocks, kDpThreads, 0, s>>>(ca, 0);
+    k_chain_dp<<<std::min(dp_blocks, ctx->dp_grid), kDpThreads, 0, s>>>(ca);
     LAUNCH_CHECK();
   }
   SelectArgs se{};
@@ -1530,38 +1485,23 @@ static void make_row(const smb_ctx *ctx, const SlotState &st, uint32_t read_len,
 static bool apply_option(smb_ctx *ctx, const char *name_in, const char *value) {
   std::string name(name_in);
   for (char &c : name) c = (char)toupper((unsigned char)c);
-  if (name == "SORT") {  // part (default) | entry | small | global
+  if (name == "SORT") {  // part (default) | entry | global
     ctx->seg_sort = strcmp(value, "global") != 0;
-    ctx->sort_small = strcmp(value, "small") == 0;
-    ctx->part_sort = strcmp(value, "entry") != 0 && !ctx->sort_small && ctx->seg_sort;
+    ctx->part_sort = strcmp(value, "entry") != 0 && ctx->seg_sort;
   } else if (name == "SEARCH") {  // lean (default) | general
     ctx->search_lean = strcmp(value, "general") != 0;
   } else if (name == "FRONT_CAP") {
     ctx->front_cap = (uint32_t)std::max(atoi(value), 0);
   } else if (name == "RUNS_CAP") {
     ctx->runs_cap_min = (uint32_t)std::max(atoi(value), 0);
-  } else if (name == "GRAB") {
-    ctx->search_grab = (uint32_t)std::max(atoi(value), 0);
-  } else if (name == "PART_FILL") {
-    ctx->part_fill = atof(value);
-  } else if (name == "PART") {
-    ctx->part_small = strcmp(value, "small") == 0;
-  } else if (name == "DP") {
-    ctx->dp_dynamic = strcmp(value, "static") != 0;
   } else if (name == "CLOUD_TILE") {  // takes effect at the next device cloud build
     ctx->cloud_tile = (uint32_t)std::min(std::max(atoi(value), 1), 1 << 30);
-  } else if (name == "INDEX") {  // kd (default) | morton; takes effect at the next index build
-    ctx->index_kd = strcmp(value, "morton") != 0;
   } else if (name == "DP_TILES") {
     ctx->dp_pass_max_entries = (uint32_t)std::max(atoi(value), 0);
   } else if (name == "SORT_QUERIES_MIN") {
     ctx->sort_queries_min = (uint32_t)std::max(atoi(value), 0);
-  } else if (name == "STAGE") {
-    ctx->stage_big = strcmp(value, "small") != 0;
   } else if (name == "PIPELINE") {
     ctx->pipeline_mode = strcmp(value, "on") == 0 ? 1 : (strcmp(value, "off") == 0 ? 2 : 0);
-  } else if (name == "PREP_BOUND") {
-    ctx->prep_bound = atoi(value) != 0;
   } else if (name == "PREP_ROUNDS") {
     ctx->prep_rounds = std::min(std::max(atoi(value), 0), 200);
   } else if (name == "DP_PASSES") {
@@ -1637,9 +1577,7 @@ int smb_create(smb_ctx **out, int device) {
     if ((e = cudaEventCreate(&ev)) != cudaSuccess) return bail("cudaEventCreate", e);
   // the per-entry sort keeps a whole part of an entry in shared memory (200 KB of the 227 KB)
   if ((e = cudaFuncSetAttribute(k_seg_sort<kSortCapBig, 1024, 8192>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)sort_smem_bytes(kSortCapBig, 8192))) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(k_seg_sort<kSortCapSmall, 512, 4096>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)sort_smem_bytes(kSortCapSmall, 4096))) != cudaSuccess)
+                                (int)sort_smem_bytes(kSortCapBig, 8192))) != cudaSuccess)
     return bail("cudaFuncSetAttribute(k_seg_sort)", e);
   // the general search kernel keeps one stack per index level in shared memory: from 7 levels on
   // (> 16.7 M points, i.e. references beyond ~8 Mbp) a CTA needs more than the default 48 KB; the
@@ -1659,13 +1597,10 @@ int smb_create(smb_ctx **out, int device) {
     ctx->n_sm = (unsigned)n_sm;
   }
   if ((e = cudaFuncSetAttribute(k_part_sort<kPartSortCap, 512, 4096>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)part_sort_smem_bytes(kPartSortCap, 4096))) != cudaSuccess ||
-      (e = cudaFuncSetAttribute(k_part_sort<kPartSortCapSmall, 256, 2304>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)part_sort_smem_bytes(kPartSortCapSmall, 2304))) != cudaSuccess)
+                                (int)part_sort_smem_bytes(kPartSortCap, 4096))) != cudaSuccess)
     return bail("cudaFuncSetAttribute(k_part_sort)", e);
-  for (const char *name : {"SORT", "SEARCH", "FRONT_CAP", "RUNS_CAP", "GRAB", "PART_FILL", "PART", "DP", "DP_PASSES",
-                           "DP_TILES", "SORT_QUERIES_MIN", "INDEX", "PREP_ROUNDS", "PREP_BOUND", "PIPELINE", "STAGE", "EVENTS_OVERLAP", "EVENTS", "UPLOAD_SLICE_MB",
-                           "CLOUD_TILE"})
+  for (const char *name : {"SORT", "SEARCH", "FRONT_CAP", "RUNS_CAP", "DP_PASSES", "DP_TILES", "SORT_QUERIES_MIN",
+                           "PREP_ROUNDS", "PIPELINE", "EVENTS_OVERLAP", "EVENTS", "UPLOAD_SLICE_MB", "CLOUD_TILE"})
     if (const char *env = getenv((std::string("SMB_") + name).c_str())) apply_option(ctx, name, env);
   {
     int per_sm = 0, n_sm = 148;

@@ -153,15 +153,13 @@ def test_part_equals_host(dev, host, genomes, world):
             assert np.array_equal(bits(got["val"]), bits(exp["val"])), (name, rank)
 
 
-@pytest.fixture(scope="module", params=["kd", "morton"])
-def golden_pair(request, host, model, golden):
+@pytest.fixture(scope="module")
+def golden_pair(host, model, golden):
     """(index from the host cloud, index built on the device) over the golden genome."""
     from sigmap_b200.mapper import Mapper
     g = golden.genome(host)
     pos, val = host.build_point_cloud(g, model[0])
     a, b = Mapper(0), Mapper(0)
-    for m in (a, b):
-        m.set_option("index", request.param)
     a.set_index(pos, val)
     a.set_contigs(g.lengths)
     b.build_index(g, model[0])
@@ -186,19 +184,15 @@ def test_index_rows_equal_host_index(golden_pair, golden, host):
     assert b.build_stats()["ms_index"] > 0
 
 
-@pytest.mark.parametrize("index", ["kd", "morton"])
 @pytest.mark.parametrize("world", [2, 3])
-def test_sharded_build_rows_equal_unsharded(multi, model, world, index):
+def test_sharded_build_rows_equal_unsharded(multi, model, world):
     from sigmap_b200 import shard
     from sigmap_b200.mapper import Mapper, default_params, full_read_params
     whole = Mapper(0)
     g = shard.ContigShardGroup([0] * world)
     try:
-        whole.set_option("index", index)
         whole.set_index(multi.pos, multi.val)
         whole.set_contigs(multi.ref.lengths)
-        for m in g.mappers:
-            m.set_option("index", index)
         g.build_index(multi.ref, model[0])
         assert sorted(set(g.owner.tolist())) == list(range(world))
         for prm in (default_params(), full_read_params()):

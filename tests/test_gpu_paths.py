@@ -26,7 +26,6 @@ def _lines(m, ds, params=None):
 PATHS = [
     # option, value, what must be visible in the stats of the run
     ("sort", "entry", lambda st: st["seg_sort_steps"] > 0 and st["part_sort_steps"] == 0),
-    ("sort", "small", lambda st: st["seg_sort_steps"] > 0 and st["part_sort_steps"] == 0),
     ("sort", "global", lambda st: st["seg_sort_steps"] == 0),
     ("runs_cap", "8", lambda st: st["part_sort_steps"] < st["steps"]),   # run tables overflow -> radix sort
     ("search", "general", lambda st: st["overflow_queries"] == st["queries"]),
@@ -38,21 +37,16 @@ PATHS = [
     ("prep_rounds", "0", lambda st: st["pending"] == st["linked"] > 0),   # every linked anchor walked by k_chain_dp
     ("prep_rounds", "2", lambda st: 0 < st["pending"] < st["linked"]),
     ("prep_rounds", "5", lambda st: 0 < st["pending"] < st["linked"]),
-    ("prep_bound", "0", lambda st: True),          # link test over the whole 5 000-position range
     ("pipeline", "on", lambda st: True),           # wave-pipelined ticks (one wave on this small input)
     ("pipeline", "off", lambda st: True),
-    ("stage", "small", lambda st: True),           # 128 staged hits per warp whatever the room
-    ("grab", "1", lambda st: True),
-    ("dp", "static", lambda st: True),
     ("dp_passes", "0", lambda st: True),   # the cooperative in-order DP path settles everything
     ("dp_passes", "3", lambda st: True),
     ("events", "thread", lambda st: True),
     ("events", "warp", lambda st: True),
     ("events_overlap", "0", lambda st: True),
-    ("part", "small", lambda st: st["part_sort_steps"] > 0),
 ]
-RESET = {"stage": "big", "pipeline": "auto", "prep_bound": "1", "prep_rounds": "1", "sort_queries_min": "200000", "dp_tiles": "4096", "sort": "part", "runs_cap": "0", "search": "lean", "front_cap": "384", "grab": "0", "dp": "dynamic",
-         "dp_passes": "1", "events": "auto", "events_overlap": "1", "part": "big"}
+RESET = {"pipeline": "auto", "prep_rounds": "1", "sort_queries_min": "200000", "dp_tiles": "4096", "sort": "part", "runs_cap": "0", "search": "lean", "front_cap": "384",
+         "dp_passes": "1", "events": "auto", "events_overlap": "1"}
 
 
 def test_every_shipped_path_gives_the_default_rows(mapper, small):
@@ -75,8 +69,10 @@ def test_every_shipped_path_gives_the_default_rows(mapper, small):
                 assert st["linked"] == linked[mode], f"{name}={value} ({mode}): linked anchors differ"
         finally:
             mapper.set_option(name, RESET[name])
-    with pytest.raises(Exception):
-        mapper.set_option("no_such_option", "1")
+    # unknown names, and the switches of paths that no longer ship, are rejected
+    for name in ("no_such_option", "index", "stage", "prep_bound", "grab", "part_fill", "part", "dp"):
+        with pytest.raises(Exception):
+            mapper.set_option(name, "1")
     assert _lines(mapper, small) == base["default"]
 
 
@@ -113,7 +109,10 @@ def test_wave_pipelined_ticks_give_identical_rows(mapper, small):
 
 def test_radius_search_paths_agree_with_the_oracle(mapper, port, small):
     """Hit sets (index + d2 bits) of the lean kernel, of the general kernel, and of the two
-    together (a frontier limit that sends a share of the queries to the general kernel)."""
+    together (a frontier limit that sends a share of the queries to the general kernel), on the
+    index of `small` and on indexes of 6, 9 and 13 points (1 to 8 windows: one leaf, which keeps
+    the windows' own order)."""
+    from sigmap_b200.mapper import Mapper
     rng = np.random.default_rng(21)
     qs = []
     for r in range(8):
@@ -122,45 +121,36 @@ def test_radius_search_paths_agree_with_the_oracle(mapper, port, small):
             qs.append(f[p:p + 6])
     q = np.stack(qs)
     q = q[rng.permutation(len(q))]
-    for radius in (0.08, 0.3):
-        exp = [port.radius_search(small.val, x, radius=radius) for x in q[:160]]
+
+    def agree(m, val, q, radius):  # -> hits
+        exp = [port.radius_search(val, x, radius=radius) for x in q]
         for name, value in (("search", "lean"), ("search", "general"), ("front_cap", "72"),
                             ("sort_queries_min", "0")):
-            mapper.set_option(name, value)
+            m.set_option(name, value)
             try:
-                off, idx, d2 = mapper.radiusSearch(q[:160], radius=radius, cap=1 << 24)
+                off, idx, d2 = m.radiusSearch(q, radius=radius, cap=1 << 24)
             finally:
-                mapper.set_option(name, RESET[name])
+                m.set_option(name, RESET[name])
             for k, (ei, ed) in enumerate(exp):
                 gi, gd = idx[off[k]:off[k + 1]], d2[off[k]:off[k + 1]]
                 assert np.array_equal(gi, ei), f"{name}={value} r={radius} query {k}: hit set differs"
                 assert np.array_equal(bits(gd), bits(ed))
-    assert sum(len(e[0]) for e in exp) > 10000  # radius 0.3: dense enough to matter
+        return sum(len(e[0]) for e in exp)
 
-
-def test_point_order_of_the_index_changes_nothing(mapper, port, small):
-    """The index keeps its points in the aligned KD order by default and in Morton order with
-    option index=morton (read when the index is built): same hit sets and d2 bits against the
-    oracle, same PAF rows."""
-    from sigmap_b200.mapper import Mapper
-    f = port.generate_events(small.pa(port, 3)[:4000])
-    q = np.stack([f[p:p + 6] for p in range(2, len(f) - 5, 2)])[:120]
-    exp = [port.radius_search(small.val, x, radius=0.08) for x in q]
-    base = _lines(mapper, small)
-    m = Mapper(0)
+    for radius in (0.08, 0.3):
+        hits = agree(mapper, small.val, q[:160], radius)
+    assert hits > 10000  # radius 0.3: dense enough to matter
+    tiny = Mapper(0)
     try:
-        m.set_option("index", "morton")
-        m.set_index(small.pos, small.val)
-        m.set_contigs(small.ref.lengths)
-        for mm in (mapper, m):
-            off, idx, d2 = mm.radiusSearch(q, radius=0.08, cap=1 << 24)
-            for k, (ei, ed) in enumerate(exp):
-                gi, gd = idx[off[k]:off[k + 1]], d2[off[k]:off[k + 1]]
-                assert np.array_equal(gi, ei), f"query {k}: hit set differs"
-                assert np.array_equal(bits(gd), bits(ed))
-        assert _lines(m, small) == base
+        for n in (6, 9, 13):
+            val = small.val[:n]
+            tiny.set_index(small.pos[:n], val)
+            w = np.stack([val[i:i + 6] for i in range(n - 5)])  # every window finds itself at d2 = 0
+            tq = np.concatenate([w, w + rng.normal(0.0, 0.1, w.shape).astype(np.float32)])
+            for radius in (0.08, 0.3):
+                assert agree(tiny, val, tq, radius) >= len(w)
     finally:
-        m.close()
+        tiny.close()
 
 
 def test_hit_cap_5000(mapper, port, small):
