@@ -18,10 +18,12 @@
 //                   position is kept
 //   k_cloud_assume / k_cloud_fix / k_cloud_chain   fix-up to the true incoming state (DESIGN.md)
 //   k_cloud_scatter warp per tile: pos / val of the kept positions at the scanned tile offsets
-// and, for one rank's part of a contig-sharded index, k_part_count / k_part_emit.
+// and, for one rank's part of a contig-sharded index, k_part_count / k_part_emit; for the index build
+// of any cloud, k_cloud_extent / k_bucket_span.
 #pragma once
 #include <cstdint>
-#include <cstring>
+
+#include "sb_device.cuh"
 
 namespace cloud {
 
@@ -511,35 +513,20 @@ __global__ void k_part_emit(const uint64_t *pos, const float *val, uint64_t n, c
   }
 }
 
-// vmin / vmax of the values, largest target, and 1 + largest target per bucket (contig<<1 | strand)
-// of the positions: what build_index needs besides the arrays themselves.
-__device__ __forceinline__ uint32_t val_ord(float f) {  // order-preserving u32 image (as k_index.cuh)
-  const uint32_t b = __float_as_uint(f);
-  return b ^ ((b >> 31) ? 0xFFFFFFFFu : 0x80000000u);
-}
-inline float ord_val(uint32_t o) {  // its inverse, on the host
-  const uint32_t b = o ^ ((o >> 31) ? 0x80000000u : 0xFFFFFFFFu);
-  float f;
-  memcpy(&f, &b, 4);
-  return f;
-}
+// What the index build needs besides the arrays themselves: vmin / vmax of the values, the
+// largest target and the largest bucket (contig << 1 | strand) of the positions ...
 struct CloudExtent {
   unsigned int vmin_ord, vmax_ord, max_tpos, max_bucket;
 };
-__global__ void k_cloud_extent(const uint64_t *pos, const float *val, uint64_t n, CloudExtent *ext,
-                               unsigned long long *bucket_span) {
+__global__ void k_cloud_extent(const uint64_t *pos, const float *val, uint64_t n, CloudExtent *ext) {
   unsigned int lo = 0xFFFFFFFFu, hi = 0, tp = 0, bk = 0;
   for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
-    const uint32_t o = val_ord(val[i]);
+    const uint32_t o = sb::f2ord(val[i]);
     lo = min(lo, o);
     hi = max(hi, o);
     const uint64_t P = pos[i];
-    const uint32_t t = (uint32_t)(P >> 1), b = (uint32_t)(((P >> 33) << 1) | (P & 1));
-    tp = max(tp, t);
-    bk = max(bk, b);
-    // points come ordered by bucket and target: the last point of a bucket holds its largest target
-    if (i + 1 == n || (pos[i + 1] >> 1 >> 32) != (P >> 1 >> 32) || (pos[i + 1] & 1) != (P & 1))
-      atomicMax(bucket_span + b, (unsigned long long)t + 1);
+    tp = max(tp, (uint32_t)(P >> 1));
+    bk = max(bk, (uint32_t)(((P >> 33) << 1) | (P & 1)));
   }
   for (int o = 16; o; o >>= 1) {
     lo = min(lo, __shfl_xor_sync(0xFFFFFFFFu, lo, o));
@@ -552,6 +539,23 @@ __global__ void k_cloud_extent(const uint64_t *pos, const float *val, uint64_t n
     atomicMax(&ext->vmax_ord, hi);
     atomicMax(&ext->max_tpos, tp);
     atomicMax(&ext->max_bucket, bk);
+  }
+}
+
+// ... and 1 + the largest target of every bucket (the table has a slot for every bucket of the
+// positions).  Each run of non-decreasing targets inside a bucket gives its last target, so any
+// point order yields the exact maximum; a cloud ordered by bucket and target, as every cloud
+// built by this library is, takes one atomic per bucket.
+__global__ void k_bucket_span(const uint64_t *pos, uint64_t n, unsigned long long *bucket_span) {
+  for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t P = pos[i];
+    const uint32_t t = (uint32_t)(P >> 1), b = (uint32_t)(((P >> 33) << 1) | (P & 1));
+    bool last = i + 1 == n;
+    if (!last) {
+      const uint64_t Q = pos[i + 1];
+      last = (uint32_t)(((Q >> 33) << 1) | (Q & 1)) != b || (uint32_t)(Q >> 1) < t;
+    }
+    if (last) atomicMax(bucket_span + b, (unsigned long long)t + 1);
   }
 }
 

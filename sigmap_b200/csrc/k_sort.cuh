@@ -35,7 +35,6 @@ constexpr int kRunsCap = 512;        // run records a k_part_sort CTA holds in s
 constexpr int kSortCapBig = 10240;
 // k_part_sort runs as <5120, 512, 4096>: two 105 KB CTAs per SM
 constexpr int kPartSortCap = 5120;   // anchors of one (entry, part) held by a k_part_sort CTA
-constexpr int kCoarseBins = 256;
 constexpr int kSmallBin = 24;        // bins up to this size: insertion sort by one thread
 constexpr int kBigBinCap = 512;      // dense bins queued for the warp-wide rank sort
 

@@ -6,9 +6,11 @@
 #ifndef SB_DEVICE_CUH
 #define SB_DEVICE_CUH
 
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cstring>
 #include <string>
 #include <vector>
 
@@ -80,6 +82,7 @@ struct DevBuf {
 constexpr int kNodeRec = 3 * kFan;       // uint2 per node record
 constexpr int kLeafRec = 4 * kLeaf;      // uint2 per leaf record (24 values + 8 payload)
 constexpr uint32_t kTopSmemMax = 64u << 10;
+constexpr float kPadValue = 1.0e18f;  // padding points: never inside any ball
 struct IndexView {
   uint64_t n_points;    // N (point cloud size); windows W = N - 5
   uint64_t n_windows;
@@ -95,6 +98,28 @@ struct IndexView {
   const uint32_t *leaf_widx;  // [n_leaves*8] window index in the original cloud (parity hook only)
   float vmin, inv_span;       // Morton quantisation of the build: cell = (v - vmin) * inv_span
 };
+
+// one binary16 pair of a node record -> two floats
+__device__ __forceinline__ float2 unpack_h2(uint32_t v) {
+  return make_float2(__half2float(__ushort_as_half((unsigned short)(v & 0xFFFFu))),
+                     __half2float(__ushort_as_half((unsigned short)(v >> 16))));
+}
+
+// order-preserving u32 image of a float (index extent and KD order) and its inverse
+__device__ __forceinline__ uint32_t f2ord(float f) {
+  const uint32_t u = __float_as_uint(f);
+  return u ^ ((u >> 31) ? 0xFFFFFFFFu : 0x80000000u);
+}
+__host__ __device__ __forceinline__ float ord2f(uint32_t o) {
+  const uint32_t u = o ^ ((o >> 31) ? 0x80000000u : 0xFFFFFFFFu);
+#ifdef __CUDA_ARCH__
+  return __uint_as_float(u);
+#else
+  float f;
+  memcpy(&f, &u, 4);
+  return f;
+#endif
+}
 
 // per-step packing of the 64-bit sort key: entry | bucket | target | query
 struct KeyLayout {
@@ -176,6 +201,9 @@ constexpr unsigned int kAbortAnchors = 1u;  // more anchors than the step's buff
 constexpr unsigned int kAbortSort = 2u;     // the chosen sort path cannot take this step (run tables, dense part)
 constexpr unsigned int kAbortQueries = 4u;  // more queries than the order buffers hold
 constexpr unsigned int kAbortPool = 8u;     // carry pools too small for the surviving chains
+
+// The index build sets the shift that puts every g of the index below kCoarseBins (k_seg_sort).
+constexpr int kCoarseBins = 256;
 
 // Part of an entry that linear coordinate g = bucket_base[bucket] + target belongs to
 // (k_sort.cuh, k_part_sort).  Any function that is monotone in g gives contiguous parts; float

@@ -1,5 +1,6 @@
-// sb_engine.cu -- context, device index build, the batched pipeline step, the read scheduler
-// and the C ABI of include/sigmap_b200.h.
+// sb_engine.cu -- the context, the batched pipeline step, the read scheduler, streaming, the
+// stage hooks and the rest of the C ABI of include/sigmap_b200.h.  Index construction (every
+// smb_index_* and smb_point_cloud_* entry point) is in sb_index.cu; the context is in sb_ctx.cuh.
 //
 // Execution model (replaces the OpenMP taskloop of sigmap.cc:618-632): instead of one host
 // thread walking one read chunk by chunk, all still-active reads advance together in ROUNDS;
@@ -28,11 +29,7 @@
 #include "k_sort.cuh"
 #include "k_events.cuh"
 #include "k_index.cuh"
-#include "k_cloud.cuh"
-#include "sb_device.cuh"
-#include "sb_exchange.cuh"
-
-using namespace sb;
+#include "sb_ctx.cuh"
 
 static_assert(kCarryMaxParts == kMaxParts, "one part limit for every run producer");
 
@@ -123,9 +120,6 @@ __global__ void k_query_table(const uint32_t *__restrict__ n_features, uint32_t 
 
 __global__ void k_clear_error_bits(Counters *c, unsigned int bits) { c->error &= ~bits; }
 
-struct RoundInfo {
-  uint32_t stop, num_events, n_chains;
-};
 __global__ void k_gather_round(const SlotState *__restrict__ slots, const uint32_t *__restrict__ ids,
                                uint32_t n, RoundInfo *__restrict__ out) {
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -178,181 +172,13 @@ __global__ void k_count_by_query(const uint64_t *__restrict__ key, unsigned long
 
 }  // namespace sb
 
-// ------------------------------------------------------------------ context
-struct SlotSpace {
-  uint32_t n_slots = 0;
-  DevBuf<SlotState> slots;
-  DevBuf<ChainRec> pool_chain[2];
-  DevBuf<CarryAnchor> pool_anchor[2];
-  std::vector<uint32_t> h_events, h_nchains;  // host mirror, refreshed every round
-  uint32_t round = 0;
-};
-
-struct Workspace {
-  // per-entry
-  DevBuf<uint32_t> entry_slot, n_features, n_raw_events, n_queries, q_off, feat_row;
-  // queries in Morton order (lean search kernel) and the ones it leaves to the general kernel
-  DevBuf<uint32_t> qkey_a, qkey_b, qpay_a, qpay_b, ovf_list;
-  DevBuf<uint2> entry_info;
-  DevBuf<unsigned char> qsort_temp;
-  // event lookahead block of the offline path: features of chunks [r0, r1) of the active reads
-  // (two of them: the next block is computed on the event stream while this one is being mapped)
-  DevBuf<float> feat_cache[2];
-  DevBuf<uint32_t> nf_cache[2], nraw_cache[2];
-  int cache_cur = 0;
-  // chunk table of the lookahead blocks (the event stream's own copies)
-  DevBuf<uint64_t> blk_chunk_start;
-  DevBuf<float> blk_chunk_offset, blk_chunk_scale;
-  DevBuf<uint8_t> absent;
-  DevBuf<uint64_t> chunk_start;
-  DevBuf<float> chunk_offset, chunk_scale;
-  // events (transposed)
-  DevBuf<float> ps, pss, t1, t2, means, features;
-  // anchors
-  DevBuf<uint64_t> key_a, key_b;
-  DevBuf<float> dist_a, dist_b, score, coef;
-  DevBuf<uint32_t> pred, link_list, link_count, pend_count, seg_qmin;
-  DevBuf<uint16_t> pend_list;
-  DevBuf<SegRec> seg;
-  DevBuf<RunRec> runs;
-  DevBuf<uint32_t> run_count, entry_total, part_base;
-  DevBuf<unsigned char> cub_temp;
-  DevBuf<ChainTmp> chain_tmp;
-  DevBuf<PickRec> pick;
-  DevBuf<float> seg_max;
-  DevBuf<uint32_t> n_scratch;
-  // contig-sharded runs (sb_exchange.cuh)
-  DevBuf<CandRec> cand_list, cand_all;
-  DevBuf<unsigned long long> cand_counts;
-  DevBuf<double> ctl;
-  DevBuf<uint32_t> tags;
-  // round readback
-  DevBuf<uint32_t> ids;
-  DevBuf<RoundInfo> round_info;
-};
-
-struct smb_ctx {
-  int device = 0;
-  cudaStream_t stream = nullptr;
-  std::string err;
-  // index
-  bool has_index = false;
-  IndexView ix{};
-  DevBuf<uint2> leaves;           // 256-byte leaf records (values + {target, bucket})
-  DevBuf<uint2> nodes;            // every node level, top level first
-  DevBuf<uint32_t> leaf_widx;
-  uint32_t max_tpos = 0, max_bucket = 0;
-  unsigned search_grid_main = 148 * 4;   // general search kernel: every CTA that fits
-  unsigned n_sm = 148;
-  bool search_lean = true;        // SMB_SEARCH=general: every query through the general kernel
-  uint32_t front_cap = kFrontCap; // SMB_FRONT_CAP=n: frontier slots of the lean kernel (tests lower it)
-  uint32_t runs_cap_min = 0;      // SMB_RUNS_CAP=n: run records per (entry, part) list (0 = from the estimate)
-  DevBuf<uint64_t> bucket_base;   // linear coordinate of every bucket's target 0 (k_sort.cuh)
-  int gshift = 0;
-  uint32_t n_coarse = 1;
-  uint64_t g_total = 1;           // linear coordinates of the whole index (sum of the bucket spans)
-  int dp_passes = kDpFreePasses;  // SMB_DP_PASSES=n
-  int prep_rounds = kPrepRounds;  // SMB_PREP_ROUNDS=n: settle rounds inside k_chain_prep (0 = none)
-  uint32_t dp_pass_max_entries = kDpPassMaxEntries;  // SMB_DP_TILES=n: per-tile DP pass up to n chunks per step (0 = never)
-  int pipeline_mode = 0;          // SMB_PIPELINE=auto|on|off: wave-pipelined ticks (see map_uploaded_impl)
-  uint32_t cloud_tile = 16384;    // SMB_CLOUD_TILE=n: window starts per tile of the device cloud's point selection
-  smb_build_stats build_stats{};  // the last device cloud build (smb_index_build_stats)
-  unsigned char *h_cloud_stage = nullptr;  // pinned: two upload slices of the device cloud build
-  uint32_t sort_queries_min = 200000;  // SMB_SORT_QUERIES_MIN=n: batches with fewer queries keep their natural order
-  unsigned dp_grid = 148 * 8;     // persistent DP grid: every block that fits on the device
-  bool part_sort = true;          // SMB_SORT=entry: always the one-CTA-per-entry sort (k_seg_sort)
-  bool seg_sort = true;           // per-entry shared-memory sort; SMB_SORT=global forces the radix sort
-  cudaStream_t stream_cp = nullptr;  // smb_map_reads: upload slices (copy + K1 filter) run here, under the mapping
-  std::vector<cudaEvent_t> slice_events;
-  size_t upload_slice_bytes = 64u << 20;  // SMB_UPLOAD_SLICE_MB=n
-  uint32_t *h_kept_pinned = nullptr;      // kept length of every read, written by the device (pinned)
-  size_t h_kept_pinned_cap = 0;
-  cudaStream_t stream_ev = nullptr;  // lookahead event blocks run here, next to the mapping rounds
-  cudaEvent_t ev_blk_t0[2] = {}, ev_blk_t1[2] = {};
-  cudaEvent_t ev_cp[2] = {};         // first / last filter-only slice of a wave-pipelined call (copy stream)
-  bool ev_overlap = true;            // SMB_EVENTS_OVERLAP=0: compute every block when it is needed
-  double ev_survival_hint = 0.0;     // share of reads that went past their first chunk in the last call
-  uint32_t ev_warp_max = 2048;    // event batches up to this many chunks run warp-per-chunk in shared memory
-                                  // (SMB_EVENTS=thread: never, =warp: always)
-  std::vector<uint32_t> contig_len;
-  // uploaded reads
-  size_t n_reads = 0;
-  DevBuf<int16_t> raw, kept;
-  DevBuf<uint64_t> d_read_off, d_kept_off;
-  DevBuf<float> d_dig, d_range, d_offset;
-  DevBuf<uint32_t> d_kept_len;
-  std::vector<uint64_t> h_kept_off;
-  std::vector<uint32_t> h_kept_len;
-  std::vector<float> h_offset, h_scale;
-  std::vector<uint32_t> h_feat_row;
-  // work
-  Workspace ws;
-  SlotSpace map_slots;
-  Counters *d_ctr = nullptr;
-  Counters *h_ctr = nullptr;  // pinned
-  cudaEvent_t ev[8] = {};
-  cudaEvent_t timer[2] = {};
-  smb_stats stats{};
-  uint32_t max_batch_chunks = 32768;
-  uint64_t max_batch_anchors = 640ull << 20;  // x 32 B of sort/DP buffers = 20 GB of the 180 GB HBM
-  uint64_t last_cap = 0;
-  double est_anchors_per_chunk = 20000.0;
-  double est_queries_per_chunk = 260.0;
-  double runs_scale = 1.0;          // raised when a step overflowed its run tables
-  // contig-sharded index: the exchange backend (null = this context holds every contig)
-  std::unique_ptr<Exchange> ex;
-  bool index_sharded = false;  // this context holds only its own contigs (smb_index_set_points_sharded)
-  std::shared_ptr<LocalGroup> local_group;
-  double *h_ctl = nullptr;  // pinned, 4 doubles
-  bool group_at_limit = false;
-  // streaming
-  SlotSpace *stream_slots = nullptr;
-  smb_params stream_params{};
-  std::vector<std::vector<int16_t>> stream_pending;  // kept samples not yet forming a chunk
-  std::vector<float> stream_offset, stream_scale;
-  std::vector<uint32_t> stream_chunks, stream_kept;
-  // raw values kept by the (30, 200) pA filter form an interval [lo, hi] per channel (the
-  // conversion is monotone in the raw value); lo > hi: nothing kept; generic: test every sample
-  std::vector<int32_t> stream_lo, stream_hi;
-  std::vector<uint8_t> stream_generic;
-  int16_t *h_stream_stage = nullptr;  // pinned: this round's chunks, channel after channel
-  size_t h_stream_stage_cap = 0;
-  DevBuf<int16_t> d_stream_stage;
-};
-
 struct smb_batch {
   smb_ctx *ctx;
   SlotSpace sp;
 };
 
-#define CK(call)                                                                      \
-  do {                                                                                \
-    cudaError_t e_ = (call);                                                          \
-    if (e_ != cudaSuccess) {                                                          \
-      ctx->err = std::string(#call) + ": " + cudaGetErrorString(e_);                  \
-      return SMB_ERR_CUDA;                                                            \
-    }                                                                                 \
-  } while (0)
-
-#define LAUNCH_CHECK()                                                                \
-  do {                                                                                \
-    ctx->stats.launches++;                                                            \
-    cudaError_t e_ = cudaGetLastError();                                              \
-    if (e_ != cudaSuccess) {                                                          \
-      ctx->err = std::string("kernel launch: ") + cudaGetErrorString(e_);             \
-      return SMB_ERR_CUDA;                                                            \
-    }                                                                                 \
-  } while (0)
-
-static int fail(smb_ctx *ctx, int code, const std::string &msg) {
-  ctx->err = msg;
-  // a failed member must not leave its in-process shard peers waiting at a rendezvous
-  if (ctx->local_group) ctx->local_group->abort_all();
-  return code;
-}
-
 // persistent grid of the general search kernel: every CTA that fits on the device, no more
-static size_t search_smem(const smb_ctx *ctx) { return kSearchWarps * search_smem_per_warp(ctx->ix.n_levels); }
+static size_t search_smem(const smb_ctx *ctx) { return kSearchWarps * search_smem_per_warp(ctx->index.ix.n_levels); }
 
 template <bool STAGE>
 static unsigned search_grid(smb_ctx *ctx) {
@@ -361,6 +187,11 @@ static unsigned search_grid(smb_ctx *ctx) {
                                                     search_smem(ctx)) != cudaSuccess || n < 1)
     n = 4;
   return ctx->n_sm * (unsigned)n;
+}
+
+void index_installed(smb_ctx *ctx) {
+  ctx->search_grid_main = search_grid<false>(ctx);
+  ctx->has_index = true;
 }
 
 // The whole radius search of one batch on stream s: Morton keys of the queries -> radix sort ->
@@ -374,7 +205,7 @@ static int launch_search(smb_ctx *ctx, SearchArgs sa, uint32_t nq_max, cudaStrea
   const size_t gsm = search_smem(ctx);
   if (!ctx->search_lean || nq_max == 0) {
     sa.work = &ctx->d_ctr->work;
-    k_radius_search<STAGE><<<STAGE ? search_grid<true>(ctx) : ctx->search_grid_main, kSearchWarps * 32, gsm, s>>>(ctx->ix, sa);
+    k_radius_search<STAGE><<<STAGE ? search_grid<true>(ctx) : ctx->search_grid_main, kSearchWarps * 32, gsm, s>>>(ctx->index.ix, sa);
     LAUNCH_CHECK();
     return SMB_OK;
   }
@@ -396,14 +227,14 @@ static int launch_search(smb_ctx *ctx, SearchArgs sa, uint32_t nq_max, cudaStrea
     CK(w.qpay_a.ensure(nq_max));
     CK(w.qpay_b.ensure(nq_max));
     if (STAGE) {
-      k_query_keys_stage<<<(nq_max + 255) / 256, 256, 0, s>>>(sa.features, nq_max, ctx->ix.vmin, ctx->ix.inv_span,
+      k_query_keys_stage<<<(nq_max + 255) / 256, 256, 0, s>>>(sa.features, nq_max, ctx->index.ix.vmin, ctx->index.ix.inv_span,
                                                               w.qkey_a.p, w.qpay_a.p);
     } else {
       // entries without queries write nothing; the sort only looks at the first q_off[B] keys,
       // but it is sized on the host: pad the tail with the largest key so it stays at the end
       CK(cudaMemsetAsync(w.qkey_a.p, 0xFF, (size_t)nq_max * sizeof(uint32_t), s));
       k_query_keys<<<sa.B, 128, 0, s>>>(sa.features, sa.feat_row, sa.q_off, sa.entry_slot, sa.slots, sa.B, sa.step,
-                                        ctx->ix.vmin, ctx->ix.inv_span, w.qkey_a.p, w.qpay_a.p, w.entry_info.p, nq_max);
+                                        ctx->index.ix.vmin, ctx->index.ix.inv_span, w.qkey_a.p, w.qpay_a.p, w.entry_info.p, nq_max);
     }
     LAUNCH_CHECK();
     size_t tb = 0;
@@ -414,283 +245,20 @@ static int launch_search(smb_ctx *ctx, SearchArgs sa, uint32_t nq_max, cudaStrea
     ctx->stats.launches += 5;
     sa.order = w.qpay_b.p;
   }
-  sa.stage_cap = lean_stage_cap(ctx->ix.smem_bytes);
+  sa.stage_cap = lean_stage_cap(ctx->index.ix.smem_bytes);
   sa.entry_info = w.entry_info.p;
   sa.front_cap = std::min<uint32_t>(std::max<uint32_t>(ctx->front_cap, 72u), (uint32_t)kFrontCap);
   sa.ovf_list = w.ovf_list.p;
   sa.work = &ctx->d_ctr->work;
-  k_search_lean<STAGE><<<ctx->n_sm, kLeanWarps * 32, lean_smem(ctx->ix.smem_bytes, sa.stage_cap), s>>>(ctx->ix, sa);
+  k_search_lean<STAGE><<<ctx->n_sm, kLeanWarps * 32, lean_smem(ctx->index.ix.smem_bytes, sa.stage_cap), s>>>(ctx->index.ix, sa);
   LAUNCH_CHECK();
   // the queries whose frontier outgrew the lean kernel's slots (none, mostly: the launch then
   // finds an empty list and returns)
   sa.qlist = w.ovf_list.p;
   sa.qlist_n = &ctx->d_ctr->n_overflow;
   sa.work = &ctx->d_ctr->work2;
-  k_radius_search<STAGE><<<STAGE ? search_grid<true>(ctx) : ctx->search_grid_main, kSearchWarps * 32, gsm, s>>>(ctx->ix, sa);
+  k_radius_search<STAGE><<<STAGE ? search_grid<true>(ctx) : ctx->search_grid_main, kSearchWarps * 32, gsm, s>>>(ctx->index.ix, sa);
   LAUNCH_CHECK();
-  return SMB_OK;
-}
-
-// ------------------------------------------------------------------ index build
-// What the KD-order build takes: device arrays plus the extent of the points the index sees.
-struct IndexInput {
-  const float *val;              // values the windows read (whole cloud, or a shard's runs)
-  const uint64_t *pos;           // position of every window (whole cloud: of every point)
-  const uint32_t *wsrc, *worig;  // shard: value index / whole-cloud index of each window (else null)
-  uint64_t W;                    // windows, >= 1 (a rank that owns none passes one padding window)
-  size_t n_points;               // points of the whole cloud
-  float vmin, vmax;
-  uint32_t max_tpos, max_bucket;
-  std::vector<uint64_t> bucket_span;  // 1 + largest target per bucket (contig << 1 | strand)
-};
-static int build_index_core(smb_ctx *ctx, IndexInput &in);
-
-// owner == nullptr: every window of the cloud.  Otherwise (contig-sharded index) only the
-// windows whose first point lies on a contig with owner[contig] == rank; a window keeps its six
-// values even where it runs into the next contig / strand (Q2), so the shard holds exactly the
-// points the unsharded index holds for those contigs.
-// part != nullptr: the rank's own part of the cloud (smbh_build_point_cloud_part) instead of the
-// whole cloud + owner table; pos / val / n are then taken from it.
-static int build_index(smb_ctx *ctx, const uint64_t *pos, const float *val, size_t n,
-                       const uint32_t *owner = nullptr, uint32_t n_contigs = 0, uint32_t rank = 0,
-                       const smbh_cloud_part *part = nullptr) {
-  if (part) {
-    pos = part->pos;
-    val = part->val;
-    n = (size_t)part->n_points_total;
-  }
-  if (n < (size_t)kDim) return fail(ctx, SMB_ERR_ARG, "point cloud smaller than the index dimension");
-  const uint64_t W_all = n - (kDim - 1);
-  // ---- which windows, and where their values start in the uploaded value array
-  std::vector<float> h_val;       // sharded: runs of owned values, each with 5 trailing values
-  std::vector<uint64_t> h_pos;    // sharded: position of every owned window
-  std::vector<uint32_t> h_wsrc, h_worig;
-  if (part) {
-    // the runs are uploaded as they are; a window starts at every own point that has five more
-    // values after it in its run and is a window of the whole cloud (index < N - 5)
-    if (part->n_values > 0xFFFFFFF0ull)
-      return fail(ctx, SMB_ERR_CAPACITY, "more than 2^32 window points on one shard: use more ranks");
-    h_val.assign(part->val, part->val + part->n_values);
-    for (size_t k = 0; k < part->n_runs; ++k) {
-      const uint64_t a = part->run_off[k], b = part->run_off[k + 1];
-      for (uint64_t i = a; i < b; ++i) {
-        const uint64_t global = part->run_first[k] + (i - a);
-        if (!part->own[i] || i + (kDim - 1) >= b || global >= W_all) continue;
-        if ((part->pos[i] >> 33) >= n_contigs) return fail(ctx, SMB_ERR_ARG, "point cloud names a contig beyond n_contigs");
-        h_pos.push_back(part->pos[i]);
-        h_wsrc.push_back((uint32_t)i);
-        h_worig.push_back((uint32_t)global);
-      }
-    }
-    if (h_pos.empty()) {  // a rank may own nothing (more ranks than contigs): keep one padding leaf
-      h_val.assign(kDim, kPadValue);
-      h_pos.push_back(~0ull);
-      h_wsrc.push_back(0);
-      h_worig.push_back(0xFFFFFFFFu);
-    }
-  } else if (owner) {
-    for (uint64_t w = 0; w < W_all;) {
-      const uint64_t c = pos[w] >> 33;
-      if (c >= n_contigs) return fail(ctx, SMB_ERR_ARG, "point cloud names a contig beyond n_contigs");
-      if (owner[c] != rank) {
-        ++w;
-        continue;
-      }
-      uint64_t e = w + 1;  // maximal run of owned windows [w, e)
-      while (e < W_all && (pos[e] >> 33) < n_contigs && owner[pos[e] >> 33] == rank) ++e;
-      const size_t base = h_val.size();
-      if (base + (e - w) + kDim > 0xFFFFFFF0ull)
-        return fail(ctx, SMB_ERR_CAPACITY, "more than 2^32 window points on one shard: use more ranks");
-      h_val.insert(h_val.end(), val + w, val + e + (kDim - 1));
-      for (uint64_t x = w; x < e; ++x) {
-        h_pos.push_back(pos[x]);
-        h_wsrc.push_back((uint32_t)(base + (x - w)));
-        h_worig.push_back((uint32_t)x);
-      }
-      w = e;
-    }
-    if (h_pos.empty()) {  // a rank may own nothing (more ranks than contigs): keep one padding leaf
-      h_val.assign(kDim, kPadValue);
-      h_pos.push_back(~0ull);
-      h_wsrc.push_back(0);
-      h_worig.push_back(0xFFFFFFFFu);
-    }
-  } else if (W_all > 0xFFFFFFF0ull) {
-    return fail(ctx, SMB_ERR_CAPACITY, "more than 2^32 window points: shard the index by contig");
-  }
-  const bool subset = owner || part;
-  const uint64_t W = subset ? h_pos.size() : W_all;
-  const float *u_val = subset ? h_val.data() : val;
-  const uint64_t *u_pos = subset ? h_pos.data() : pos;
-  const size_t n_val = subset ? h_val.size() : n, n_pos = subset ? h_pos.size() : n;
-  const size_t n_seen = part ? part->n_values : n;  // points this rank can look at
-  float vmin = n_seen ? val[0] : 0.0f, vmax = vmin;
-  uint32_t max_tpos = 0, max_bucket = 0;
-  std::vector<uint64_t> bucket_span;  // 1 + largest target seen per bucket
-  if (part && n_contigs) {
-    // every rank must agree on the bucket numbering (the exchanges are indexed by bucket)
-    max_bucket = 2u * n_contigs - 1u;
-    bucket_span.assign((size_t)max_bucket + 1, 0);
-  }
-  for (size_t i = 0; i < n_seen; ++i) {
-    vmin = std::min(vmin, val[i]);
-    vmax = std::max(vmax, val[i]);
-    const uint32_t t = (uint32_t)(pos[i] >> 1), b = (uint32_t)(((pos[i] >> 33) << 1) | (pos[i] & 1));
-    max_tpos = std::max(max_tpos, t);
-    max_bucket = std::max(max_bucket, b);
-    if (b >= bucket_span.size()) bucket_span.resize((size_t)b + 1, 0);
-    bucket_span[b] = std::max<uint64_t>(bucket_span[b], (uint64_t)t + 1);
-  }
-  cudaStream_t s = ctx->stream;
-  DevBuf<float> d_val;
-  DevBuf<uint64_t> d_pos;
-  DevBuf<uint32_t> d_wsrc, d_worig;
-  CK(d_val.ensure(n_val));
-  CK(d_pos.ensure(n_pos));
-  CK(cudaMemcpyAsync(d_val.p, u_val, n_val * sizeof(float), cudaMemcpyHostToDevice, s));
-  CK(cudaMemcpyAsync(d_pos.p, u_pos, n_pos * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-  if (subset) {
-    CK(d_wsrc.ensure(W));
-    CK(d_worig.ensure(W));
-    CK(cudaMemcpyAsync(d_wsrc.p, h_wsrc.data(), W * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(d_worig.p, h_worig.data(), W * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-  }
-  IndexInput in{d_val.p, d_pos.p, d_wsrc.p, d_worig.p, W, n, vmin, vmax, max_tpos, max_bucket, std::move(bucket_span)};
-  const int rc = build_index_core(ctx, in);
-  cudaStreamSynchronize(s);
-  d_val.release();
-  d_pos.release();
-  d_wsrc.release();
-  d_worig.release();
-  return rc;
-}
-
-// The KD-order build from device arrays, wherever they came from (host_index.cc's cloud uploaded
-// by build_index, or the device-built cloud of k_cloud.cuh).  Window w starts at value
-// wsrc[w] (w itself when wsrc is null) and is point worig[w] of the whole cloud.
-static int build_index_core(smb_ctx *ctx, IndexInput &in) {
-  const uint64_t W = in.W;
-  const uint32_t n_leaves = (uint32_t)((W + kLeaf - 1) / kLeaf);
-  const float vmin = in.vmin, span = std::max(in.vmax - in.vmin, 1e-6f);
-  const std::vector<uint64_t> &bucket_span = in.bucket_span;
-  const float *d_val = in.val;
-  const uint64_t *d_pos = in.pos;
-  const uint32_t *d_wsrc = in.wsrc, *d_worig = in.worig;
-  cudaStream_t s = ctx->stream;
-  DevBuf<uint64_t> code_a, code_b;
-  DevBuf<uint32_t> w_a, w_b;
-  DevBuf<unsigned char> tmp;
-  DevBuf<uint32_t> ext_min, ext_max;
-  const uint32_t *d_order = nullptr;  // null: the windows' own order (one leaf holds them all)
-  if (W > (uint64_t)kLeaf) {
-    // aligned KD order (k_index.cuh): one pass per power-of-two segment size, top down
-    CK(code_a.ensure(W));
-    CK(code_b.ensure(W));
-    CK(w_a.ensure(W));
-    CK(w_b.ensure(W));
-    int log2s = 4;
-    while ((1ull << log2s) < W) ++log2s;
-    const unsigned blocks = (unsigned)((W + kKdThreads - 1) / kKdThreads);
-    const size_t n_ext = (size_t)((W + 15) / 16) * kDim;
-    CK(ext_min.ensure(n_ext));
-    CK(ext_max.ensure(n_ext));
-    size_t tb = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, tb, code_a.p, code_b.p, w_a.p, w_b.p, (uint64_t)W, 0, 64, s);
-    CK(tmp.ensure(tb));
-    uint32_t *ia = w_a.p, *ib = w_b.p;
-    bool first = true;
-    for (; log2s >= 4; --log2s) {
-      const uint64_t n_seg = (W + (1ull << log2s) - 1) >> log2s;
-      CK(cudaMemsetAsync(ext_min.p, 0xFF, n_seg * kDim * sizeof(uint32_t), s));
-      CK(cudaMemsetAsync(ext_max.p, 0x00, n_seg * kDim * sizeof(uint32_t), s));
-      k_kd_extent<<<blocks, kKdThreads, 0, s>>>(d_val, first ? nullptr : ia, d_wsrc, W, log2s, ext_min.p, ext_max.p);
-      LAUNCH_CHECK();
-      k_kd_keys<<<blocks, kKdThreads, 0, s>>>(d_val, first ? nullptr : ia, d_wsrc, W, log2s, ext_min.p, ext_max.p,
-                                              code_a.p, ia);
-      LAUNCH_CHECK();
-      int seg_bits = 0;
-      while ((1ull << seg_bits) < n_seg) ++seg_bits;
-      CK(cub::DeviceRadixSort::SortPairs(tmp.p, tb, code_a.p, code_b.p, ia, ib, (uint64_t)W, 0, 32 + seg_bits, s));
-      std::swap(ia, ib);
-      first = false;
-      ctx->stats.launches += 9;
-    }
-    d_order = ia;
-  }
-  CK(ctx->leaves.ensure((size_t)n_leaves * kLeafRec));
-  CK(ctx->leaf_widx.ensure((size_t)n_leaves * kLeaf));
-  k_build_leaves<<<(unsigned)(((uint64_t)n_leaves * kLeaf + 255) / 256), 256, 0, s>>>(
-      d_val, d_pos, d_order, W, n_leaves, ctx->leaves.p, ctx->leaf_widx.p, d_wsrc, d_worig);
-  LAUNCH_CHECK();
-  IndexView ix{};
-  ix.n_points = in.n_points;
-  ix.n_windows = W;
-  ix.n_leaves = n_leaves;
-  ix.vmin = vmin;
-  ix.inv_span = 1.0f / span;
-  // level sizes bottom-up; storage top-down in one buffer, so the levels every query walks are a
-  // prefix of it (staged in shared memory by the lean search kernel)
-  int L = 0;
-  for (uint32_t n_child = n_leaves;;) {
-    if (L >= kMaxLevels) return fail(ctx, SMB_ERR_CAPACITY, "index hierarchy deeper than kMaxLevels");
-    const uint32_t n_nodes = (n_child + kFan - 1) / kFan;
-    if (n_nodes >= (1u << 28)) return fail(ctx, SMB_ERR_CAPACITY, "index level exceeds 2^28 nodes");
-    ix.level_count[L++] = n_nodes;
-    if (n_nodes <= (uint32_t)kFan) break;  // the search starts from all nodes of the top level
-    n_child = n_nodes;
-  }
-  ix.n_levels = L;
-  uint64_t total_rec = 0;
-  ix.smem_from = L;
-  ix.smem_bytes = 0;
-  for (int l = L - 1; l >= 0; --l) {
-    if (total_rec * kNodeRec > 0xFFFFFFF0ull) return fail(ctx, SMB_ERR_CAPACITY, "node levels exceed 2^32 records: shard the index");
-    ix.level_off[l] = (uint32_t)(total_rec * kNodeRec);
-    total_rec += ix.level_count[l];
-    if (ix.smem_from == l + 1 && total_rec * kNodeRec * sizeof(uint2) <= kTopSmemMax) {
-      ix.smem_from = l;
-      ix.smem_bytes = (uint32_t)(total_rec * kNodeRec * sizeof(uint2));
-    }
-  }
-  CK(ctx->nodes.ensure((size_t)total_rec * kNodeRec));
-  for (int l = 0; l < L; ++l) {
-    const uint32_t n_nodes = ix.level_count[l];
-    const unsigned blocks = (unsigned)(((uint64_t)n_nodes * kFan + 255) / 256);
-    if (l == 0)
-      k_nodes_level0<<<blocks, 256, 0, s>>>(ctx->leaves.p, n_leaves, n_nodes, ctx->nodes.p + ix.level_off[0]);
-    else
-      k_nodes_up<<<blocks, 256, 0, s>>>(ctx->nodes.p + ix.level_off[l - 1], ix.level_count[l - 1], n_nodes,
-                                        ctx->nodes.p + ix.level_off[l]);
-    LAUNCH_CHECK();
-  }
-  ix.nodes = ctx->nodes.p;
-  ix.leaves = ctx->leaves.p;
-  ix.leaf_widx = ctx->leaf_widx.p;
-  CK(cudaStreamSynchronize(s));
-  code_a.release();
-  code_b.release();
-  w_a.release();
-  w_b.release();
-  tmp.release();
-  ext_min.release();
-  ext_max.release();
-  {
-    // linear coordinate g = bucket_base[bucket] + target: monotone in the sort order, dense
-    // enough to be cut into equal-width bins by the per-entry sort
-    std::vector<uint64_t> base(bucket_span.size() + 1, 0);
-    for (size_t b = 0; b < bucket_span.size(); ++b) base[b + 1] = base[b] + bucket_span[b];
-    CK(ctx->bucket_base.ensure(base.size()));
-    CK(cudaMemcpy(ctx->bucket_base.p, base.data(), base.size() * sizeof(uint64_t), cudaMemcpyHostToDevice));
-    ctx->g_total = base.back();
-    ctx->gshift = 0;
-    while ((base.back() >> ctx->gshift) >= (uint64_t)kCoarseBins) ++ctx->gshift;
-    ctx->n_coarse = (uint32_t)(base.back() >> ctx->gshift) + 1;
-  }
-  ctx->ix = ix;
-  ctx->search_grid_main = search_grid<false>(ctx);
-  ctx->max_tpos = in.max_tpos;
-  ctx->max_bucket = in.max_bucket;
-  ctx->has_index = true;
   return SMB_OK;
 }
 
@@ -842,14 +410,14 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   const uint32_t B = en.B, Bpres = en.B_present;
   if (B == 0) return SMB_OK;
   if (!ctx->has_index) return fail(ctx, SMB_ERR_STATE, "no index loaded");
-  const bool sharded = ctx->ex && ctx->index_sharded;
+  const bool sharded = ctx->ex && ctx->index.sharded;
   // ---- key layout for this step
   uint32_t max_ev = 0;
   for (uint32_t b = 0; b < Bpres; ++b) max_ev = std::max(max_ev, sp.h_events[en.slot[b]]);
   KeyLayout kl;
   kl.qbits = bits_for((uint64_t)max_ev + kFeatCap);
-  kl.tbits = bits_for(ctx->max_tpos);
-  kl.bbits = bits_for(ctx->max_bucket);
+  kl.tbits = bits_for(ctx->index.max_tpos);
+  kl.bbits = bits_for(ctx->index.max_bucket);
   kl.ebits = bits_for(B - 1);
   if (kl.total() > 64) return fail(ctx, SMB_ERR_CAPACITY, "sort key exceeds 64 bits: lower max_batch_chunks");
   if (ctx->max_batch_anchors >= (1ull << 30)) return fail(ctx, SMB_ERR_ARG, "max_batch_anchors must stay below 2^30");
@@ -925,13 +493,13 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   // entry fills kPartFill (70 %) of one k_part_sort CTA; more than kMaxParts -> one list, k_seg_sort
   constexpr double kPartFill = 0.70;
   uint32_t n_parts = 1;
-  uint64_t span = std::max<uint64_t>(ctx->g_total, 1);
+  uint64_t span = std::max<uint64_t>(ctx->index.g_total, 1);
   if (mode == SORT_PART) {
-    const double per_coord = std::max(ctx->est_anchors_per_chunk, 1.0) / (double)std::max<uint64_t>(ctx->g_total, 1);
+    const double per_coord = std::max(ctx->est_anchors_per_chunk, 1.0) / (double)std::max<uint64_t>(ctx->index.g_total, 1);
     const double want = kPartFill * (double)kPartSortCap / per_coord;
-    if (want < (double)ctx->g_total) {
+    if (want < (double)ctx->index.g_total) {
       const uint64_t sp2 = std::max<uint64_t>((uint64_t)want, 1);
-      const uint64_t np = (ctx->g_total + sp2 - 1) / sp2;
+      const uint64_t np = (ctx->index.g_total + sp2 - 1) / sp2;
       if (np <= (uint64_t)kMaxParts) {
         n_parts = (uint32_t)np;
         span = sp2;
@@ -963,7 +531,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   k_inject_carry<<<(B * 32 + kCarryThreads - 1) / kCarryThreads, kCarryThreads, 0, s>>>(
       w.entry_slot.p, w.n_queries.p, sp.slots.p, sp.pool_anchor[0].p, sp.pool_anchor[1].p, B, kl, w.key_a.p,
       w.dist_a.p, cap, ctx->d_ctr, want_seg ? w.runs.p : nullptr, w.run_count.p, w.entry_total.p,
-      runs_cap, n_parts, inv_span, ctx->bucket_base.p, w.seg_qmin.p);
+      runs_cap, n_parts, inv_span, ctx->index.bucket_base.p, w.seg_qmin.p);
   LAUNCH_CHECK();
   SearchArgs sa{};
   sa.features = src == SRC_CACHED ? w.feat_cache[w.cache_cur].p : w.features.p;
@@ -986,8 +554,8 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   sa.runs_cap = runs_cap;
   sa.n_parts = n_parts;
   sa.inv_span = inv_span;
-  sa.bucket_base = ctx->bucket_base.p;
-  sa.n_buckets = ctx->max_bucket + 1u;
+  sa.bucket_base = ctx->index.bucket_base.p;
+  sa.n_buckets = ctx->index.max_bucket + 1u;
   // query-order buffers are sized from a running estimate (the exact count is on the device)
   const uint32_t q_per_chunk_max = (uint32_t)(kFeatCap - kDim) / (uint32_t)prm.step_size;
   const uint32_t nq_max = (uint32_t)std::min<uint64_t>(
@@ -1058,8 +626,8 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     ps.n_parts = n_parts;
     ps.span = span;
     ps.kl = kl;
-    ps.bucket_base = ctx->bucket_base.p;
-    ps.n_buckets = ctx->max_bucket + 1u;
+    ps.bucket_base = ctx->index.bucket_base.p;
+    ps.n_buckets = ctx->index.max_bucket + 1u;
     ps.ctr = ctx->d_ctr;
     k_part_sort<kPartSortCap, 512, 4096><<<(unsigned)n_lists, 512, part_sort_smem_bytes(kPartSortCap, 4096), s>>>(ps);
     LAUNCH_CHECK();
@@ -1076,9 +644,9 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     ss.n_parts = n_parts;
     ss.B = B;
     ss.kl = kl;
-    ss.bucket_base = ctx->bucket_base.p;
-    ss.gshift = ctx->gshift;
-    ss.n_coarse = ctx->n_coarse;
+    ss.bucket_base = ctx->index.bucket_base.p;
+    ss.gshift = ctx->index.gshift;
+    ss.n_coarse = ctx->index.n_coarse;
     ss.ctr = ctx->d_ctr;
     k_seg_sort<kSortCapBig, 1024, 8192><<<B, 1024, sort_smem_bytes(kSortCapBig, 8192), s>>>(ss);
     LAUNCH_CHECK();
@@ -1148,7 +716,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   se.n_features = w.n_features.p;
   se.slots = sp.slots.p;
   se.B = B;
-  se.max_chains = std::min<uint32_t>(3u * (ctx->max_bucket + 1u), 4096u);
+  se.max_chains = std::min<uint32_t>(3u * (ctx->index.max_bucket + 1u), 4096u);
   CK(w.chain_tmp.ensure((size_t)B * se.max_chains));
   CK(w.n_scratch.ensure(B));
   CK(w.pick.ensure(B));
@@ -1331,7 +899,7 @@ static void slots_release(SlotSpace &sp) {
 static int round_begin(smb_ctx *ctx, SlotSpace &sp, const std::vector<uint32_t> &slots, int step,
                        uint32_t out_pool) {
   uint64_t need_anchor = 0, need_chain = 0;
-  const uint32_t max_chains = std::min<uint32_t>(3u * (ctx->max_bucket + 1u), 4096u);
+  const uint32_t max_chains = std::min<uint32_t>(3u * (ctx->index.max_bucket + 1u), 4096u);
   for (uint32_t sl : slots) {
     // a chain has strictly increasing query positions: <= one anchor per seed position
     need_anchor += (uint64_t)(sp.h_events[sl] + kFeatCap) / (uint32_t)std::max(step, 1) + 4ull * max_chains;
@@ -1363,7 +931,7 @@ static int run_round(smb_ctx *ctx, SlotSpace &sp, const std::vector<uint32_t> &p
   // absent slots ride along with the first step (pure copy-forward)
   size_t at = 0;
   bool absent_done = absent.empty();
-  const int kbits = bits_for(ctx->max_tpos) + bits_for(ctx->max_bucket);
+  const int kbits = bits_for(ctx->index.max_tpos) + bits_for(ctx->index.max_bucket);
   while (at < present.size() || !absent_done) {
     uint32_t max_ev = 0;
     for (size_t i = at; i < present.size(); ++i) max_ev = std::max(max_ev, sp.h_events[present[i]]);
@@ -1387,7 +955,7 @@ static int run_round(smb_ctx *ctx, SlotSpace &sp, const std::vector<uint32_t> &p
       if (rc == 2) continue;  // aborted on the device, cause dealt with: again
       if (rc == 1) {  // anchor buffer overflow: grow the buffers, or halve the step at the limit
         ctx->est_anchors_per_chunk *= 2.0;
-        if ((ctx->ex && ctx->index_sharded) ? ctx->group_at_limit : ctx->last_cap >= ctx->max_batch_anchors) {
+        if ((ctx->ex && ctx->index.sharded) ? ctx->group_at_limit : ctx->last_cap >= ctx->max_batch_anchors) {
           if (count <= 1) return fail(ctx, SMB_ERR_CAPACITY, "one chunk overflows max_batch_anchors");
           count = (count + 1) / 2;
         }
@@ -1407,7 +975,7 @@ static int run_round(smb_ctx *ctx, SlotSpace &sp, const std::vector<uint32_t> &p
 // chain 0's anchors (SlotState::owned0); everybody else contributes zeros, so a SUM all-reduce
 // of the bit patterns hands every rank the owner's values.  flags bit0 (5000-hit cap) is OR-ed.
 static int merge_owner_tags(smb_ctx *ctx, std::vector<SlotState> &st, size_t n) {
-  if (!ctx->ex || !ctx->index_sharded || n == 0) return SMB_OK;
+  if (!ctx->ex || !ctx->index.sharded || n == 0) return SMB_OK;
   std::vector<uint32_t> h(n * 6);
   auto bits = [](float f) { uint32_t u; memcpy(&u, &f, 4); return u; };
   for (size_t r = 0; r < n; ++r) {
@@ -1559,6 +1127,10 @@ int smb_create(smb_ctx **out, int device) {
   }
   smb_ctx *ctx = new smb_ctx();
   ctx->device = device;
+  ctx->front_cap = kFrontCap;
+  ctx->dp_passes = kDpFreePasses;
+  ctx->prep_rounds = kPrepRounds;
+  ctx->dp_pass_max_entries = kDpPassMaxEntries;
   auto bail = [&](const char *what, cudaError_t err) {
     g_create_error = std::string(what) + ": " + cudaGetErrorString(err);
     delete ctx;
@@ -1645,7 +1217,7 @@ void smb_destroy(smb_ctx *ctx) {
   w.cand_counts.release(); w.ctl.release(); w.tags.release();
   ctx->ex.reset();
   ctx->local_group.reset();
-  ctx->leaves.release(); ctx->nodes.release(); ctx->leaf_widx.release(); ctx->bucket_base.release();
+  ctx->index.leaves.release(); ctx->index.nodes.release(); ctx->index.leaf_widx.release(); ctx->index.bucket_base.release();
   w.qkey_a.release(); w.qkey_b.release(); w.qpay_a.release(); w.qpay_b.release(); w.ovf_list.release();
   w.entry_info.release(); w.qsort_temp.release();
   ctx->raw.release(); ctx->kept.release(); ctx->d_read_off.release(); ctx->d_kept_off.release();
@@ -1704,137 +1276,6 @@ int smb_set_limits(smb_ctx *ctx, uint32_t max_batch_chunks, uint64_t max_batch_a
 int smb_set_option(smb_ctx *ctx, const char *name, const char *value) {
   if (!name || !value) return fail(ctx, SMB_ERR_ARG, "smb_set_option: null name or value");
   if (!apply_option(ctx, name, value)) return fail(ctx, SMB_ERR_ARG, std::string("smb_set_option: unknown option ") + name);
-  return SMB_OK;
-}
-
-// -------------------------------------------------------------------- index
-int smb_index_set_points(smb_ctx *ctx, const uint64_t *pos, const float *val, size_t n) {
-  CK(cudaSetDevice(ctx->device));
-  ctx->index_sharded = false;
-  return build_index(ctx, pos, val, n);
-}
-
-int smb_index_load(smb_ctx *ctx, const char *prefix) {
-  uint64_t *pos = nullptr;
-  float *val = nullptr;
-  size_t n = 0;
-  int dim = 0, ml = 0;
-  int rc = smbh_pt_read(prefix, &pos, &val, &n, &dim, &ml);
-  if (rc) return fail(ctx, rc, std::string("cannot read ") + prefix + ".pt");
-  if (dim != kDim) {
-    smbh_free(pos);
-    smbh_free(val);
-    return fail(ctx, SMB_ERR_ARG, "index dimension is not 6");
-  }
-  rc = smb_index_set_points(ctx, pos, val, n);
-  smbh_free(pos);
-  smbh_free(val);
-  return rc;
-}
-
-int smb_index_set_contigs(smb_ctx *ctx, const uint32_t *lengths, uint32_t n_contigs) {
-  ctx->contig_len.assign(lengths, lengths + n_contigs);
-  return SMB_OK;
-}
-
-int smb_index_set_points_sharded(smb_ctx *ctx, const uint64_t *pos, const float *val, size_t n,
-                                 const uint32_t *contig_owner, uint32_t n_contigs) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->ex) return fail(ctx, SMB_ERR_STATE, "join a shard group first (smb_shard_local_group / smb_shard_nccl_init)");
-  for (uint32_t c = 0; c < n_contigs; ++c)
-    if (contig_owner[c] >= (uint32_t)ctx->ex->world) return fail(ctx, SMB_ERR_ARG, "contig owner out of range");
-  const int rc = build_index(ctx, pos, val, n, contig_owner, n_contigs, (uint32_t)ctx->ex->rank);
-  ctx->index_sharded = rc == SMB_OK;
-  return rc;
-}
-
-int smb_index_set_points_part(smb_ctx *ctx, const smbh_cloud_part *part, uint32_t n_contigs) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->ex) return fail(ctx, SMB_ERR_STATE, "join a shard group first (smb_shard_local_group / smb_shard_nccl_init)");
-  if (!part || !n_contigs) return fail(ctx, SMB_ERR_ARG, "smb_index_set_points_part: no part / no contigs");
-  const int rc = build_index(ctx, nullptr, nullptr, 0, nullptr, n_contigs, (uint32_t)ctx->ex->rank, part);
-  ctx->index_sharded = rc == SMB_OK;
-  return rc;
-}
-
-// Read-sharded runs (SURVEY.md 8e mode 1): the index is built once, on `root`, and travels to
-// the other ranks of the group over NVLink (ncclBroadcast, or peer copies inside one process)
-// instead of being rebuilt from the point cloud by every rank.  Collective: every rank of the
-// group calls it; only the root needs an index (and contigs) beforehand.
-int smb_index_broadcast(smb_ctx *ctx, int root) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->ex) return fail(ctx, SMB_ERR_STATE, "join a group first (smb_shard_local_group / smb_shard_nccl_init)");
-  if (root < 0 || root >= ctx->ex->world) return fail(ctx, SMB_ERR_ARG, "bad root");
-  const bool is_root = ctx->ex->rank == root;
-  if (is_root && !ctx->has_index) return fail(ctx, SMB_ERR_STATE, "the root has no index to broadcast");
-  cudaStream_t s = ctx->stream;
-  // ---- header: the view (without pointers), bucket tables, contig lengths
-  struct Header {
-    IndexView ix;
-    uint32_t max_tpos, max_bucket, n_coarse, n_contigs;
-    int gshift;
-    uint64_t g_total, n_bucket_base, n_nodes_rec, n_leaf_rec, n_widx;
-  } h{};
-  if (is_root) {
-    h.ix = ctx->ix;
-    h.max_tpos = ctx->max_tpos;
-    h.max_bucket = ctx->max_bucket;
-    h.n_coarse = ctx->n_coarse;
-    h.gshift = ctx->gshift;
-    h.g_total = ctx->g_total;
-    h.n_contigs = (uint32_t)ctx->contig_len.size();
-    h.n_bucket_base = (uint64_t)ctx->max_bucket + 2;
-    uint64_t rec = 0;
-    for (int l = 0; l < ctx->ix.n_levels; ++l) rec += ctx->ix.level_count[l];
-    h.n_nodes_rec = rec * kNodeRec;
-    h.n_leaf_rec = (uint64_t)ctx->ix.n_leaves * kLeafRec;
-    h.n_widx = (uint64_t)ctx->ix.n_leaves * kLeaf;
-  }
-  DevBuf<unsigned char> d_h;
-  CK(d_h.ensure(sizeof(Header)));
-  if (is_root) CK(cudaMemcpyAsync(d_h.p, &h, sizeof(Header), cudaMemcpyHostToDevice, s));
-  int rc = ctx->ex->broadcast(d_h.p, sizeof(Header), root, s, ctx->err);
-  if (rc) return rc;
-  CK(cudaMemcpyAsync(&h, d_h.p, sizeof(Header), cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  d_h.release();
-  // ---- the arrays, in place in the receivers' own buffers
-  if (!is_root) {
-    CK(ctx->nodes.ensure(h.n_nodes_rec));
-    CK(ctx->leaves.ensure(h.n_leaf_rec));
-    CK(ctx->leaf_widx.ensure(h.n_widx));
-    CK(ctx->bucket_base.ensure(h.n_bucket_base));
-  }
-  DevBuf<uint32_t> d_len;
-  CK(d_len.ensure(std::max<uint32_t>(h.n_contigs, 1)));
-  if (is_root && h.n_contigs)
-    CK(cudaMemcpyAsync(d_len.p, ctx->contig_len.data(), h.n_contigs * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-  if ((rc = ctx->ex->broadcast(ctx->nodes.p, h.n_nodes_rec * sizeof(uint2), root, s, ctx->err))) return rc;
-  if ((rc = ctx->ex->broadcast(ctx->leaves.p, h.n_leaf_rec * sizeof(uint2), root, s, ctx->err))) return rc;
-  if ((rc = ctx->ex->broadcast(ctx->leaf_widx.p, h.n_widx * sizeof(uint32_t), root, s, ctx->err))) return rc;
-  if ((rc = ctx->ex->broadcast(ctx->bucket_base.p, h.n_bucket_base * sizeof(uint64_t), root, s, ctx->err))) return rc;
-  if ((rc = ctx->ex->broadcast(d_len.p, std::max<uint32_t>(h.n_contigs, 1) * sizeof(uint32_t), root, s, ctx->err))) return rc;
-  ctx->stats.exchanges += 6;
-  if (!is_root) {
-    ctx->contig_len.resize(h.n_contigs);
-    if (h.n_contigs)
-      CK(cudaMemcpyAsync(ctx->contig_len.data(), d_len.p, h.n_contigs * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    IndexView ix = h.ix;
-    ix.nodes = ctx->nodes.p;
-    ix.leaves = ctx->leaves.p;
-    ix.leaf_widx = ctx->leaf_widx.p;
-    ctx->ix = ix;
-    ctx->max_tpos = h.max_tpos;
-    ctx->max_bucket = h.max_bucket;
-    ctx->n_coarse = h.n_coarse;
-    ctx->gshift = h.gshift;
-    ctx->g_total = h.g_total;
-    ctx->search_grid_main = search_grid<false>(ctx);
-    ctx->has_index = true;
-  }
-  CK(cudaStreamSynchronize(s));
-  d_len.release();
-  ctx->index_sharded = false;
   return SMB_OK;
 }
 
@@ -1917,9 +1358,6 @@ int smb_shard_nccl_init(smb_ctx *ctx, int rank, int world, const char *id128) {
 
 int smb_shard_rank(const smb_ctx *ctx) { return ctx->ex ? ctx->ex->rank : 0; }
 int smb_shard_world(const smb_ctx *ctx) { return ctx->ex ? ctx->ex->world : 1; }
-
-uint64_t smb_index_num_points(const smb_ctx *ctx) { return ctx->has_index ? ctx->ix.n_points : 0; }
-uint32_t smb_index_num_contigs(const smb_ctx *ctx) { return (uint32_t)ctx->contig_len.size(); }
 
 // ------------------------------------------------------------ whole hot path
 }  // extern "C"
@@ -2109,7 +1547,7 @@ static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping
   // wave run while the current one is being mapped (option pipeline=on: also with resident samples,
   // which then join in waves of filter-only slices).  Contig shards must run identical ticks on every
   // rank: no timing-dependent admission there.
-  const bool sharded_index = ctx->ex && ctx->index_sharded;
+  const bool sharded_index = ctx->ex && ctx->index.sharded;
   // auto: only when the samples arrive from the host during the call.  With resident samples the
   // GPU is busy mapping from the first tick on and the overlap only adds contention and steps
   // (measured on config 3: 437 ms pipelined against 403 ms; with host buffers on two GPUs e2e
@@ -2982,519 +2420,6 @@ int smb_stream_round(smb_ctx *ctx, const uint32_t *channels, uint32_t n, const i
       make_row(ctx, st[ch], ctx->stream_kept[ch] + (uint32_t)ctx->stream_pending[ch].size(), used, &maps[i]);
     }
   }
-  return SMB_OK;
-}
-
-}  // extern "C"
-
-// ================================================================== device index build
-// The point cloud of host_index.cc's build_cloud, built on the device (k_cloud.cuh), and the
-// index built from it without a host copy.  DESIGN.md, "device index build".
-namespace {
-
-template <class T>
-struct DevArr {  // exact-size device array, freed with its owner
-  T *p = nullptr;
-  size_t n = 0;
-  DevArr() = default;
-  DevArr(const DevArr &) = delete;
-  DevArr &operator=(const DevArr &) = delete;
-  ~DevArr() { reset(); }
-  void reset() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    n = 0;
-  }
-  cudaError_t alloc(size_t k) {
-    reset();
-    const cudaError_t e = cudaMalloc((void **)&p, std::max<size_t>(k, 1) * sizeof(T));
-    if (e != cudaSuccess) {
-      p = nullptr;
-      cudaGetLastError();  // an out-of-memory return is not sticky; clear it
-      return e;
-    }
-    n = k;
-    return e;
-  }
-};
-
-struct StageTimer {  // CUDA events between the stages of one build
-  cudaEvent_t ev[9] = {};
-  int n = 0;
-  ~StageTimer() {
-    for (cudaEvent_t e : ev)
-      if (e) cudaEventDestroy(e);
-  }
-  cudaError_t mark(cudaStream_t s) {
-    if (!ev[n]) {
-      const cudaError_t e = cudaEventCreate(&ev[n]);
-      if (e != cudaSuccess) return e;
-    }
-    return cudaEventRecord(ev[n++], s);
-  }
-  double ms(int a, int b) const {
-    float f = 0.0f;
-    if (a < n && b < n) cudaEventElapsedTime(&f, ev[a], ev[b]);
-    return f;
-  }
-};
-
-constexpr size_t kCloudSlice = 16u << 20;  // bytes per pinned upload slice
-
-}  // namespace
-
-#define CLOUD_ALLOC(arr, k, what)                                                                             \
-  do {                                                                                                        \
-    if ((arr).alloc(k) != cudaSuccess)                                                                        \
-      return fail(ctx, SMB_ERR_CAPACITY,                                                                      \
-                  std::string("device index build: out of device memory for ") + (what) + " (" +            \
-                      std::to_string(((size_t)(k) * sizeof(*(arr).p)) >> 20) + " MiB more)");              \
-  } while (0)
-
-// The whole cloud in device memory (*pos / *val, *count points).  Stage times go to
-// ctx->build_stats (ms_index is left to the caller).
-static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
-                       const float *level_mean, DevArr<uint64_t> &pos, DevArr<float> &val, uint64_t *count) {
-  using namespace cloud;
-  if (n && (!seqs || !lengths)) return fail(ctx, SMB_ERR_ARG, "device index build: null sequences / lengths");
-  if (!level_mean) return fail(ctx, SMB_ERR_ARG, "device index build: null level table");
-  CK(cudaSetDevice(ctx->device));
-  cudaStream_t s = ctx->stream;
-  smb_build_stats &bs = ctx->build_stats;
-  memset(&bs, 0, sizeof bs);
-  bs.tile = ctx->cloud_tile;
-  *count = 0;
-  // segments: + strands by contig, then - strands (contigs under 11 bases have no window)
-  std::vector<Seg> segs;
-  std::vector<uint64_t> plus_off(n, 0);
-  uint64_t n_bases = 0, n_pos = 0;
-  for (uint32_t c = 0; c < n; ++c) {
-    if (lengths[c] < (uint32_t)kMaskK) continue;
-    if (!seqs[c]) return fail(ctx, SMB_ERR_ARG, "device index build: null sequence");
-    plus_off[c] = n_bases;
-    n_bases += lengths[c];
-  }
-  for (uint32_t strand = 0; strand < 2; ++strand)
-    for (uint32_t c = 0; c < n; ++c) {
-      if (lengths[c] < (uint32_t)kMaskK) continue;
-      segs.push_back(Seg{plus_off[c], n_pos, lengths[c], c, strand, 0});
-      n_pos += lengths[c] - kK + 1;
-    }
-  if (segs.empty()) {
-    CLOUD_ALLOC(pos, 0, "the point cloud");
-    CLOUD_ALLOC(val, 0, "the point cloud");
-    return SMB_OK;
-  }
-  const uint32_t n_segs = (uint32_t)segs.size(), n_plus = n_segs / 2;
-  bs.strands = n_segs;
-  StageTimer tm;
-  CK(tm.mark(s));
-  // ---- upload the + strands through two pinned slices
-  DevArr<unsigned char> d_seq;
-  CLOUD_ALLOC(d_seq, n_bases, "the reference sequences");
-  {
-    const size_t slice = kCloudSlice;
-    cudaEvent_t done[2] = {};
-    if (!ctx->h_cloud_stage) CK(cudaHostAlloc((void **)&ctx->h_cloud_stage, 2 * slice, cudaHostAllocDefault));
-    CK(cudaEventCreateWithFlags(&done[0], cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&done[1], cudaEventDisableTiming));
-    int k = 0;
-    cudaError_t e = cudaSuccess;
-    for (uint32_t c = 0; c < n && e == cudaSuccess; ++c) {
-      if (lengths[c] < (uint32_t)kMaskK) continue;
-      for (uint64_t a = 0; a < lengths[c] && e == cudaSuccess; a += slice) {
-        const size_t len = (size_t)std::min<uint64_t>(slice, lengths[c] - a);
-        unsigned char *h = ctx->h_cloud_stage + (size_t)k * slice;
-        if ((e = cudaEventSynchronize(done[k])) != cudaSuccess) break;
-        memcpy(h, seqs[c] + a, len);
-        if ((e = cudaMemcpyAsync(d_seq.p + plus_off[c] + a, h, len, cudaMemcpyHostToDevice, s)) != cudaSuccess) break;
-        e = cudaEventRecord(done[k], s);
-        k ^= 1;
-      }
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    cudaEventDestroy(done[0]);
-    cudaEventDestroy(done[1]);
-    if (e != cudaSuccess) return fail(ctx, SMB_ERR_CUDA, std::string("device index build: upload: ") + cudaGetErrorString(e));
-  }
-  ctx->stats.h2d_bytes += n_bases;
-  DevArr<Seg> d_segs;
-  CLOUD_ALLOC(d_segs, n_segs, "the segment table");
-  CK(cudaMemcpyAsync(d_segs.p, segs.data(), n_segs * sizeof(Seg), cudaMemcpyHostToDevice, s));
-  CK(tm.mark(s));
-  // ---- 11-mer census over the + strands
-  std::vector<Chunk> chunks;
-  for (uint32_t i = 0; i < n_plus; ++i)
-    for (uint32_t p = 0; p < segs[i].len - kMaskK + 1; p += kChunkPos) chunks.push_back(Chunk{i, p});
-  const size_t n_census = chunks.size();
-  for (uint32_t i = 0; i < n_segs; ++i)
-    for (uint32_t p = 0; p < segs[i].len - kK + 1; p += kChunkPos) chunks.push_back(Chunk{i, p});
-  DevArr<Chunk> d_chunks;
-  DevArr<uint32_t> d_hist;
-  DevArr<unsigned long long> d_total;
-  CLOUD_ALLOC(d_chunks, chunks.size(), "the chunk table");
-  CLOUD_ALLOC(d_hist, (size_t)1 << (2 * kMaskK), "the 11-mer histogram");
-  CLOUD_ALLOC(d_total, 1, "the 11-mer histogram");
-  CK(cudaMemcpyAsync(d_chunks.p, chunks.data(), chunks.size() * sizeof(Chunk), cudaMemcpyHostToDevice, s));
-  CK(cudaMemsetAsync(d_hist.p, 0, d_hist.n * sizeof(uint32_t), s));
-  CK(cudaMemsetAsync(d_total.p, 0, sizeof(unsigned long long), s));
-  k_cloud_census<<<(unsigned)n_census, 256, 0, s>>>(d_seq.p, d_segs.p, d_chunks.p, d_hist.p, d_total.p);
-  LAUNCH_CHECK();
-  CK(tm.mark(s));
-  // ---- level hashes and mask, both strands
-  DevArr<uint16_t> d_hm;
-  CLOUD_ALLOC(d_hm, n_pos, "the per-position level hashes");
-  k_cloud_hm<<<(unsigned)(chunks.size() - n_census), 256, 0, s>>>(d_seq.p, d_segs.p, d_chunks.p + n_census, d_hist.p,
-                                                                   d_total.p, d_hm.p);
-  LAUNCH_CHECK();
-  CK(tm.mark(s));
-  CK(cudaStreamSynchronize(s));
-  d_seq.reset();
-  d_hist.reset();
-  d_chunks.reset();
-  // ---- z-normalisation: sequential double sums per strand -> z table per segment
-  DevArr<float> d_lv, d_ztab;
-  CLOUD_ALLOC(d_lv, kTable, "the level table");
-  CLOUD_ALLOC(d_ztab, (size_t)n_segs * kTable, "the z tables");
-  CK(cudaMemcpyAsync(d_lv.p, level_mean, kTable * sizeof(float), cudaMemcpyHostToDevice, s));
-  // the mean as an exact integer sum in units of the smallest ulp of the table (k_cloud_zsums):
-  // possible when every level is finite and a strand's sum of |level| / unit stays in an int64
-  int unit_exp = 0, int_ok = 1;
-  {
-    int lo = 1 << 30;
-    double q_max = 0.0;
-    for (int i = 0; i < kTable; ++i) {
-      const float x = level_mean[i];
-      if (!std::isfinite(x)) int_ok = 0;
-      else if (x != 0.0f) lo = std::min(lo, std::max(std::ilogb(x), -126) - 23);
-    }
-    if (lo == 1 << 30) lo = 0;
-    for (int i = 0; i < kTable && int_ok; ++i) q_max = std::max(q_max, std::ldexp(std::fabs((double)level_mean[i]), -lo));
-    uint32_t max_len = 0;
-    for (const Seg &g : segs) max_len = std::max(max_len, g.len);
-    if (!int_ok || q_max * (double)max_len >= 9.0e18) int_ok = 0;
-    unit_exp = lo;
-  }
-  DevArr<unsigned int> d_serial;
-  CLOUD_ALLOC(d_serial, 1, "the z sums");
-  CK(cudaMemsetAsync(d_serial.p, 0, sizeof(unsigned int), s));
-  k_cloud_zsums<<<(n_segs + kZWarps - 1) / kZWarps, kZWarps * 32, 0, s>>>(d_segs.p, n_segs, d_hm.p, d_lv.p, int_ok,
-                                                                           unit_exp, d_ztab.p, d_serial.p);
-  LAUNCH_CHECK();
-  CK(cudaMemcpyAsync(&bs.strands_serial_mean, d_serial.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, s));
-  CK(tm.mark(s));
-  // ---- point selection: speculative tiles, fix-up, chain
-  std::vector<Tile> tiles;
-  const uint32_t T = std::max<uint32_t>(ctx->cloud_tile, 1);
-  uint64_t n_tiles64 = 0;
-  for (const Seg &g : segs) n_tiles64 += (g.len - kMaskK + 1 + (uint64_t)T - 1) / T;
-  if (n_tiles64 >= 0xFFFFFFFFull) return fail(ctx, SMB_ERR_ARG, "device index build: more than 2^32 tiles: raise cloud_tile");
-  tiles.reserve(n_tiles64);
-  for (uint32_t i = 0; i < n_segs; ++i) {
-    const uint32_t nw = segs[i].len - kMaskK + 1;
-    for (uint32_t p = 0; p < nw; p += std::min(T, nw - p)) tiles.push_back(Tile{i, p, p + std::min(T, nw - p), 0});
-  }
-  const uint32_t n_tiles = (uint32_t)tiles.size();
-  DevArr<Tile> d_tiles;
-  DevArr<TileState> d_ts;
-  DevArr<uint8_t> d_flags;
-  DevArr<ChainStats> d_cs;
-  DevArr<unsigned long long> d_cnt, d_off;
-  CLOUD_ALLOC(d_tiles, n_tiles, "the tile table");
-  CLOUD_ALLOC(d_ts, n_tiles, "the tile states");
-  CLOUD_ALLOC(d_flags, n_pos, "the keep flags");
-  CLOUD_ALLOC(d_cs, 1, "the tile states");
-  CLOUD_ALLOC(d_cnt, n_tiles, "the tile counts");
-  CLOUD_ALLOC(d_off, n_tiles, "the tile counts");
-  CK(cudaMemcpyAsync(d_tiles.p, tiles.data(), n_tiles * sizeof(Tile), cudaMemcpyHostToDevice, s));
-  const unsigned tb = 128, tg = (n_tiles + tb - 1) / tb;
-  k_cloud_spec<<<tg, tb, 0, s>>>(d_segs.p, d_tiles.p, n_tiles, d_hm.p, d_ztab.p, d_flags.p, d_ts.p);
-  LAUNCH_CHECK();
-  k_cloud_assume<<<1, 1, 0, s>>>(d_ts.p, n_tiles);
-  LAUNCH_CHECK();
-  k_cloud_fix<<<tg, tb, 0, s>>>(d_segs.p, d_tiles.p, n_tiles, d_hm.p, d_ztab.p, d_flags.p, d_ts.p);
-  LAUNCH_CHECK();
-  k_cloud_chain<<<1, 1, 0, s>>>(d_segs.p, d_tiles.p, n_tiles, d_hm.p, d_ztab.p, d_flags.p, d_ts.p, d_cs.p);
-  LAUNCH_CHECK();
-  k_cloud_counts<<<tg, tb, 0, s>>>(d_ts.p, n_tiles, d_cnt.p);
-  LAUNCH_CHECK();
-  {
-    size_t tmp_bytes = 0;
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_cnt.p, d_off.p, (int64_t)n_tiles, s));
-    DevArr<unsigned char> tmp;
-    CLOUD_ALLOC(tmp, tmp_bytes, "the tile scan");
-    CK(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, d_cnt.p, d_off.p, (int64_t)n_tiles, s));
-    ctx->stats.launches += 2;
-    unsigned long long last_off = 0, last_cnt = 0;
-    ChainStats cs{};
-    CK(cudaMemcpyAsync(&last_off, d_off.p + n_tiles - 1, sizeof last_off, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(&last_cnt, d_cnt.p + n_tiles - 1, sizeof last_cnt, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(&cs, d_cs.p, sizeof cs, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    *count = last_off + last_cnt;
-    bs.tiles = n_tiles;
-    bs.tiles_rewalked = cs.rewalked;
-    bs.tiles_unconverged = cs.unconverged;
-    bs.tiles_redone = cs.redone;
-  }
-  CK(tm.mark(s));
-  // ---- scatter
-  CLOUD_ALLOC(pos, *count, "the point cloud");
-  CLOUD_ALLOC(val, *count, "the point cloud");
-  k_cloud_scatter<<<(unsigned)(((uint64_t)n_tiles * 32 + 255) / 256), 256, 0, s>>>(d_segs.p, d_tiles.p, n_tiles, d_hm.p,
-                                                                                     d_ztab.p, d_flags.p, d_off.p, pos.p, val.p);
-  LAUNCH_CHECK();
-  CK(tm.mark(s));
-  CK(cudaStreamSynchronize(s));
-  bs.points = *count;
-  bs.ms_upload = tm.ms(0, 1);
-  bs.ms_census = tm.ms(1, 2);
-  bs.ms_levels = tm.ms(2, 3);
-  bs.ms_zsums = tm.ms(3, 4);
-  bs.ms_select = tm.ms(4, 5);
-  bs.ms_scatter = tm.ms(5, 6);
-  return SMB_OK;
-}
-
-namespace {
-struct DevPart {  // one rank's part of the cloud in device memory (host_index.cc PartSink)
-  DevArr<uint64_t> pos, run_off, run_first, w_pos;
-  DevArr<float> val;
-  DevArr<uint8_t> own;
-  DevArr<uint32_t> w_src, w_orig;
-  uint64_t n_values = 0, n_runs = 0, n_windows = 0;
-};
-}  // namespace
-
-// The rank's part of the device cloud; with windows, also the window table of its shard.
-static int part_build(smb_ctx *ctx, const DevArr<uint64_t> &pos, const DevArr<float> &val, uint64_t n,
-                      const uint32_t *owner, uint32_t n_contigs, uint32_t rank, bool windows, DevPart &out) {
-  using namespace cloud;
-  cudaStream_t s = ctx->stream;
-  DevArr<uint32_t> d_owner;
-  CLOUD_ALLOC(d_owner, n_contigs, "the owner table");
-  CK(cudaMemcpyAsync(d_owner.p, owner, n_contigs * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-  const uint64_t nb64 = (n + kPartBlock - 1) / kPartBlock;
-  if (nb64 >= 0x7FFFFFFFull) return fail(ctx, SMB_ERR_CAPACITY, "device index build: cloud too large for one part pass");
-  const uint32_t nb = (uint32_t)std::max<uint64_t>(nb64, 1);
-  DevArr<unsigned long long> blk, cnt3, off3;
-  CLOUD_ALLOC(blk, nb, "the part counters");
-  CLOUD_ALLOC(cnt3, 3 * (size_t)nb, "the part counters");
-  CLOUD_ALLOC(off3, 3 * (size_t)nb + 3, "the part counters");
-  CK(cudaMemsetAsync(blk.p, 0, nb * sizeof(unsigned long long), s));
-  if (n) {
-    k_part_count<<<nb, kPartThreads, 0, s>>>(pos.p, n, d_owner.p, rank, blk.p);
-    LAUNCH_CHECK();
-  }
-  k_part_unpack<<<(nb + 255) / 256, 256, 0, s>>>(blk.p, nb, cnt3.p);
-  LAUNCH_CHECK();
-  size_t tmp_bytes = 0;
-  CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, cnt3.p, off3.p, (int64_t)nb, s));
-  DevArr<unsigned char> tmp;
-  CLOUD_ALLOC(tmp, tmp_bytes, "the part scan");
-  for (int k = 0; k < 3; ++k)
-    CK(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, cnt3.p + (size_t)k * nb, off3.p + (size_t)k * nb, (int64_t)nb, s));
-  ctx->stats.launches += 3;
-  unsigned long long last[6];
-  for (int k = 0; k < 3; ++k) {
-    CK(cudaMemcpyAsync(last + 2 * k, off3.p + (size_t)k * nb + nb - 1, 8, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(last + 2 * k + 1, cnt3.p + (size_t)k * nb + nb - 1, 8, cudaMemcpyDeviceToHost, s));
-  }
-  CK(cudaStreamSynchronize(s));
-  out.n_values = last[0] + last[1];
-  out.n_runs = last[2] + last[3];
-  out.n_windows = last[4] + last[5];
-  CLOUD_ALLOC(out.pos, out.n_values, "the rank's part");
-  CLOUD_ALLOC(out.val, out.n_values, "the rank's part");
-  CLOUD_ALLOC(out.own, out.n_values, "the rank's part");
-  CLOUD_ALLOC(out.run_off, out.n_runs + 1, "the rank's part");
-  CLOUD_ALLOC(out.run_first, out.n_runs, "the rank's part");
-  if (windows) {
-    CLOUD_ALLOC(out.w_pos, out.n_windows, "the shard's windows");
-    CLOUD_ALLOC(out.w_src, out.n_windows, "the shard's windows");
-    CLOUD_ALLOC(out.w_orig, out.n_windows, "the shard's windows");
-  }
-  if (n) {
-    k_part_emit<<<nb, kPartThreads, 0, s>>>(pos.p, val.p, n, d_owner.p, rank, off3.p, nb, out.pos.p, out.val.p,
-                                            out.own.p, out.run_off.p, out.run_first.p, windows ? out.w_pos.p : nullptr,
-                                            out.w_src.p, out.w_orig.p);
-    LAUNCH_CHECK();
-  }
-  const uint64_t end = out.n_values;
-  CK(cudaMemcpyAsync(out.run_off.p + out.n_runs, &end, sizeof end, cudaMemcpyHostToDevice, s));
-  CK(cudaStreamSynchronize(s));
-  return SMB_OK;
-}
-
-// Extent of the points the index sees (build_index's host loop, as device reductions).
-static int cloud_extent(smb_ctx *ctx, const uint64_t *pos, const float *val, uint64_t n, uint32_t n_buckets,
-                        bool fixed_buckets, IndexInput &in) {
-  using namespace cloud;
-  cudaStream_t s = ctx->stream;
-  DevArr<CloudExtent> d_ext;
-  DevArr<unsigned long long> d_span;
-  CLOUD_ALLOC(d_ext, 1, "the cloud extent");
-  CLOUD_ALLOC(d_span, n_buckets, "the cloud extent");
-  const CloudExtent init{0xFFFFFFFFu, 0u, 0u, 0u};
-  CK(cudaMemcpyAsync(d_ext.p, &init, sizeof init, cudaMemcpyHostToDevice, s));
-  CK(cudaMemsetAsync(d_span.p, 0, n_buckets * sizeof(unsigned long long), s));
-  if (n) {
-    const unsigned grid = (unsigned)std::min<uint64_t>((n + 255) / 256, (uint64_t)ctx->n_sm * 8);
-    k_cloud_extent<<<grid, 256, 0, s>>>(pos, val, n, d_ext.p, d_span.p);
-    LAUNCH_CHECK();
-  }
-  CloudExtent ext{};
-  std::vector<uint64_t> span(n_buckets);
-  CK(cudaMemcpyAsync(&ext, d_ext.p, sizeof ext, cudaMemcpyDeviceToHost, s));
-  CK(cudaMemcpyAsync(span.data(), d_span.p, n_buckets * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  in.vmin = n ? ord_val(ext.vmin_ord) : 0.0f;
-  in.vmax = n ? ord_val(ext.vmax_ord) : 0.0f;
-  in.max_tpos = ext.max_tpos;
-  // the host loop sizes the bucket table by the largest bucket seen (a shard: every bucket)
-  in.max_bucket = fixed_buckets ? n_buckets - 1 : ext.max_bucket;
-  span.resize(fixed_buckets ? n_buckets : (n ? (size_t)ext.max_bucket + 1 : 0));
-  in.bucket_span = std::move(span);
-  return SMB_OK;
-}
-
-extern "C" {
-
-int smb_point_cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
-                          const float *level_mean, uint64_t **pos, float **val, size_t *count) {
-  if (!pos || !val || !count) return fail(ctx, SMB_ERR_ARG, "smb_point_cloud_build: null output");
-  *pos = nullptr;
-  *val = nullptr;
-  *count = 0;
-  DevArr<uint64_t> d_pos;
-  DevArr<float> d_val;
-  uint64_t c = 0;
-  int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &c);
-  if (rc) return rc;
-  uint64_t *P = (uint64_t *)malloc(std::max<uint64_t>(c, 1) * sizeof(uint64_t));
-  float *V = (float *)malloc(std::max<uint64_t>(c, 1) * sizeof(float));
-  if (!P || !V) {
-    free(P);
-    free(V);
-    return fail(ctx, SMB_ERR_IO, "smb_point_cloud_build: out of host memory");
-  }
-  cudaError_t e = cudaMemcpy(P, d_pos.p, c * sizeof(uint64_t), cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess) e = cudaMemcpy(V, d_val.p, c * sizeof(float), cudaMemcpyDeviceToHost);
-  if (e != cudaSuccess) {
-    free(P);
-    free(V);
-    return fail(ctx, SMB_ERR_CUDA, std::string("smb_point_cloud_build: ") + cudaGetErrorString(e));
-  }
-  ctx->stats.d2h_bytes += c * 12;
-  *pos = P;
-  *val = V;
-  *count = c;
-  return SMB_OK;
-}
-
-int smb_point_cloud_build_part(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
-                               const float *level_mean, const uint32_t *owner, uint32_t rank, smbh_cloud_part *out) {
-  if (!out) return fail(ctx, SMB_ERR_ARG, "smb_point_cloud_build_part: null output");
-  memset(out, 0, sizeof *out);
-  if (!owner) return fail(ctx, SMB_ERR_ARG, "smb_point_cloud_build_part: null owner table");
-  DevPart part;
-  {
-    DevArr<uint64_t> d_pos;
-    DevArr<float> d_val;
-    uint64_t c = 0;
-    int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &c);
-    if (rc) return rc;
-    rc = part_build(ctx, d_pos, d_val, c, owner, n, rank, false, part);
-    if (rc) return rc;
-    out->n_points_total = c;
-  }
-  out->n_values = part.n_values;
-  out->n_runs = part.n_runs;
-  auto take = [](const void *src, size_t bytes, cudaError_t &e) -> void * {
-    void *p = malloc(bytes ? bytes : 1);
-    if (p && bytes && e == cudaSuccess) e = cudaMemcpy(p, src, bytes, cudaMemcpyDeviceToHost);
-    return p;
-  };
-  cudaError_t e = cudaSuccess;
-  out->pos = (uint64_t *)take(part.pos.p, part.n_values * sizeof(uint64_t), e);
-  out->val = (float *)take(part.val.p, part.n_values * sizeof(float), e);
-  out->own = (uint8_t *)take(part.own.p, part.n_values, e);
-  out->run_off = (uint64_t *)take(part.run_off.p, (part.n_runs + 1) * sizeof(uint64_t), e);
-  out->run_first = (uint64_t *)take(part.run_first.p, part.n_runs * sizeof(uint64_t), e);
-  if (!out->pos || !out->val || !out->own || !out->run_off || !out->run_first || e != cudaSuccess) {
-    smbh_cloud_part_free(out);
-    return e != cudaSuccess ? fail(ctx, SMB_ERR_CUDA, std::string("smb_point_cloud_build_part: ") + cudaGetErrorString(e))
-                            : fail(ctx, SMB_ERR_IO, "smb_point_cloud_build_part: out of host memory");
-  }
-  return SMB_OK;
-}
-
-int smb_index_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
-                    const float *level_mean, const uint32_t *contig_owner) {
-  CK(cudaSetDevice(ctx->device));
-  if (contig_owner) {
-    if (!ctx->ex) return fail(ctx, SMB_ERR_STATE, "join a shard group first (smb_shard_local_group / smb_shard_nccl_init)");
-    if (!n) return fail(ctx, SMB_ERR_ARG, "smb_index_build: no contigs");
-    for (uint32_t c = 0; c < n; ++c)
-      if (contig_owner[c] >= (uint32_t)ctx->ex->world) return fail(ctx, SMB_ERR_ARG, "contig owner out of range");
-  }
-  DevArr<uint64_t> d_pos;
-  DevArr<float> d_val;
-  uint64_t N = 0;
-  int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &N);
-  if (rc) return rc;
-  if (N < (uint64_t)kDim) return fail(ctx, SMB_ERR_ARG, "point cloud smaller than the index dimension");
-  StageTimer tm;
-  CK(tm.mark(ctx->stream));
-  const uint64_t W_all = N - (kDim - 1);
-  if (!contig_owner) {
-    if (W_all > 0xFFFFFFF0ull) return fail(ctx, SMB_ERR_CAPACITY, "more than 2^32 window points: shard the index by contig");
-    IndexInput in{d_val.p, d_pos.p, nullptr, nullptr, W_all, (size_t)N, 0.0f, 0.0f, 0u, 0u, {}};
-    rc = cloud_extent(ctx, d_pos.p, d_val.p, N, 2 * n, false, in);
-    if (!rc) rc = build_index_core(ctx, in);
-    ctx->index_sharded = false;
-  } else {
-    const uint32_t rank = (uint32_t)ctx->ex->rank;
-    DevPart part;
-    rc = part_build(ctx, d_pos, d_val, N, contig_owner, n, rank, true, part);
-    if (rc) return rc;
-    d_pos.reset();  // the rank keeps its part only
-    d_val.reset();
-    if (part.n_values > 0xFFFFFFF0ull)
-      return fail(ctx, SMB_ERR_CAPACITY, "more than 2^32 window points on one shard: use more ranks");
-    IndexInput in{part.val.p, part.w_pos.p, part.w_src.p, part.w_orig.p, part.n_windows, (size_t)N, 0.0f, 0.0f, 0u, 0u, {}};
-    rc = cloud_extent(ctx, part.pos.p, part.val.p, part.n_values, 2 * n, true, in);
-    if (rc) return rc;
-    if (part.n_windows == 0) {  // a rank may own nothing (more ranks than contigs): one padding leaf
-      const float pad[kDim] = {kPadValue, kPadValue, kPadValue, kPadValue, kPadValue, kPadValue};
-      const uint64_t pad_pos = ~0ull;
-      const uint32_t zero = 0, none = 0xFFFFFFFFu;
-      CLOUD_ALLOC(part.val, kDim, "the padding leaf");
-      CLOUD_ALLOC(part.w_pos, 1, "the padding leaf");
-      CLOUD_ALLOC(part.w_src, 1, "the padding leaf");
-      CLOUD_ALLOC(part.w_orig, 1, "the padding leaf");
-      CK(cudaMemcpy(part.val.p, pad, sizeof pad, cudaMemcpyHostToDevice));
-      CK(cudaMemcpy(part.w_pos.p, &pad_pos, 8, cudaMemcpyHostToDevice));
-      CK(cudaMemcpy(part.w_src.p, &zero, 4, cudaMemcpyHostToDevice));
-      CK(cudaMemcpy(part.w_orig.p, &none, 4, cudaMemcpyHostToDevice));
-      in.val = part.val.p;
-      in.pos = part.w_pos.p;
-      in.wsrc = part.w_src.p;
-      in.worig = part.w_orig.p;
-      in.W = 1;
-    }
-    rc = build_index_core(ctx, in);
-    ctx->index_sharded = rc == SMB_OK;
-  }
-  CK(tm.mark(ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  ctx->build_stats.ms_index = tm.ms(0, 1);
-  return rc;
-}
-
-int smb_index_build_stats(smb_ctx *ctx, smb_build_stats *out) {
-  if (!out) return fail(ctx, SMB_ERR_ARG, "smb_index_build_stats: null output");
-  *out = ctx->build_stats;
   return SMB_OK;
 }
 
