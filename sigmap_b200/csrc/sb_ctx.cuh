@@ -97,7 +97,7 @@ struct DeviceIndex : IndexScalars {
 
 struct smb_ctx {
   int device = 0;
-  cudaStream_t stream = nullptr;
+  Stream stream;
   std::string err;
   // index
   bool has_index = false;
@@ -114,19 +114,18 @@ struct smb_ctx {
   int pipeline_mode = 0;          // SMB_PIPELINE=auto|on|off: wave-pipelined ticks (see map_uploaded_impl)
   uint32_t cloud_tile = 16384;    // SMB_CLOUD_TILE=n: window starts per tile of the device cloud's point selection
   smb_build_stats build_stats{};  // the last device cloud build (smb_index_build_stats)
-  unsigned char *h_cloud_stage = nullptr;  // pinned: two upload slices of the device cloud build
+  PinnedBuf<unsigned char> h_cloud_stage;  // two upload slices of the device cloud build
   uint32_t sort_queries_min = 200000;  // SMB_SORT_QUERIES_MIN=n: batches with fewer queries keep their natural order
   unsigned dp_grid = 148 * 8;     // persistent DP grid: every block that fits on the device
   bool part_sort = true;          // SMB_SORT=entry: always the one-CTA-per-entry sort (k_seg_sort)
   bool seg_sort = true;           // per-entry shared-memory sort; SMB_SORT=global forces the radix sort
-  cudaStream_t stream_cp = nullptr;  // smb_map_reads: upload slices (copy + K1 filter) run here, under the mapping
-  std::vector<cudaEvent_t> slice_events;
+  Stream stream_cp;  // smb_map_reads: upload slices (copy + K1 filter) run here, under the mapping
+  std::vector<Event> slice_events;
   size_t upload_slice_bytes = 64u << 20;  // SMB_UPLOAD_SLICE_MB=n
-  uint32_t *h_kept_pinned = nullptr;      // kept length of every read, written by the device (pinned)
-  size_t h_kept_pinned_cap = 0;
-  cudaStream_t stream_ev = nullptr;  // lookahead event blocks run here, next to the mapping rounds
-  cudaEvent_t ev_blk_t0[2] = {}, ev_blk_t1[2] = {};
-  cudaEvent_t ev_cp[2] = {};         // first / last filter-only slice of a wave-pipelined call (copy stream)
+  PinnedBuf<uint32_t> h_kept_pinned;  // kept length of every read, written by the device
+  Stream stream_ev;  // lookahead event blocks run here, next to the mapping rounds
+  Event ev_blk_t0[2], ev_blk_t1[2];
+  Event ev_cp[2];  // first / last filter-only slice of a wave-pipelined call (copy stream)
   bool ev_overlap = true;            // SMB_EVENTS_OVERLAP=0: compute every block when it is needed
   double ev_survival_hint = 0.0;     // share of reads that went past their first chunk in the last call
   uint32_t ev_warp_max = 2048;    // event batches up to this many chunks run warp-per-chunk in shared memory
@@ -145,10 +144,10 @@ struct smb_ctx {
   // work
   Workspace ws;
   SlotSpace map_slots;
-  Counters *d_ctr = nullptr;
-  Counters *h_ctr = nullptr;  // pinned
-  cudaEvent_t ev[8] = {};
-  cudaEvent_t timer[2] = {};
+  DevBuf<Counters> d_ctr;
+  PinnedBuf<Counters> h_ctr;
+  Event ev[8];
+  Event timer[2];
   smb_stats stats{};
   uint32_t max_batch_chunks = 32768;
   uint64_t max_batch_anchors = 640ull << 20;  // x 32 B of sort/DP buffers = 20 GB of the 180 GB HBM
@@ -159,10 +158,10 @@ struct smb_ctx {
   // contig-sharded index: the exchange backend (null = this context holds every contig)
   std::unique_ptr<Exchange> ex;
   std::shared_ptr<LocalGroup> local_group;
-  double *h_ctl = nullptr;  // pinned, 4 doubles
+  PinnedBuf<double> h_ctl;  // 4 doubles
   bool group_at_limit = false;
   // streaming
-  SlotSpace *stream_slots = nullptr;
+  std::unique_ptr<SlotSpace> stream_slots;
   smb_params stream_params{};
   std::vector<std::vector<int16_t>> stream_pending;  // kept samples not yet forming a chunk
   std::vector<float> stream_offset, stream_scale;
@@ -171,8 +170,7 @@ struct smb_ctx {
   // conversion is monotone in the raw value); lo > hi: nothing kept; generic: test every sample
   std::vector<int32_t> stream_lo, stream_hi;
   std::vector<uint8_t> stream_generic;
-  int16_t *h_stream_stage = nullptr;  // pinned: this round's chunks, channel after channel
-  size_t h_stream_stage_cap = 0;
+  PinnedBuf<int16_t> h_stream_stage;  // this round's chunks, channel after channel
   DevBuf<int16_t> d_stream_stage;
 };
 

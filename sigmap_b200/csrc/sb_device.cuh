@@ -10,8 +10,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <cstring>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/sigmap_b200.h"
@@ -44,27 +46,85 @@ inline void dev_free(void *q) {
   else cudaFree(q);
 }
 
-// growable device buffer (contents are NOT preserved across growth)
-template <class T>
-struct DevBuf {
+struct DeviceMem {
+  static cudaError_t alloc(void **q, size_t bytes) { return cudaMalloc(q, bytes); }
+  static void free(void *q) { dev_free(q); }
+};
+struct PinnedMem {
+  static cudaError_t alloc(void **q, size_t bytes) { return cudaMallocHost(q, bytes); }
+  static void free(void *q) { cudaFreeHost(q); }
+};
+
+// An array that frees itself: device memory (DevBuf) or pinned host memory (PinnedBuf).  Move-only.
+// The destructor frees on the current device, so an owner must be destroyed with its context's
+// device current: every entry point calls cudaSetDevice first, and smb_destroy / smb_batch_destroy
+// do so before they delete.  cudaFree waits for the work queued on the device, so a buffer that goes
+// out of scope on an error return waits for that work as an explicit release() would.
+template <class T, class Mem>
+struct Buf {
   T *p = nullptr;
-  size_t cap = 0;
+  size_t cap = 0;  // elements
+  Buf() = default;
+  Buf(const Buf &) = delete;
+  Buf &operator=(const Buf &) = delete;
+  Buf(Buf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+  Buf &operator=(Buf &&o) noexcept {
+    if (this != &o) {
+      release();
+      p = std::exchange(o.p, nullptr);
+      cap = std::exchange(o.cap, 0);
+    }
+    return *this;
+  }
+  ~Buf() { release(); }
+  // at least n elements, with room to grow (contents are NOT preserved across growth)
   cudaError_t ensure(size_t n) {
     if (n <= cap) return cudaSuccess;
-    if (p) dev_free(p);
+    const size_t want = n + n / 4 + 64;
+    return take(want, want);
+  }
+  // exactly n elements (one when n = 0, so that p is a valid pointer)
+  cudaError_t alloc(size_t n) { return take(std::max<size_t>(n, 1), n); }
+  void release() {
+    if (p) Mem::free(p);
     p = nullptr;
     cap = 0;
-    size_t want = n + n / 4 + 64;
-    cudaError_t e = cudaMalloc((void **)&p, want * sizeof(T));
-    if (e == cudaSuccess) cap = want;
+  }
+
+ private:
+  cudaError_t take(size_t elems, size_t n) {
+    release();
+    const cudaError_t e = Mem::alloc((void **)&p, elems * sizeof(T));
+    if (e != cudaSuccess) {
+      p = nullptr;
+      cudaGetLastError();  // an out-of-memory return is not sticky: clear it, or the next launch check reports it
+      return e;
+    }
+    cap = n;
     return e;
   }
-  void release() {
-    if (p) dev_free(p);
-    p = nullptr;
-    cap = 0;
-  }
 };
+template <class T>
+using DevBuf = Buf<T, DeviceMem>;
+template <class T>
+using PinnedBuf = Buf<T, PinnedMem>;
+
+// A stream or an event that destroys itself.  Create it with cudaStreamCreate*(&s.h) /
+// cudaEventCreate*(&e.h); it converts to the raw handle.  Same device rule as Buf.
+template <class H, cudaError_t (*Destroy)(H)>
+struct Handle {
+  H h = nullptr;
+  Handle() = default;
+  Handle(const Handle &) = delete;
+  Handle &operator=(const Handle &) = delete;
+  Handle(Handle &&o) noexcept : h(std::exchange(o.h, nullptr)) {}
+  ~Handle() {
+    if (h) Destroy(h);
+  }
+  operator H() const { return h; }
+};
+using Stream = Handle<cudaStream_t, cudaStreamDestroy>;
+using Event = Handle<cudaEvent_t, cudaEventDestroy>;
 
 // ---- flat device index over the ordered window points (replaces nanoflann) ----
 // Leaves hold 8 consecutive points of the point order (aligned KD order, k_index.cuh); a node

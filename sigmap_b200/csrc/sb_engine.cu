@@ -204,7 +204,7 @@ static int launch_search(smb_ctx *ctx, SearchArgs sa, uint32_t nq_max, cudaStrea
   Workspace &w = ctx->ws;
   const size_t gsm = search_smem(ctx);
   if (!ctx->search_lean || nq_max == 0) {
-    sa.work = &ctx->d_ctr->work;
+    sa.work = &ctx->d_ctr.p->work;
     k_radius_search<STAGE><<<STAGE ? search_grid<true>(ctx) : ctx->search_grid_main, kSearchWarps * 32, gsm, s>>>(ctx->index.ix, sa);
     LAUNCH_CHECK();
     return SMB_OK;
@@ -249,14 +249,14 @@ static int launch_search(smb_ctx *ctx, SearchArgs sa, uint32_t nq_max, cudaStrea
   sa.entry_info = w.entry_info.p;
   sa.front_cap = std::min<uint32_t>(std::max<uint32_t>(ctx->front_cap, 72u), (uint32_t)kFrontCap);
   sa.ovf_list = w.ovf_list.p;
-  sa.work = &ctx->d_ctr->work;
+  sa.work = &ctx->d_ctr.p->work;
   k_search_lean<STAGE><<<ctx->n_sm, kLeanWarps * 32, lean_smem(ctx->index.ix.smem_bytes, sa.stage_cap), s>>>(ctx->index.ix, sa);
   LAUNCH_CHECK();
   // the queries whose frontier outgrew the lean kernel's slots (none, mostly: the launch then
   // finds an empty list and returns)
   sa.qlist = w.ovf_list.p;
-  sa.qlist_n = &ctx->d_ctr->n_overflow;
-  sa.work = &ctx->d_ctr->work2;
+  sa.qlist_n = &ctx->d_ctr.p->n_overflow;
+  sa.work = &ctx->d_ctr.p->work2;
   k_radius_search<STAGE><<<STAGE ? search_grid<true>(ctx) : ctx->search_grid_main, kSearchWarps * 32, gsm, s>>>(ctx->index.ix, sa);
   LAUNCH_CHECK();
   return SMB_OK;
@@ -309,7 +309,7 @@ static int run_events(smb_ctx *ctx, StepSource src, const void *samples, uint32_
     float *feat = d_features ? d_features : w.features.p;
     uint32_t *nfeat = d_n_features ? d_n_features : w.n_features.p;
     uint32_t *nraw = d_n_raw ? d_n_raw : w.n_raw_events.p;
-    Counters *ctr = d_n_raw ? nullptr : ctx->d_ctr;
+    Counters *ctr = d_n_raw ? nullptr : ctx->d_ctr.p;
     if (src == SRC_RAW_KEPT)
       k_ev_chunk_warp<true><<<B, 32, kEvWarpSmem, s>>>(samples, ct.start, ct.offset, ct.scale,
                                                        w.means.p, feat, nfeat, nraw, nullptr, B, ctr);
@@ -336,7 +336,7 @@ static int run_events(smb_ctx *ctx, StepSource src, const void *samples, uint32_
                                                 d_features ? d_features : w.features.p,
                                                 d_n_features ? d_n_features : w.n_features.p,
                                                 d_n_raw ? d_n_raw : w.n_raw_events.p, d_peaks_out, B, Bp,
-                                                d_n_raw ? nullptr : ctx->d_ctr);
+                                                d_n_raw ? nullptr : ctx->d_ctr.p);
   LAUNCH_CHECK();
   return SMB_OK;
 }
@@ -388,13 +388,9 @@ static cudaError_t grow_keep(DevBuf<T> &buf, size_t want, cudaStream_t s) {
   if (buf.p && buf.cap) {
     e = cudaMemcpyAsync(bigger.p, buf.p, buf.cap * sizeof(T), cudaMemcpyDeviceToDevice, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess) {
-      bigger.release();
-      return e;
-    }
+    if (e != cudaSuccess) return e;
   }
-  buf.release();
-  buf = bigger;
+  buf = std::move(bigger);
   return cudaSuccess;
 }
 
@@ -448,7 +444,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     ctx->stats.h2d_bytes += B * sizeof(uint32_t);
   }
   CK(cudaEventRecord(ctx->ev[0], s));
-  k_reset_step<<<1, 1, 0, s>>>(ctx->d_ctr);
+  k_reset_step<<<1, 1, 0, s>>>(ctx->d_ctr.p);
   LAUNCH_CHECK();
   CK(cudaMemsetAsync(w.n_features.p, 0, B * sizeof(uint32_t), s));
   if (Bpres > 0) {
@@ -457,7 +453,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
       LAUNCH_CHECK();
     } else if (src == SRC_CACHED) {
       k_gather_nfeat<<<(Bpres + 255) / 256, 256, 0, s>>>(w.nf_cache[w.cache_cur].p, w.nraw_cache[w.cache_cur].p, w.feat_row.p, Bpres,
-                                                         w.n_features.p, ctx->d_ctr);
+                                                         w.n_features.p, ctx->d_ctr.p);
       LAUNCH_CHECK();
     } else {
       CK(w.chunk_start.ensure(Bpres));
@@ -476,7 +472,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     }
   }
   CK(cudaEventRecord(ctx->ev[1], s));
-  k_query_table<<<1, 1024, 0, s>>>(w.n_features.p, B, Bpres, prm.step_size, w.n_queries.p, w.q_off.p, ctx->d_ctr);
+  k_query_table<<<1, 1024, 0, s>>>(w.n_features.p, B, Bpres, prm.step_size, w.n_queries.p, w.q_off.p, ctx->d_ctr.p);
   LAUNCH_CHECK();
 
   // ---- anchors: carried ones first, then the radius search appends its hits
@@ -530,7 +526,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   LAUNCH_CHECK();
   k_inject_carry<<<(B * 32 + kCarryThreads - 1) / kCarryThreads, kCarryThreads, 0, s>>>(
       w.entry_slot.p, w.n_queries.p, sp.slots.p, sp.pool_anchor[0].p, sp.pool_anchor[1].p, B, kl, w.key_a.p,
-      w.dist_a.p, cap, ctx->d_ctr, want_seg ? w.runs.p : nullptr, w.run_count.p, w.entry_total.p,
+      w.dist_a.p, cap, ctx->d_ctr.p, want_seg ? w.runs.p : nullptr, w.run_count.p, w.entry_total.p,
       runs_cap, n_parts, inv_span, ctx->index.bucket_base.p, w.seg_qmin.p);
   LAUNCH_CHECK();
   SearchArgs sa{};
@@ -547,7 +543,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   sa.out_key = w.key_a.p;
   sa.out_dist = w.dist_a.p;
   sa.cap = cap;
-  sa.ctr = ctx->d_ctr;
+  sa.ctr = ctx->d_ctr.p;
   sa.runs = want_seg ? w.runs.p : nullptr;
   sa.run_count = w.run_count.p;
   sa.entry_total = w.entry_total.p;
@@ -568,38 +564,38 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   ctx->stats.search_launches++;
   CK(cudaEventRecord(ctx->ev[3], s));
   if (want_seg) {
-    k_max_u32<<<148, 256, 0, s>>>(w.entry_total.p, n_lists, &ctx->d_ctr->max_entry_anchors);
+    k_max_u32<<<148, 256, 0, s>>>(w.entry_total.p, n_lists, &ctx->d_ctr.p->max_entry_anchors);
     LAUNCH_CHECK();
   }
   if (sharded) {
     // Sharded: every rank must take the same path through this step (the exchanges below are
     // collective), so overflow and the estimate are agreed on first -- with a host round trip.
-    CK(cudaMemcpyAsync(ctx->h_ctr, ctx->d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(ctx->h_ctr.p, ctx->d_ctr.p, sizeof(Counters), cudaMemcpyDeviceToHost, s));
     int rc = host_sync(ctx);
     if (rc) return rc;
     ctx->stats.d2h_bytes += sizeof(Counters);
-    const unsigned long long n_local = ctx->h_ctr->n_anchors;
+    const unsigned long long n_local = ctx->h_ctr.p->n_anchors;
     const bool overflow_local = n_local > cap;
     CK(w.ctl.ensure(4));
-    ctx->h_ctl[0] = overflow_local ? 1.0 : 0.0;
-    ctx->h_ctl[1] = (overflow_local && ctx->last_cap >= ctx->max_batch_anchors) ? 1.0 : 0.0;
-    ctx->h_ctl[2] = (double)n_local;
-    ctx->h_ctl[3] = (ctx->h_ctr->error & 64u) ? 1.0 : 0.0;
-    CK(cudaMemcpyAsync(w.ctl.p, ctx->h_ctl, 4 * sizeof(double), cudaMemcpyHostToDevice, s));
+    ctx->h_ctl.p[0] = overflow_local ? 1.0 : 0.0;
+    ctx->h_ctl.p[1] = (overflow_local && ctx->last_cap >= ctx->max_batch_anchors) ? 1.0 : 0.0;
+    ctx->h_ctl.p[2] = (double)n_local;
+    ctx->h_ctl.p[3] = (ctx->h_ctr.p->error & 64u) ? 1.0 : 0.0;
+    CK(cudaMemcpyAsync(w.ctl.p, ctx->h_ctl.p, 4 * sizeof(double), cudaMemcpyHostToDevice, s));
     rc = ctx->ex->allreduce(w.ctl.p, 4, EX_F64, EX_MAX, s, ctx->err);
     if (rc) return rc;
-    CK(cudaMemcpyAsync(ctx->h_ctl, w.ctl.p, 4 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(ctx->h_ctl.p, w.ctl.p, 4 * sizeof(double), cudaMemcpyDeviceToHost, s));
     rc = host_sync(ctx);
     if (rc) return rc;
     ctx->stats.exchanges++;
-    ctx->group_at_limit = ctx->h_ctl[1] > 0.0;
-    if (ctx->h_ctl[3] > 0.0) {  // some rank ran out of query-order slots: everybody redoes the step
+    ctx->group_at_limit = ctx->h_ctl.p[1] > 0.0;
+    if (ctx->h_ctl.p[3] > 0.0) {  // some rank ran out of query-order slots: everybody redoes the step
       ctx->est_queries_per_chunk = 1.1 * (double)q_per_chunk_max;
       return 2;
     }
-    if (ctx->h_ctl[0] > 0.0) return 1;  // nothing has been committed to the slots yet
+    if (ctx->h_ctl.p[0] > 0.0) return 1;  // nothing has been committed to the slots yet
   }
-  k_step_check<<<1, 1, 0, s>>>(ctx->d_ctr, cap, mode, 8u * (unsigned)kPartSortCap, 8ull * (unsigned)kSortCapBig, n_parts);
+  k_step_check<<<1, 1, 0, s>>>(ctx->d_ctr.p, cap, mode, 8u * (unsigned)kPartSortCap, 8ull * (unsigned)kSortCapBig, n_parts);
   LAUNCH_CHECK();
 
   // ---- sort by (entry, bucket, target, query)
@@ -628,7 +624,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     ps.kl = kl;
     ps.bucket_base = ctx->index.bucket_base.p;
     ps.n_buckets = ctx->index.max_bucket + 1u;
-    ps.ctr = ctx->d_ctr;
+    ps.ctr = ctx->d_ctr.p;
     k_part_sort<kPartSortCap, 512, 4096><<<(unsigned)n_lists, 512, part_sort_smem_bytes(kPartSortCap, 4096), s>>>(ps);
     LAUNCH_CHECK();
   } else if (mode == SORT_SEG) {
@@ -647,14 +643,14 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     ss.bucket_base = ctx->index.bucket_base.p;
     ss.gshift = ctx->index.gshift;
     ss.n_coarse = ctx->index.n_coarse;
-    ss.ctr = ctx->d_ctr;
+    ss.ctr = ctx->d_ctr.p;
     k_seg_sort<kSortCapBig, 1024, 8192><<<B, 1024, sort_smem_bytes(kSortCapBig, 8192), s>>>(ss);
     LAUNCH_CHECK();
   } else {
     // radix sort on (entry, bucket, target) only; k_fix_ties orders equal-target runs by query.
     // The sort is sized for the buffers (the count lives on the device): the slots past the
     // step's anchors are filled with the largest key and stay at the end.
-    k_pad_keys<<<(unsigned)((cap + 255) / 256), 256, 0, s>>>(w.key_a.p, ctx->d_ctr, cap);
+    k_pad_keys<<<(unsigned)((cap + 255) / 256), 256, 0, s>>>(w.key_a.p, ctx->d_ctr.p, cap);
     LAUNCH_CHECK();
     size_t tb = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, tb, w.key_a.p, w.key_b.p, w.dist_a.p, w.dist_b.p,
@@ -663,7 +659,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     CK(cub::DeviceRadixSort::SortPairs(w.cub_temp.p, tb, w.key_a.p, w.key_b.p, w.dist_a.p, w.dist_b.p,
                                        (uint64_t)cap, kl.qbits, 64, s));
     ctx->stats.launches += 2 + (64 - kl.qbits + 7) / 8;
-    k_fix_ties<<<(unsigned)((cap + 255) / 256), 256, 0, s>>>(w.key_b.p, w.dist_b.p, ctx->d_ctr, kl.qbits);
+    k_fix_ties<<<(unsigned)((cap + 255) / 256), 256, 0, s>>>(w.key_b.p, w.dist_b.p, ctx->d_ctr.p, kl.qbits);
     LAUNCH_CHECK();
   }
   CK(cudaEventRecord(ctx->ev[5], s));
@@ -684,7 +680,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   CK(w.seg_max.ensure(ca.n_slots));
   ca.seg = w.seg.p;
   ca.seg_max = w.seg_max.p;
-  ca.ctr = ctx->d_ctr;
+  ca.ctr = ctx->d_ctr.p;
   ca.dp_passes = ctx->dp_passes;
   CK(cudaMemsetAsync(w.seg.p, 0xFF, (size_t)ca.n_slots * sizeof(SegRec), s));
   CK(cudaMemsetAsync(w.seg_max.p, 0, (size_t)ca.n_slots * sizeof(float), s));
@@ -749,7 +745,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     // exchange 3: candidate counts, then the candidate records padded to the largest count
     const uint32_t world = (uint32_t)ctx->ex->world;
     CK(w.cand_counts.ensure(world + 1));
-    int rc = ctx->ex->allgather(&ctx->d_ctr->n_cand, w.cand_counts.p, sizeof(unsigned long long), s, ctx->err);
+    int rc = ctx->ex->allgather(&ctx->d_ctr.p->n_cand, w.cand_counts.p, sizeof(unsigned long long), s, ctx->err);
     if (rc) return rc;
     std::vector<unsigned long long> h_counts(world);
     CK(cudaMemcpyAsync(h_counts.data(), w.cand_counts.p, world * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
@@ -776,11 +772,11 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   const unsigned final_blocks = (unsigned)(((uint64_t)B * 32 + kFinalThreads - 1) / kFinalThreads);
   k_sel_pick<<<final_blocks, kFinalThreads, 0, s>>>(se, w.pick.p);
   LAUNCH_CHECK();
-  k_pool_check<<<1, 1, 0, s>>>(ctx->d_ctr, out_pool, se.pool_chain_cap, se.pool_anchor_cap);
+  k_pool_check<<<1, 1, 0, s>>>(ctx->d_ctr.p, out_pool, se.pool_chain_cap, se.pool_anchor_cap);
   LAUNCH_CHECK();
   if (sharded) {
     // a rank-local abort (sort path, carry pools) becomes everybody's: all ranks redo the step
-    int rc = ctx->ex->allreduce(&ctx->d_ctr->abort, 1, EX_U32, EX_MAX, s, ctx->err);
+    int rc = ctx->ex->allreduce(&ctx->d_ctr.p->abort, 1, EX_U32, EX_MAX, s, ctx->err);
     if (rc) return rc;
     ctx->stats.exchanges++;
   }
@@ -788,7 +784,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   LAUNCH_CHECK();
   CK(cudaEventRecord(ctx->ev[6], s));
   // ---- the step's one look at the device: counters, and what the round wants read back
-  CK(cudaMemcpyAsync(ctx->h_ctr, ctx->d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(ctx->h_ctr.p, ctx->d_ctr.p, sizeof(Counters), cudaMemcpyDeviceToHost, s));
   ctx->stats.d2h_bytes += sizeof(Counters);
   uint32_t n_ids = 0;
   if (rout && rout->ids && rout->info) {
@@ -816,7 +812,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
     int rc = host_sync(ctx);
     if (rc) return rc;
   }
-  const Counters &hc = *ctx->h_ctr;
+  const Counters &hc = *ctx->h_ctr.p;
   if (hc.abort) {
     // nothing was committed; adjust what was too small and let the caller run the step again
     if (hc.abort & kAbortAnchors) return 1;
@@ -863,7 +859,7 @@ static int run_step(smb_ctx *ctx, SlotSpace &sp, const StepEntries &en, StepSour
   if (hc.error & 32u) return fail(ctx, SMB_ERR_CAPACITY, "chain candidate exchange list overflow");
   if (Bpres) {
     double n_est = (double)n;
-    if (sharded) n_est = std::max(n_est, ctx->h_ctl[2]);
+    if (sharded) n_est = std::max(n_est, ctx->h_ctl.p[2]);
     ctx->est_anchors_per_chunk = 0.5 * ctx->est_anchors_per_chunk + 0.5 * (n_est / Bpres);
     ctx->est_queries_per_chunk = std::max(0.9 * ctx->est_queries_per_chunk, (double)hc.n_queries / Bpres);
   }
@@ -887,14 +883,6 @@ static int slots_init(smb_ctx *ctx, SlotSpace &sp, uint32_t n_slots) {
   return SMB_OK;
 }
 
-static void slots_release(SlotSpace &sp) {
-  sp.slots.release();
-  for (int p = 0; p < 2; ++p) {
-    sp.pool_chain[p].release();
-    sp.pool_anchor[p].release();
-  }
-}
-
 // prepare the out pool of a round: capacity for every participating slot, counters zeroed
 static int round_begin(smb_ctx *ctx, SlotSpace &sp, const std::vector<uint32_t> &slots, int step,
                        uint32_t out_pool) {
@@ -910,9 +898,9 @@ static int round_begin(smb_ctx *ctx, SlotSpace &sp, const std::vector<uint32_t> 
   CK(sp.pool_chain[out_pool].ensure(need_chain + 64));
   if (!sp.pool_anchor[1 - out_pool].p) CK(sp.pool_anchor[1 - out_pool].ensure(64));
   if (!sp.pool_chain[1 - out_pool].p) CK(sp.pool_chain[1 - out_pool].ensure(64));
-  CK(cudaMemsetAsync(&ctx->d_ctr->carry_anchor_used[out_pool], 0, sizeof(unsigned long long), ctx->stream));
-  CK(cudaMemsetAsync(&ctx->d_ctr->carry_chain_used[out_pool], 0, sizeof(unsigned long long), ctx->stream));
-  CK(cudaMemsetAsync(&ctx->d_ctr->error, 0, sizeof(unsigned int), ctx->stream));
+  CK(cudaMemsetAsync(&ctx->d_ctr.p->carry_anchor_used[out_pool], 0, sizeof(unsigned long long), ctx->stream));
+  CK(cudaMemsetAsync(&ctx->d_ctr.p->carry_chain_used[out_pool], 0, sizeof(unsigned long long), ctx->stream));
+  CK(cudaMemsetAsync(&ctx->d_ctr.p->error, 0, sizeof(unsigned int), ctx->stream));
   return SMB_OK;
 }
 
@@ -1137,16 +1125,15 @@ int smb_create(smb_ctx **out, int device) {
     return SMB_ERR_CUDA;
   };
   if ((e = cudaSetDevice(device)) != cudaSuccess) return bail("cudaSetDevice", e);
-  if ((e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess)
+  if ((e = cudaStreamCreateWithFlags(&ctx->stream.h, cudaStreamNonBlocking)) != cudaSuccess)
     return bail("cudaStreamCreate", e);
-  if ((e = cudaMalloc((void **)&ctx->d_ctr, sizeof(Counters))) != cudaSuccess) return bail("cudaMalloc", e);
-  if ((e = cudaMemset(ctx->d_ctr, 0, sizeof(Counters))) != cudaSuccess) return bail("cudaMemset", e);
-  if ((e = cudaMallocHost((void **)&ctx->h_ctr, sizeof(Counters))) != cudaSuccess) return bail("cudaMallocHost", e);
-  if ((e = cudaMallocHost((void **)&ctx->h_ctl, 4 * sizeof(double))) != cudaSuccess) return bail("cudaMallocHost", e);
+  if ((e = ctx->d_ctr.alloc(1)) != cudaSuccess) return bail("cudaMalloc", e);
+  if ((e = cudaMemset(ctx->d_ctr.p, 0, sizeof(Counters))) != cudaSuccess) return bail("cudaMemset", e);
+  if ((e = ctx->h_ctr.alloc(1)) != cudaSuccess || (e = ctx->h_ctl.alloc(4)) != cudaSuccess) return bail("cudaMallocHost", e);
   for (auto &ev : ctx->ev)
-    if ((e = cudaEventCreate(&ev)) != cudaSuccess) return bail("cudaEventCreate", e);
+    if ((e = cudaEventCreate(&ev.h)) != cudaSuccess) return bail("cudaEventCreate", e);
   for (auto &ev : ctx->timer)
-    if ((e = cudaEventCreate(&ev)) != cudaSuccess) return bail("cudaEventCreate", e);
+    if ((e = cudaEventCreate(&ev.h)) != cudaSuccess) return bail("cudaEventCreate", e);
   // the per-entry sort keeps a whole part of an entry in shared memory (200 KB of the 227 KB)
   if ((e = cudaFuncSetAttribute(k_seg_sort<kSortCapBig, 1024, 8192>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)sort_smem_bytes(kSortCapBig, 8192))) != cudaSuccess)
@@ -1186,12 +1173,12 @@ int smb_create(smb_ctx **out, int device) {
       (e = cudaFuncSetAttribute(k_ev_chunk_warp<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)kEvWarpSmem)) != cudaSuccess)
     return bail("cudaFuncSetAttribute(k_ev_chunk_warp)", e);
-  if ((e = cudaStreamCreateWithFlags(&ctx->stream_ev, cudaStreamNonBlocking)) != cudaSuccess ||
-      (e = cudaStreamCreateWithFlags(&ctx->stream_cp, cudaStreamNonBlocking)) != cudaSuccess)
+  if ((e = cudaStreamCreateWithFlags(&ctx->stream_ev.h, cudaStreamNonBlocking)) != cudaSuccess ||
+      (e = cudaStreamCreateWithFlags(&ctx->stream_cp.h, cudaStreamNonBlocking)) != cudaSuccess)
     return bail("cudaStreamCreate", e);
   for (int c = 0; c < 2; ++c)
-    if ((e = cudaEventCreate(&ctx->ev_blk_t0[c])) != cudaSuccess || (e = cudaEventCreate(&ctx->ev_blk_t1[c])) != cudaSuccess ||
-        (e = cudaEventCreate(&ctx->ev_cp[c])) != cudaSuccess)
+    if ((e = cudaEventCreate(&ctx->ev_blk_t0[c].h)) != cudaSuccess || (e = cudaEventCreate(&ctx->ev_blk_t1[c].h)) != cudaSuccess ||
+        (e = cudaEventCreate(&ctx->ev_cp[c].h)) != cudaSuccess)
       return bail("cudaEventCreate", e);
   *out = ctx;
   return SMB_OK;
@@ -1201,41 +1188,9 @@ void smb_destroy(smb_ctx *ctx) {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
-  if (ctx->stream_ev) cudaStreamSynchronize(ctx->stream_ev);
-  if (ctx->stream_cp) cudaStreamSynchronize(ctx->stream_cp);
+  cudaStreamSynchronize(ctx->stream_ev);
+  cudaStreamSynchronize(ctx->stream_cp);
   smb_stream_close(ctx);
-  slots_release(ctx->map_slots);
-  Workspace &w = ctx->ws;
-  w.entry_slot.release(); w.n_features.release(); w.n_raw_events.release(); w.n_queries.release();
-  w.q_off.release(); w.feat_row.release(); for (int c = 0; c < 2; ++c) { w.feat_cache[c].release(); w.nf_cache[c].release(); w.nraw_cache[c].release(); }
-  w.blk_chunk_start.release(); w.blk_chunk_offset.release(); w.blk_chunk_scale.release(); w.absent.release(); w.chunk_start.release(); w.chunk_offset.release();
-  w.chunk_scale.release(); w.ps.release(); w.pss.release(); w.t1.release(); w.t2.release();
-  w.means.release(); w.features.release(); w.key_a.release(); w.key_b.release(); w.dist_a.release();
-  w.dist_b.release(); w.score.release(); w.coef.release(); w.pred.release(); w.seg.release(); w.runs.release(); w.run_count.release(); w.entry_total.release(); w.part_base.release(); w.link_list.release(); w.link_count.release(); w.pend_list.release(); w.pend_count.release(); w.seg_qmin.release(); w.cub_temp.release();
-  w.chain_tmp.release(); w.ids.release(); w.round_info.release();
-  w.seg_max.release(); w.n_scratch.release(); w.cand_list.release(); w.cand_all.release();
-  w.cand_counts.release(); w.ctl.release(); w.tags.release();
-  ctx->ex.reset();
-  ctx->local_group.reset();
-  ctx->index.leaves.release(); ctx->index.nodes.release(); ctx->index.leaf_widx.release(); ctx->index.bucket_base.release();
-  w.qkey_a.release(); w.qkey_b.release(); w.qpay_a.release(); w.qpay_b.release(); w.ovf_list.release();
-  w.entry_info.release(); w.qsort_temp.release();
-  ctx->raw.release(); ctx->kept.release(); ctx->d_read_off.release(); ctx->d_kept_off.release();
-  ctx->d_dig.release(); ctx->d_range.release(); ctx->d_offset.release(); ctx->d_kept_len.release();
-  for (auto &ev : ctx->ev) if (ev) cudaEventDestroy(ev);
-  for (auto &ev : ctx->timer) if (ev) cudaEventDestroy(ev);
-  for (auto &ev : ctx->ev_blk_t0) if (ev) cudaEventDestroy(ev);
-  for (auto &ev : ctx->ev_cp) if (ev) cudaEventDestroy(ev);
-  for (auto &ev : ctx->ev_blk_t1) if (ev) cudaEventDestroy(ev);
-  if (ctx->stream_ev) cudaStreamDestroy(ctx->stream_ev);
-  if (ctx->stream_cp) cudaStreamDestroy(ctx->stream_cp);
-  for (auto &ev : ctx->slice_events) cudaEventDestroy(ev);
-  if (ctx->h_kept_pinned) cudaFreeHost(ctx->h_kept_pinned);
-  if (ctx->d_ctr) cudaFree(ctx->d_ctr);
-  if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
-  if (ctx->h_ctl) cudaFreeHost(ctx->h_ctl);
-  if (ctx->h_cloud_stage) cudaFreeHost(ctx->h_cloud_stage);
-  if (ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
 }
 
@@ -1386,13 +1341,7 @@ static int reads_prepare(smb_ctx *ctx, const uint64_t *read_off, const float *di
   CK(ctx->d_range.ensure(n_reads));
   CK(ctx->d_offset.ensure(n_reads));
   CK(ctx->d_kept_len.ensure(n_reads));
-  if (n_reads > ctx->h_kept_pinned_cap) {
-    if (ctx->h_kept_pinned) cudaFreeHost(ctx->h_kept_pinned);
-    ctx->h_kept_pinned = nullptr;
-    ctx->h_kept_pinned_cap = 0;
-    CK(cudaMallocHost((void **)&ctx->h_kept_pinned, (n_reads + n_reads / 4 + 64) * sizeof(uint32_t)));
-    ctx->h_kept_pinned_cap = n_reads + n_reads / 4 + 64;
-  }
+  CK(ctx->h_kept_pinned.ensure(n_reads));
   CK(cudaMemcpyAsync(ctx->d_read_off.p, read_off, (n_reads + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
   CK(cudaMemcpyAsync(ctx->d_kept_off.p, ctx->h_kept_off.data(), n_reads * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
   CK(cudaMemcpyAsync(ctx->d_dig.p, dig, n_reads * sizeof(float), cudaMemcpyHostToDevice, s));
@@ -1428,7 +1377,7 @@ static int filter_slice(smb_ctx *ctx, size_t r0, size_t r1, cudaStream_t s) {
                                                                 ctx->d_kept_off.p + r0, ctx->kept.p,
                                                                 ctx->d_kept_len.p + r0, (uint32_t)(r1 - r0));
   LAUNCH_CHECK();
-  CK(cudaMemcpyAsync(ctx->h_kept_pinned + r0, ctx->d_kept_len.p + r0, (r1 - r0) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(ctx->h_kept_pinned.p + r0, ctx->d_kept_len.p + r0, (r1 - r0) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
   ctx->stats.d2h_bytes += (r1 - r0) * 4;
   return SMB_OK;
 }
@@ -1445,7 +1394,7 @@ static int filter_reads(smb_ctx *ctx) {
   CK(cudaEventRecord(ctx->ev[4], s));
   rc = host_sync(ctx);
   if (rc) return rc;
-  memcpy(ctx->h_kept_len.data(), ctx->h_kept_pinned, n_reads * sizeof(uint32_t));
+  memcpy(ctx->h_kept_len.data(), ctx->h_kept_pinned.p, n_reads * sizeof(uint32_t));
   float ms = 0;
   cudaEventElapsedTime(&ms, ctx->ev[5], ctx->ev[4]);
   ctx->stats.ms_filter += ms;
@@ -1474,10 +1423,10 @@ struct DeferFrees {
 
 static int slice_event(smb_ctx *ctx, size_t k, cudaEvent_t *out) {
   while (k >= ctx->slice_events.size()) {
-    cudaEvent_t e;
-    if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess)
+    Event e;
+    if (cudaEventCreateWithFlags(&e.h, cudaEventDisableTiming) != cudaSuccess)
       return fail(ctx, SMB_ERR_CUDA, "cudaEventCreate (upload slice)");
-    ctx->slice_events.push_back(e);
+    ctx->slice_events.push_back(std::move(e));
   }
   *out = ctx->slice_events[k];
   return SMB_OK;
@@ -1517,7 +1466,7 @@ static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping
   auto chunk_limit = [&](uint32_t r) { return std::min<uint32_t>(n_chunks[r], (uint32_t)prm.max_num_chunks); };
   auto admit = [&](size_t r0, size_t r1) {
     for (size_t r = r0; r < r1; ++r) {
-      ctx->h_kept_len[r] = ctx->h_kept_pinned[r];
+      ctx->h_kept_len[r] = ctx->h_kept_pinned.p[r];
       n_chunks[r] = ctx->h_kept_len[r] / kChunk;  // tail dropped, sigmap.cc:643
       t_admit[r] = round;
       if (n_chunks[r] > 0 && prm.max_num_chunks > 0) active.push_back((uint32_t)r);
@@ -1698,7 +1647,7 @@ static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping
           return fail(ctx, SMB_ERR_CUDA, std::string("upload slice: ") + cudaGetErrorString(q));
         }
         for (size_t r = plan->first_read[k]; r < plan->first_read[k + 1]; ++r) {
-          ctx->h_kept_len[r] = ctx->h_kept_pinned[r];
+          ctx->h_kept_len[r] = ctx->h_kept_pinned.p[r];
           n_chunks[r] = ctx->h_kept_len[r] / kChunk;  // tail dropped, sigmap.cc:643
           if (n_chunks[r] > 0) {
             into.push_back((uint32_t)r);
@@ -1944,7 +1893,6 @@ int smb_stage_raw_to_pa(smb_ctx *ctx, const int16_t *raw, size_t n, float dig, f
   LAUNCH_CHECK();
   CK(cudaMemcpyAsync(out, d.p, kept * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
-  d.release();
   return SMB_OK;
 }
 
@@ -1965,7 +1913,6 @@ static int stage_events_common(smb_ctx *ctx, const float *pa, size_t n_chunks, u
   int rc = run_events(ctx, SRC_PA_FLOAT, d_pa.p, B, d_peaks);
   if (rc) return rc;
   CK(cudaStreamSynchronize(s));
-  d_pa.release();
   return SMB_OK;
 }
 
@@ -1995,7 +1942,6 @@ int smb_stage_detect(smb_ctx *ctx, const float *pa, float *tstat1, float *tstat2
   if (tstat2) CK(cudaMemcpy2D(tstat2, sizeof(float), ctx->ws.t2.p, Bp * sizeof(float), sizeof(float), kChunk + 1, cudaMemcpyDeviceToHost));
   if (peaks && ne) CK(cudaMemcpy(peaks, d_peaks.p, ne * sizeof(uint32_t), cudaMemcpyDeviceToHost));
   if (means && ne) CK(cudaMemcpy(means, ctx->ws.means.p, ne * sizeof(float), cudaMemcpyDeviceToHost));
-  d_peaks.release();
   return SMB_OK;
 }
 
@@ -2019,7 +1965,7 @@ int smb_stage_radius(smb_ctx *ctx, const float *queries, size_t nq, float radius
   CK(d_b.ensure(dcap));
   CK(cnt.ensure(nq));
   CK(cudaMemcpyAsync(d_q.p, queries, nq * kDim * sizeof(float), cudaMemcpyHostToDevice, s));
-  k_reset_step<<<1, 1, 0, s>>>(ctx->d_ctr);
+  k_reset_step<<<1, 1, 0, s>>>(ctx->d_ctr.p);
   LAUNCH_CHECK();
   SearchArgs sa{};
   sa.features = d_q.p;
@@ -2028,14 +1974,14 @@ int smb_stage_radius(smb_ctx *ctx, const float *queries, size_t nq, float radius
   sa.out_key = k_a.p;
   sa.out_dist = d_a.p;
   sa.cap = dcap;
-  sa.ctr = ctx->d_ctr;
+  sa.ctr = ctx->d_ctr.p;
   {
     int rc = launch_search<true>(ctx, sa, (uint32_t)nq, s);
     if (rc) return rc;
   }
-  CK(cudaMemcpyAsync(ctx->h_ctr, ctx->d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(ctx->h_ctr.p, ctx->d_ctr.p, sizeof(Counters), cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
-  const unsigned long long n = ctx->h_ctr->n_anchors;
+  const unsigned long long n = ctx->h_ctr.p->n_anchors;
   if (n > cap) return fail(ctx, SMB_ERR_CAPACITY, "smb_stage_radius: more hits than cap");
   CK(cudaMemsetAsync(cnt.p, 0, nq * sizeof(unsigned long long), s));
   const uint64_t *keys = k_a.p;
@@ -2062,7 +2008,6 @@ int smb_stage_radius(smb_ctx *ctx, const float *queries, size_t nq, float radius
   CK(cudaStreamSynchronize(s));
   for (size_t q = 0; q < nq; ++q) hit_off[q + 1] = hit_off[q] + h_cnt[q];
   for (unsigned long long i = 0; i < n; ++i) hit_idx[i] = h_keys[i] & 0xFFFFFFFFull;
-  d_q.release(); d_a.release(); d_b.release(); k_a.release(); k_b.release(); cnt.release(); tmp.release();
   return SMB_OK;
 }
 
@@ -2083,7 +2028,6 @@ void smb_batch_destroy(smb_batch *b) {
   if (!b) return;
   cudaSetDevice(b->ctx->device);
   cudaStreamSynchronize(b->ctx->stream);
-  slots_release(b->sp);
   delete b;
 }
 
@@ -2124,8 +2068,6 @@ int smb_batch_generate_chains(smb_batch *b, const uint32_t *slots, uint32_t n, c
   rout.info = &info;
   int rc = run_round(ctx, b->sp, present, absent, SRC_FEATURES, *prm, fill, &rout);
   cudaStreamSynchronize(ctx->stream);
-  d_feat.release();
-  d_off.release();
   return rc;
 }
 
@@ -2183,7 +2125,7 @@ int smb_stream_open(smb_ctx *ctx, uint32_t n_channels, const smb_params *params)
   CK(cudaSetDevice(ctx->device));
   if (!ctx->has_index) return fail(ctx, SMB_ERR_STATE, "no index loaded");
   if (ctx->stream_slots) smb_stream_close(ctx);
-  ctx->stream_slots = new SlotSpace();
+  ctx->stream_slots = std::make_unique<SlotSpace>();
   int rc = slots_init(ctx, *ctx->stream_slots, n_channels);
   if (rc) return rc;
   ctx->stream_params = *params;
@@ -2202,15 +2144,9 @@ int smb_stream_close(smb_ctx *ctx) {
   if (ctx->stream_slots) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
-    slots_release(*ctx->stream_slots);
-    delete ctx->stream_slots;
-    ctx->stream_slots = nullptr;
+    ctx->stream_slots.reset();
   }
-  if (ctx->h_stream_stage) {
-    cudaFreeHost(ctx->h_stream_stage);
-    ctx->h_stream_stage = nullptr;
-    ctx->h_stream_stage_cap = 0;
-  }
+  ctx->h_stream_stage.release();
   ctx->d_stream_stage.release();
   return SMB_OK;
 }
@@ -2279,14 +2215,7 @@ int smb_stream_round(smb_ctx *ctx, const uint32_t *channels, uint32_t n, const i
   const smb_params &prm = ctx->stream_params;
   // host-side range filter of the incoming samples (same decisions as K1) and chunk cutting;
   // completed chunks go straight into the pinned staging buffer
-  if ((size_t)n * kChunk > ctx->h_stream_stage_cap) {
-    if (ctx->h_stream_stage) cudaFreeHost(ctx->h_stream_stage);
-    ctx->h_stream_stage = nullptr;
-    ctx->h_stream_stage_cap = 0;
-    const size_t want = (size_t)std::max(n, sp.n_slots) * kChunk;
-    CK(cudaMallocHost((void **)&ctx->h_stream_stage, want * sizeof(int16_t)));
-    ctx->h_stream_stage_cap = want;
-  }
+  if ((size_t)n * kChunk > ctx->h_stream_stage.cap) CK(ctx->h_stream_stage.alloc((size_t)std::max(n, sp.n_slots) * kChunk));
   const auto t_stage0 = std::chrono::steady_clock::now();
   std::vector<uint32_t> present;
   present.reserve(n);
@@ -2310,7 +2239,7 @@ int smb_stream_round(smb_ctx *ctx, const uint32_t *channels, uint32_t n, const i
     std::vector<int16_t> &pend = ctx->stream_pending[ch];
     const int16_t *in = samples + sample_off[i];
     const size_t cnt = sample_off[i + 1] - sample_off[i];
-    int16_t *slot = ctx->h_stream_stage + (size_t)i * kChunk;
+    int16_t *slot = ctx->h_stream_stage.p + (size_t)i * kChunk;
     const bool wants = ctx->stream_chunks[ch] < (uint32_t)prm.max_num_chunks;
     bool clean = false;
     if (!ctx->stream_generic[ch]) {
@@ -2357,7 +2286,7 @@ int smb_stream_round(smb_ctx *ctx, const uint32_t *channels, uint32_t n, const i
   for (uint32_t i = 0; i < n; ++i) {
     if (!ready[i]) continue;
     if (present.size() != i)
-      memmove(ctx->h_stream_stage + present.size() * kChunk, ctx->h_stream_stage + (size_t)i * kChunk, kChunk * sizeof(int16_t));
+      memmove(ctx->h_stream_stage.p + present.size() * kChunk, ctx->h_stream_stage.p + (size_t)i * kChunk, kChunk * sizeof(int16_t));
     present.push_back(channels[i]);
   }
   ctx->stats.ms_stream_stage +=
@@ -2377,7 +2306,7 @@ int smb_stream_round(smb_ctx *ctx, const uint32_t *channels, uint32_t n, const i
     const size_t n_stage = present.size() * kChunk;
     CK(ctx->d_stream_stage.ensure(std::max<size_t>(n_stage, 8)));
     if (n_stage)
-      CK(cudaMemcpyAsync(ctx->d_stream_stage.p, ctx->h_stream_stage, n_stage * sizeof(int16_t),
+      CK(cudaMemcpyAsync(ctx->d_stream_stage.p, ctx->h_stream_stage.p, n_stage * sizeof(int16_t),
                          cudaMemcpyHostToDevice, ctx->stream));
     ctx->stats.h2d_bytes += n_stage * 2;
     auto fill = [&](StepEntries &en, size_t first, uint32_t count) {

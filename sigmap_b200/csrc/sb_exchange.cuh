@@ -100,7 +100,6 @@ struct LocalExchange : Exchange {
   std::shared_ptr<LocalGroup> g;
   int device = 0;
   DevBuf<unsigned char> tmp;
-  ~LocalExchange() override { tmp.release(); }
 
   int allgather(const void *d_send, void *d_recv, size_t bytes, cudaStream_t s, std::string &err) override {
     cudaError_t e = cudaStreamSynchronize(s);  // my send buffer is complete

@@ -19,42 +19,12 @@
 
 namespace {
 
-template <class T>
-struct DevArr {  // exact-size device array, freed with its owner
-  T *p = nullptr;
-  size_t n = 0;
-  DevArr() = default;
-  DevArr(const DevArr &) = delete;
-  DevArr &operator=(const DevArr &) = delete;
-  ~DevArr() { reset(); }
-  void reset() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    n = 0;
-  }
-  cudaError_t alloc(size_t k) {
-    reset();
-    const cudaError_t e = cudaMalloc((void **)&p, std::max<size_t>(k, 1) * sizeof(T));
-    if (e != cudaSuccess) {
-      p = nullptr;
-      cudaGetLastError();  // an out-of-memory return is not sticky; clear it
-      return e;
-    }
-    n = k;
-    return e;
-  }
-};
-
 struct StageTimer {  // CUDA events between the stages of one build
-  cudaEvent_t ev[9] = {};
+  Event ev[9];
   int n = 0;
-  ~StageTimer() {
-    for (cudaEvent_t e : ev)
-      if (e) cudaEventDestroy(e);
-  }
   cudaError_t mark(cudaStream_t s) {
     if (!ev[n]) {
-      const cudaError_t e = cudaEventCreate(&ev[n]);
+      const cudaError_t e = cudaEventCreate(&ev[n].h);
       if (e != cudaSuccess) return e;
     }
     return cudaEventRecord(ev[n++], s);
@@ -194,13 +164,6 @@ static int build_index_core(smb_ctx *ctx, IndexInput &in) {
   ix.leaves = di.leaves.p;
   ix.leaf_widx = di.leaf_widx.p;
   CK(cudaStreamSynchronize(s));
-  code_a.release();
-  code_b.release();
-  w_a.release();
-  w_b.release();
-  tmp.release();
-  ext_min.release();
-  ext_max.release();
   {
     // linear coordinate g = bucket_base[bucket] + target: monotone in the sort order, dense
     // enough to be cut into equal-width bins by the per-entry sort
@@ -224,7 +187,7 @@ static int build_index_core(smb_ctx *ctx, IndexInput &in) {
 // The whole cloud in device memory (*pos / *val, *count points).  Stage times go to
 // ctx->build_stats (ms_index is left to the caller).
 static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengths, uint32_t n,
-                       const float *level_mean, DevArr<uint64_t> &pos, DevArr<float> &val, uint64_t *count) {
+                       const float *level_mean, DevBuf<uint64_t> &pos, DevBuf<float> &val, uint64_t *count) {
   using namespace cloud;
   if (n && (!seqs || !lengths)) return fail(ctx, SMB_ERR_ARG, "device index build: null sequences / lengths");
   if (!level_mean) return fail(ctx, SMB_ERR_ARG, "device index build: null level table");
@@ -260,21 +223,21 @@ static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *le
   StageTimer tm;
   CK(tm.mark(s));
   // ---- upload the + strands through two pinned slices
-  DevArr<unsigned char> d_seq;
+  DevBuf<unsigned char> d_seq;
   CLOUD_ALLOC(d_seq, n_bases, "the reference sequences");
   {
     const size_t slice = kCloudSlice;
-    cudaEvent_t done[2] = {};
-    if (!ctx->h_cloud_stage) CK(cudaHostAlloc((void **)&ctx->h_cloud_stage, 2 * slice, cudaHostAllocDefault));
-    CK(cudaEventCreateWithFlags(&done[0], cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&done[1], cudaEventDisableTiming));
+    Event done[2];
+    if (!ctx->h_cloud_stage.p) CK(ctx->h_cloud_stage.alloc(2 * slice));
+    CK(cudaEventCreateWithFlags(&done[0].h, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&done[1].h, cudaEventDisableTiming));
     int k = 0;
     cudaError_t e = cudaSuccess;
     for (uint32_t c = 0; c < n && e == cudaSuccess; ++c) {
       if (lengths[c] < (uint32_t)kMaskK) continue;
       for (uint64_t a = 0; a < lengths[c] && e == cudaSuccess; a += slice) {
         const size_t len = (size_t)std::min<uint64_t>(slice, lengths[c] - a);
-        unsigned char *h = ctx->h_cloud_stage + (size_t)k * slice;
+        unsigned char *h = ctx->h_cloud_stage.p + (size_t)k * slice;
         if ((e = cudaEventSynchronize(done[k])) != cudaSuccess) break;
         memcpy(h, seqs[c] + a, len);
         if ((e = cudaMemcpyAsync(d_seq.p + plus_off[c] + a, h, len, cudaMemcpyHostToDevice, s)) != cudaSuccess) break;
@@ -283,12 +246,10 @@ static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *le
       }
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    cudaEventDestroy(done[0]);
-    cudaEventDestroy(done[1]);
     if (e != cudaSuccess) return fail(ctx, SMB_ERR_CUDA, std::string("device index build: upload: ") + cudaGetErrorString(e));
   }
   ctx->stats.h2d_bytes += n_bases;
-  DevArr<Seg> d_segs;
+  DevBuf<Seg> d_segs;
   CLOUD_ALLOC(d_segs, n_segs, "the segment table");
   CK(cudaMemcpyAsync(d_segs.p, segs.data(), n_segs * sizeof(Seg), cudaMemcpyHostToDevice, s));
   CK(tm.mark(s));
@@ -299,31 +260,31 @@ static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *le
   const size_t n_census = chunks.size();
   for (uint32_t i = 0; i < n_segs; ++i)
     for (uint32_t p = 0; p < segs[i].len - kK + 1; p += kChunkPos) chunks.push_back(Chunk{i, p});
-  DevArr<Chunk> d_chunks;
-  DevArr<uint32_t> d_hist;
-  DevArr<unsigned long long> d_total;
+  DevBuf<Chunk> d_chunks;
+  DevBuf<uint32_t> d_hist;
+  DevBuf<unsigned long long> d_total;
   CLOUD_ALLOC(d_chunks, chunks.size(), "the chunk table");
   CLOUD_ALLOC(d_hist, (size_t)1 << (2 * kMaskK), "the 11-mer histogram");
   CLOUD_ALLOC(d_total, 1, "the 11-mer histogram");
   CK(cudaMemcpyAsync(d_chunks.p, chunks.data(), chunks.size() * sizeof(Chunk), cudaMemcpyHostToDevice, s));
-  CK(cudaMemsetAsync(d_hist.p, 0, d_hist.n * sizeof(uint32_t), s));
+  CK(cudaMemsetAsync(d_hist.p, 0, d_hist.cap * sizeof(uint32_t), s));
   CK(cudaMemsetAsync(d_total.p, 0, sizeof(unsigned long long), s));
   k_cloud_census<<<(unsigned)n_census, 256, 0, s>>>(d_seq.p, d_segs.p, d_chunks.p, d_hist.p, d_total.p);
   LAUNCH_CHECK();
   CK(tm.mark(s));
   // ---- level hashes and mask, both strands
-  DevArr<uint16_t> d_hm;
+  DevBuf<uint16_t> d_hm;
   CLOUD_ALLOC(d_hm, n_pos, "the per-position level hashes");
   k_cloud_hm<<<(unsigned)(chunks.size() - n_census), 256, 0, s>>>(d_seq.p, d_segs.p, d_chunks.p + n_census, d_hist.p,
                                                                    d_total.p, d_hm.p);
   LAUNCH_CHECK();
   CK(tm.mark(s));
   CK(cudaStreamSynchronize(s));
-  d_seq.reset();
-  d_hist.reset();
-  d_chunks.reset();
+  d_seq.release();
+  d_hist.release();
+  d_chunks.release();
   // ---- z-normalisation: sequential double sums per strand -> z table per segment
-  DevArr<float> d_lv, d_ztab;
+  DevBuf<float> d_lv, d_ztab;
   CLOUD_ALLOC(d_lv, kTable, "the level table");
   CLOUD_ALLOC(d_ztab, (size_t)n_segs * kTable, "the z tables");
   CK(cudaMemcpyAsync(d_lv.p, level_mean, kTable * sizeof(float), cudaMemcpyHostToDevice, s));
@@ -345,7 +306,7 @@ static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *le
     if (!int_ok || q_max * (double)max_len >= 9.0e18) int_ok = 0;
     unit_exp = lo;
   }
-  DevArr<unsigned int> d_serial;
+  DevBuf<unsigned int> d_serial;
   CLOUD_ALLOC(d_serial, 1, "the z sums");
   CK(cudaMemsetAsync(d_serial.p, 0, sizeof(unsigned int), s));
   k_cloud_zsums<<<(n_segs + kZWarps - 1) / kZWarps, kZWarps * 32, 0, s>>>(d_segs.p, n_segs, d_hm.p, d_lv.p, int_ok,
@@ -365,11 +326,11 @@ static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *le
     for (uint32_t p = 0; p < nw; p += std::min(T, nw - p)) tiles.push_back(Tile{i, p, p + std::min(T, nw - p), 0});
   }
   const uint32_t n_tiles = (uint32_t)tiles.size();
-  DevArr<Tile> d_tiles;
-  DevArr<TileState> d_ts;
-  DevArr<uint8_t> d_flags;
-  DevArr<ChainStats> d_cs;
-  DevArr<unsigned long long> d_cnt, d_off;
+  DevBuf<Tile> d_tiles;
+  DevBuf<TileState> d_ts;
+  DevBuf<uint8_t> d_flags;
+  DevBuf<ChainStats> d_cs;
+  DevBuf<unsigned long long> d_cnt, d_off;
   CLOUD_ALLOC(d_tiles, n_tiles, "the tile table");
   CLOUD_ALLOC(d_ts, n_tiles, "the tile states");
   CLOUD_ALLOC(d_flags, n_pos, "the keep flags");
@@ -391,7 +352,7 @@ static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *le
   {
     size_t tmp_bytes = 0;
     CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_cnt.p, d_off.p, (int64_t)n_tiles, s));
-    DevArr<unsigned char> tmp;
+    DevBuf<unsigned char> tmp;
     CLOUD_ALLOC(tmp, tmp_bytes, "the tile scan");
     CK(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, d_cnt.p, d_off.p, (int64_t)n_tiles, s));
     ctx->stats.launches += 2;
@@ -428,26 +389,26 @@ static int cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *le
 
 namespace {
 struct DevPart {  // one rank's part of the cloud in device memory (host_index.cc PartSink)
-  DevArr<uint64_t> pos, run_off, run_first, w_pos;
-  DevArr<float> val;
-  DevArr<uint8_t> own;
-  DevArr<uint32_t> w_src, w_orig;
+  DevBuf<uint64_t> pos, run_off, run_first, w_pos;
+  DevBuf<float> val;
+  DevBuf<uint8_t> own;
+  DevBuf<uint32_t> w_src, w_orig;
   uint64_t n_values = 0, n_runs = 0, n_windows = 0;
 };
 }  // namespace
 
 // The rank's part of the device cloud; with windows, also the window table of its shard.
-static int part_build(smb_ctx *ctx, const DevArr<uint64_t> &pos, const DevArr<float> &val, uint64_t n,
+static int part_build(smb_ctx *ctx, const DevBuf<uint64_t> &pos, const DevBuf<float> &val, uint64_t n,
                       const uint32_t *owner, uint32_t n_contigs, uint32_t rank, bool windows, DevPart &out) {
   using namespace cloud;
   cudaStream_t s = ctx->stream;
-  DevArr<uint32_t> d_owner;
+  DevBuf<uint32_t> d_owner;
   CLOUD_ALLOC(d_owner, n_contigs, "the owner table");
   CK(cudaMemcpyAsync(d_owner.p, owner, n_contigs * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
   const uint64_t nb64 = (n + kPartBlock - 1) / kPartBlock;
   if (nb64 >= 0x7FFFFFFFull) return fail(ctx, SMB_ERR_CAPACITY, "device index build: cloud too large for one part pass");
   const uint32_t nb = (uint32_t)std::max<uint64_t>(nb64, 1);
-  DevArr<unsigned long long> blk, cnt3, off3;
+  DevBuf<unsigned long long> blk, cnt3, off3;
   CLOUD_ALLOC(blk, nb, "the part counters");
   CLOUD_ALLOC(cnt3, 3 * (size_t)nb, "the part counters");
   CLOUD_ALLOC(off3, 3 * (size_t)nb + 3, "the part counters");
@@ -460,7 +421,7 @@ static int part_build(smb_ctx *ctx, const DevArr<uint64_t> &pos, const DevArr<fl
   LAUNCH_CHECK();
   size_t tmp_bytes = 0;
   CK(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, cnt3.p, off3.p, (int64_t)nb, s));
-  DevArr<unsigned char> tmp;
+  DevBuf<unsigned char> tmp;
   CLOUD_ALLOC(tmp, tmp_bytes, "the part scan");
   for (int k = 0; k < 3; ++k)
     CK(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, cnt3.p + (size_t)k * nb, off3.p + (size_t)k * nb, (int64_t)nb, s));
@@ -510,7 +471,7 @@ static int cloud_extent(smb_ctx *ctx, const uint64_t *pos, const float *val, uin
                         bool all_buckets, IndexInput &in) {
   using namespace cloud;
   cudaStream_t s = ctx->stream;
-  DevArr<CloudExtent> d_ext;
+  DevBuf<CloudExtent> d_ext;
   CLOUD_ALLOC(d_ext, 1, "the cloud extent");
   const CloudExtent init{0xFFFFFFFFu, 0u, 0u, 0u};
   CK(cudaMemcpyAsync(d_ext.p, &init, sizeof init, cudaMemcpyHostToDevice, s));
@@ -525,7 +486,7 @@ static int cloud_extent(smb_ctx *ctx, const uint64_t *pos, const float *val, uin
   if (n && (ext.max_bucket >> 1) >= contig_limit)
     return fail(ctx, SMB_ERR_ARG, "point cloud names a contig beyond n_contigs");
   const size_t n_buckets = all_buckets ? 2 * (size_t)contig_limit : (n ? (size_t)ext.max_bucket + 1 : 0);
-  DevArr<unsigned long long> d_span;
+  DevBuf<unsigned long long> d_span;
   CLOUD_ALLOC(d_span, n_buckets, "the cloud extent");
   CK(cudaMemsetAsync(d_span.p, 0, n_buckets * sizeof(unsigned long long), s));
   if (n) {
@@ -543,7 +504,7 @@ static int cloud_extent(smb_ctx *ctx, const uint64_t *pos, const float *val, uin
 }
 
 template <class T>
-static int upload(smb_ctx *ctx, DevArr<T> &d, const T *h, size_t n, const char *what) {
+static int upload(smb_ctx *ctx, DevBuf<T> &d, const T *h, size_t n, const char *what) {
   CLOUD_ALLOC(d, n, what);
   CK(cudaMemcpyAsync(d.p, h, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
   return SMB_OK;
@@ -590,8 +551,8 @@ extern "C" {
 
 int smb_index_set_points(smb_ctx *ctx, const uint64_t *pos, const float *val, size_t n) {
   CK(cudaSetDevice(ctx->device));
-  DevArr<uint64_t> d_pos;
-  DevArr<float> d_val;
+  DevBuf<uint64_t> d_pos;
+  DevBuf<float> d_val;
   int rc;
   if ((rc = upload(ctx, d_pos, pos, n, "the point cloud")) || (rc = upload(ctx, d_val, val, n, "the point cloud")))
     return rc;
@@ -629,8 +590,8 @@ int smb_index_set_points_sharded(smb_ctx *ctx, const uint64_t *pos, const float 
   if (!ctx->ex) return fail(ctx, SMB_ERR_STATE, "join a shard group first (smb_shard_local_group / smb_shard_nccl_init)");
   for (uint32_t c = 0; c < n_contigs; ++c)
     if (contig_owner[c] >= (uint32_t)ctx->ex->world) return fail(ctx, SMB_ERR_ARG, "contig owner out of range");
-  DevArr<uint64_t> d_pos;
-  DevArr<float> d_val;
+  DevBuf<uint64_t> d_pos;
+  DevBuf<float> d_val;
   int rc;
   if ((rc = upload(ctx, d_pos, pos, n, "the point cloud")) || (rc = upload(ctx, d_val, val, n, "the point cloud")))
     return rc;
@@ -638,8 +599,8 @@ int smb_index_set_points_sharded(smb_ctx *ctx, const uint64_t *pos, const float 
   if ((rc = cloud_extent(ctx, d_pos.p, d_val.p, n, n_contigs, false, in))) return rc;
   DevPart part;
   if ((rc = part_build(ctx, d_pos, d_val, n, contig_owner, n_contigs, (uint32_t)ctx->ex->rank, true, part))) return rc;
-  d_pos.reset();
-  d_val.reset();
+  d_pos.release();
+  d_val.release();
   return build_shard(ctx, part, in);
 }
 
@@ -706,7 +667,6 @@ int smb_index_broadcast(smb_ctx *ctx, int root) {
   if (rc) return rc;
   CK(cudaMemcpyAsync(&h, d_h.p, sizeof(Header), cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
-  d_h.release();
   // ---- the arrays, in place in the receivers' own buffers
   const IndexView &ix = h.index.ix;
   uint64_t n_nodes_rec = 0;
@@ -740,7 +700,6 @@ int smb_index_broadcast(smb_ctx *ctx, int root) {
     index_installed(ctx);
   }
   CK(cudaStreamSynchronize(s));
-  d_len.release();
   di.sharded = false;
   return SMB_OK;
 }
@@ -754,8 +713,8 @@ int smb_point_cloud_build(smb_ctx *ctx, const char *const *seqs, const uint32_t 
   *pos = nullptr;
   *val = nullptr;
   *count = 0;
-  DevArr<uint64_t> d_pos;
-  DevArr<float> d_val;
+  DevBuf<uint64_t> d_pos;
+  DevBuf<float> d_val;
   uint64_t c = 0;
   int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &c);
   if (rc) return rc;
@@ -787,8 +746,8 @@ int smb_point_cloud_build_part(smb_ctx *ctx, const char *const *seqs, const uint
   if (!owner) return fail(ctx, SMB_ERR_ARG, "smb_point_cloud_build_part: null owner table");
   DevPart part;
   {
-    DevArr<uint64_t> d_pos;
-    DevArr<float> d_val;
+    DevBuf<uint64_t> d_pos;
+    DevBuf<float> d_val;
     uint64_t c = 0;
     int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &c);
     if (rc) return rc;
@@ -826,8 +785,8 @@ int smb_index_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengt
     for (uint32_t c = 0; c < n; ++c)
       if (contig_owner[c] >= (uint32_t)ctx->ex->world) return fail(ctx, SMB_ERR_ARG, "contig owner out of range");
   }
-  DevArr<uint64_t> d_pos;
-  DevArr<float> d_val;
+  DevBuf<uint64_t> d_pos;
+  DevBuf<float> d_val;
   uint64_t N = 0;
   int rc = cloud_build(ctx, seqs, lengths, n, level_mean, d_pos, d_val, &N);
   if (rc) return rc;
@@ -839,8 +798,8 @@ int smb_index_build(smb_ctx *ctx, const char *const *seqs, const uint32_t *lengt
     DevPart part;
     rc = part_build(ctx, d_pos, d_val, N, contig_owner, n, (uint32_t)ctx->ex->rank, true, part);
     if (rc) return rc;
-    d_pos.reset();  // the rank keeps its part only
-    d_val.reset();
+    d_pos.release();  // the rank keeps its part only
+    d_val.release();
     IndexInput in{nullptr, nullptr, nullptr, nullptr, 0, (size_t)N, 0.0f, 0.0f, 0u, 0u, {}};
     rc = cloud_extent(ctx, part.pos.p, part.val.p, part.n_values, n, true, in);
     if (!rc) rc = build_shard(ctx, part, in);
