@@ -230,11 +230,28 @@ int smb_index_build_stats(smb_ctx *ctx, smb_build_stats *out);
 /* Replaces the per-read body of Sigmap::StreamingMap (sigmap.cc:630-866) for n_reads
  * reads at once: raw int16 samples of read r are raw[read_off[r] .. read_off[r+1]);
  * digitisation/range/offset are the per-read SLOW5 fields (signal_batch.cc:187-191).
- * raw may be a host pointer (copied in, pinned or pageable) -- see smb_map_reads_device.
- * out[r] receives read r's row. */
+ * raw is a host pointer (copied in, pinned or pageable); samples already in device memory go
+ * through smb_map_reads_device.  out[r] receives read r's row. */
 int smb_map_reads(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off,
                   const float *digitisation, const float *range, const float *offset,
                   size_t n_reads, const smb_params *params, smb_mapping *out);
+/* smb_map_reads for samples already in device memory on this context's device.  Read r is
+ * raw[read_start[r] .. read_start[r] + read_len[r]) (int16 elements; reads may be in any order,
+ * have gaps between them, or be the rows of a padded [n_reads][stride] tensor).  read_start,
+ * read_len, digitisation, range, offset and out are host arrays.  The library reads raw and
+ * never writes it; the samples are not copied.  stream (a cudaStream_t, may be NULL for the legacy
+ * default stream): the call's device work is ordered after what is queued on it.  raw may be
+ * reused by the caller when the call returns.  Rows are those smb_map_reads returns for the same
+ * samples, bit for bit.
+ * raw must be device (or managed) memory of the context's device, else SMB_ERR_ARG; it is neither
+ * read nor checked when every read_len is 0 (such a read gets an unmapped row).  Precondition the
+ * library cannot check: every read lies inside the caller's allocation.
+ * Afterwards the context holds no uploaded read set: smb_map_uploaded returns SMB_ERR_STATE until
+ * the next smb_reads_upload or smb_map_reads. */
+int smb_map_reads_device(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_start,
+                         const uint32_t *read_len, const float *digitisation, const float *range,
+                         const float *offset, size_t n_reads, const smb_params *params,
+                         smb_mapping *out, void *stream);
 /* Two-phase variant used to time with inputs resident in HBM: upload once, map many. */
 int smb_reads_upload(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off,
                      const float *digitisation, const float *range, const float *offset,

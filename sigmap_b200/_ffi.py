@@ -201,6 +201,8 @@ PROTOTYPES = {
     "smb_index_build_stats": (C.c_int, [C.c_void_p, C.POINTER(BuildStats)]),
     "smb_map_reads": (C.c_int, [C.c_void_p, i16p, u64p, f32p, f32p, f32p, C.c_size_t,
                                 C.POINTER(Params), C.POINTER(Mapping)]),
+    "smb_map_reads_device": (C.c_int, [C.c_void_p, C.c_void_p, u64p, u32p, f32p, f32p, f32p, C.c_size_t,
+                                       C.POINTER(Params), C.POINTER(Mapping), C.c_void_p]),
     "smb_reads_upload": (C.c_int, [C.c_void_p, i16p, u64p, f32p, f32p, f32p, C.c_size_t]),
     "smb_map_uploaded": (C.c_int, [C.c_void_p, C.POINTER(Params), C.POINTER(Mapping)]),
     "smb_stage_raw_to_pa": (C.c_int, [C.c_void_p, i16p, C.c_size_t, C.c_float, C.c_float,

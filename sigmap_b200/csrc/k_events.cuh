@@ -25,6 +25,8 @@ namespace sb {
 // One block per read.  pA = (float(raw) + offset) * (range / digitisation); keep iff
 // 30 < pA < 200 (signal_batch.cc:196-207).  Kept RAW samples are compacted (order kept)
 // to kept + kept_off[r]; the events kernel redoes the identical conversion.
+// Read r is raw[read_beg[r] .. read_end[r]): reads packed end to end pass read_off and
+// read_off + 1, reads anywhere in a caller's device buffer a start and an end table.
 constexpr int kFilterThreads = 256;
 constexpr int kFilterPerThread = 8;
 
@@ -33,13 +35,14 @@ __device__ __forceinline__ float raw_to_pa(int16_t raw, float offset, float scal
 }
 
 __global__ void __launch_bounds__(kFilterThreads)
-k_filter_compact(const int16_t *__restrict__ raw, const uint64_t *__restrict__ read_off,
+k_filter_compact(const int16_t *__restrict__ raw, const uint64_t *__restrict__ read_beg,
+                 const uint64_t *__restrict__ read_end,
                  const float *__restrict__ dig, const float *__restrict__ range,
                  const float *__restrict__ offset, const uint64_t *__restrict__ kept_off,
                  int16_t *__restrict__ kept, uint32_t *__restrict__ kept_len, uint32_t n_reads) {
   const uint32_t r = blockIdx.x;
   if (r >= n_reads) return;
-  const uint64_t beg = read_off[r], n = read_off[r + 1] - beg;
+  const uint64_t beg = read_beg[r], n = read_end[r] - beg;
   const float off = offset[r], scale = __fdiv_rn(range[r], dig[r]);
   int16_t *out = kept + kept_off[r];
   __shared__ uint32_t warp_tot[kFilterThreads / 32];

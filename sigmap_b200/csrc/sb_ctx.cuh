@@ -133,7 +133,12 @@ struct smb_ctx {
   std::vector<uint32_t> contig_len;
   // uploaded reads
   size_t n_reads = 0;
+  // the read set came from smb_map_reads_device: its samples stayed in the caller's buffer, `raw`
+  // does not hold them, and smb_map_uploaded has nothing to map
+  bool device_input = false;
+  Event ev_input;  // smb_map_reads_device: orders the context's streams after the caller's
   DevBuf<int16_t> raw, kept;
+  // read_off of an upload (n + 1); for device input the n read starts, then the n read ends
   DevBuf<uint64_t> d_read_off, d_kept_off;
   DevBuf<float> d_dig, d_range, d_offset;
   DevBuf<uint32_t> d_kept_len;

@@ -1180,6 +1180,8 @@ int smb_create(smb_ctx **out, int device) {
     if ((e = cudaEventCreate(&ctx->ev_blk_t0[c].h)) != cudaSuccess || (e = cudaEventCreate(&ctx->ev_blk_t1[c].h)) != cudaSuccess ||
         (e = cudaEventCreate(&ctx->ev_cp[c].h)) != cudaSuccess)
       return bail("cudaEventCreate", e);
+  if ((e = cudaEventCreateWithFlags(&ctx->ev_input.h, cudaEventDisableTiming)) != cudaSuccess)
+    return bail("cudaEventCreate", e);
   *out = ctx;
   return SMB_OK;
 }
@@ -1317,37 +1319,49 @@ int smb_shard_world(const smb_ctx *ctx) { return ctx->ex ? ctx->ex->world : 1; }
 // ------------------------------------------------------------ whole hot path
 }  // extern "C"
 
-// device buffers and the per-read tables of a read set (everything but the samples), on stream s
-static int reads_prepare(smb_ctx *ctx, const uint64_t *read_off, const float *dig, const float *range,
+// device buffers and the per-read tables of a read set (everything but the samples and where they
+// lie), on stream s.  pack_off (n_reads + 1): the reads laid end to end, which lays out `kept`.
+static int reads_prepare(smb_ctx *ctx, const uint64_t *pack_off, const float *dig, const float *range,
                          const float *offset, size_t n_reads, cudaStream_t s) {
   ctx->n_reads = n_reads;
   if (n_reads == 0) return SMB_OK;
   if (n_reads > 0xFFFFFFF0ull) return fail(ctx, SMB_ERR_ARG, "too many reads");
-  const uint64_t total = read_off[n_reads];
+  const uint64_t total = pack_off[n_reads];
   ctx->h_kept_off.resize(n_reads);
   ctx->h_offset.assign(offset, offset + n_reads);
   ctx->h_scale.resize(n_reads);
   for (size_t r = 0; r < n_reads; ++r) {
     // 64-sample (128-byte) aligned, non-overlapping regions: the events kernel loads int4
-    ctx->h_kept_off[r] = ((read_off[r] + 63) & ~63ull) + 64ull * r;
+    ctx->h_kept_off[r] = ((pack_off[r] + 63) & ~63ull) + 64ull * r;
     ctx->h_scale[r] = range[r] / dig[r];  // float / float as signal_batch.cc:195
   }
   const uint64_t kept_total = ((total + 63) & ~63ull) + 64ull * n_reads + 64;
-  CK(ctx->raw.ensure(total + 8));
   CK(ctx->kept.ensure(kept_total));
-  CK(ctx->d_read_off.ensure(n_reads + 1));
   CK(ctx->d_kept_off.ensure(n_reads));
   CK(ctx->d_dig.ensure(n_reads));
   CK(ctx->d_range.ensure(n_reads));
   CK(ctx->d_offset.ensure(n_reads));
   CK(ctx->d_kept_len.ensure(n_reads));
   CK(ctx->h_kept_pinned.ensure(n_reads));
-  CK(cudaMemcpyAsync(ctx->d_read_off.p, read_off, (n_reads + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
   CK(cudaMemcpyAsync(ctx->d_kept_off.p, ctx->h_kept_off.data(), n_reads * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
   CK(cudaMemcpyAsync(ctx->d_dig.p, dig, n_reads * sizeof(float), cudaMemcpyHostToDevice, s));
   CK(cudaMemcpyAsync(ctx->d_range.p, range, n_reads * sizeof(float), cudaMemcpyHostToDevice, s));
   CK(cudaMemcpyAsync(ctx->d_offset.p, offset, n_reads * sizeof(float), cudaMemcpyHostToDevice, s));
-  ctx->stats.h2d_bytes += n_reads * 28 + 8;
+  ctx->stats.h2d_bytes += n_reads * 20;
+  return SMB_OK;
+}
+
+// reads_prepare for samples that the call copies from the host into `raw`: read_off goes up as
+// K1's offset table
+static int reads_prepare_host(smb_ctx *ctx, const uint64_t *read_off, const float *dig, const float *range,
+                              const float *offset, size_t n_reads, cudaStream_t s) {
+  ctx->device_input = false;
+  const int rc = reads_prepare(ctx, read_off, dig, range, offset, n_reads, s);
+  if (rc || n_reads == 0) return rc;
+  CK(ctx->raw.ensure(read_off[n_reads] + 8));
+  CK(ctx->d_read_off.ensure(n_reads + 1));
+  CK(cudaMemcpyAsync(ctx->d_read_off.p, read_off, (n_reads + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+  ctx->stats.h2d_bytes += n_reads * 8 + 8;
   return SMB_OK;
 }
 
@@ -1357,7 +1371,7 @@ int smb_reads_upload(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off,
                      const float *range, const float *offset, size_t n_reads) {
   CK(cudaSetDevice(ctx->device));
   cudaStream_t s = ctx->stream;
-  int rc = reads_prepare(ctx, read_off, dig, range, offset, n_reads, s);
+  int rc = reads_prepare_host(ctx, read_off, dig, range, offset, n_reads, s);
   if (rc || n_reads == 0) return rc;
   const uint64_t total = read_off[n_reads];
   CK(cudaMemcpyAsync(ctx->raw.p, raw, total * sizeof(int16_t), cudaMemcpyHostToDevice, s));
@@ -1368,11 +1382,22 @@ int smb_reads_upload(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off,
 
 }  // extern "C"
 
+// K1's input: read r is raw[beg[r] .. end[r])
+struct ReadSource {
+  const int16_t *raw;
+  const uint64_t *beg, *end;
+};
+
+// the samples of smb_reads_upload / smb_map_reads, packed in `raw` as read_off says
+static ReadSource uploaded_source(const smb_ctx *ctx) {
+  return {ctx->raw.p, ctx->d_read_off.p, ctx->d_read_off.p + 1};
+}
+
 // K1 over reads [r0, r1) on stream s: (30,200) pA filter + compaction, kept lengths to the
 // pinned host mirror (no wait here)
-static int filter_slice(smb_ctx *ctx, size_t r0, size_t r1, cudaStream_t s) {
+static int filter_slice(smb_ctx *ctx, const ReadSource &src, size_t r0, size_t r1, cudaStream_t s) {
   if (r1 <= r0) return SMB_OK;
-  k_filter_compact<<<(unsigned)(r1 - r0), kFilterThreads, 0, s>>>(ctx->raw.p, ctx->d_read_off.p + r0, ctx->d_dig.p + r0,
+  k_filter_compact<<<(unsigned)(r1 - r0), kFilterThreads, 0, s>>>(src.raw, src.beg + r0, src.end + r0, ctx->d_dig.p + r0,
                                                                 ctx->d_range.p + r0, ctx->d_offset.p + r0,
                                                                 ctx->d_kept_off.p + r0, ctx->kept.p,
                                                                 ctx->d_kept_len.p + r0, (uint32_t)(r1 - r0));
@@ -1382,14 +1407,14 @@ static int filter_slice(smb_ctx *ctx, size_t r0, size_t r1, cudaStream_t s) {
   return SMB_OK;
 }
 
-// K1 over all uploaded reads, then kept lengths to the host
-static int filter_reads(smb_ctx *ctx) {
+// K1 over all reads of the read set, then kept lengths to the host
+static int filter_reads(smb_ctx *ctx, const ReadSource &src) {
   const size_t n_reads = ctx->n_reads;
   ctx->h_kept_len.resize(n_reads);
   if (!n_reads) return SMB_OK;
   cudaStream_t s = ctx->stream;
   CK(cudaEventRecord(ctx->ev[5], s));
-  int rc = filter_slice(ctx, 0, n_reads, s);
+  int rc = filter_slice(ctx, src, 0, n_reads, s);
   if (rc) return rc;
   CK(cudaEventRecord(ctx->ev[4], s));
   rc = host_sync(ctx);
@@ -1434,10 +1459,14 @@ static int slice_event(smb_ctx *ctx, size_t k, cudaEvent_t *out) {
 
 extern "C" {
 
-static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out, UploadPlan *plan);
+static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out, UploadPlan *plan,
+                             const ReadSource &src);
 
 int smb_map_uploaded(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out) {
-  const int rc = map_uploaded_impl(ctx, prm_in, out, nullptr);
+  if (ctx->device_input)
+    return fail(ctx, SMB_ERR_STATE, "no uploaded reads: the last read set was mapped from device memory "
+                                    "(smb_map_reads_device); upload one with smb_reads_upload or smb_map_reads");
+  const int rc = map_uploaded_impl(ctx, prm_in, out, nullptr, uploaded_source(ctx));
   if (rc) cudaStreamSynchronize(ctx->stream_cp);  // filter-only slices of a failed wave-pipelined call
   // a failed member must not leave its in-process peers waiting at a rendezvous
   if (rc && ctx->local_group) ctx->local_group->abort_all();
@@ -1446,7 +1475,10 @@ int smb_map_uploaded(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out) {
 
 }  // extern "C"
 
-static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out, UploadPlan *plan) {
+// plan == nullptr: K1 runs here over the samples `src` names; otherwise the caller's upload slices
+// have filtered them
+static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out, UploadPlan *plan,
+                             const ReadSource &src) {
   CK(cudaSetDevice(ctx->device));
   if (!ctx->has_index) return fail(ctx, SMB_ERR_STATE, "no index loaded");
   smb_params prm = *prm_in;
@@ -1518,7 +1550,7 @@ static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping
       cudaEvent_t done_ev;
       rc = slice_event(ctx, local_plan.done.size(), &done_ev);
       if (rc) return rc;
-      rc = filter_slice(ctx, r0, r1, ctx->stream_cp);
+      rc = filter_slice(ctx, src, r0, r1, ctx->stream_cp);
       if (rc) return rc;
       CK(cudaEventRecord(done_ev, ctx->stream_cp));
       local_plan.first_read.push_back(r0);
@@ -1530,7 +1562,7 @@ static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping
     plan = &local_plan;
   }
   if (!plan) {
-    rc = filter_reads(ctx);  // K1: part of the mapped path, redone on every call
+    rc = filter_reads(ctx, src);  // K1: part of the mapped path, redone on every call
     if (rc) return rc;
     admit(0, R);
   } else if (sharded_index) {
@@ -1837,9 +1869,10 @@ int smb_map_reads(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off, co
   // copy -> K1 filter of the slice's reads -> kept lengths to the host -> event.  The mapping loop
   // admits a slice's reads once its event has fired, so the rest of the upload hides behind the
   // mapping of the reads that are already there (raw should be pinned host memory for that).
-  int rc = reads_prepare(ctx, read_off, dig, range, offset, n_reads, cs);
+  int rc = reads_prepare_host(ctx, read_off, dig, range, offset, n_reads, cs);
   DeferFrees defer_frees;
   UploadPlan plan;
+  const ReadSource src = uploaded_source(ctx);
   if (!rc && n_reads) {
     const uint64_t slice_samples = ctx->upload_slice_bytes / sizeof(int16_t);
     size_t r0 = 0;
@@ -1856,7 +1889,7 @@ int smb_map_reads(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off, co
         break;
       }
       ctx->stats.h2d_bytes += (b - a) * 2;
-      rc = filter_slice(ctx, r0, r1, cs);
+      rc = filter_slice(ctx, src, r0, r1, cs);
       if (rc) break;
       cudaEventRecord(done_ev, cs);
       plan.first_read.push_back(r0);
@@ -1865,9 +1898,80 @@ int smb_map_reads(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off, co
     }
     plan.first_read.push_back(n_reads);
   }
-  if (!rc) rc = map_uploaded_impl(ctx, params, out, n_reads ? &plan : nullptr);
+  if (!rc) rc = map_uploaded_impl(ctx, params, out, n_reads ? &plan : nullptr, src);
   cudaStreamSynchronize(cs);  // nothing of this call may still be in flight when it returns (or when buffers are freed)
   if (rc) {
+    // a failed member must not leave its in-process peers waiting at a rendezvous
+    if (ctx->local_group) ctx->local_group->abort_all();
+  }
+  return rc;
+}
+
+}  // extern "C"
+
+// raw must be device (or managed) memory of this context's device
+static int check_device_input(smb_ctx *ctx, const void *raw) {
+  cudaPointerAttributes a{};
+  const cudaError_t e = cudaPointerGetAttributes(&a, raw);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ctx, SMB_ERR_ARG, std::string("raw: cudaPointerGetAttributes: ") + cudaGetErrorString(e));
+  }
+  if (a.type == cudaMemoryTypeUnregistered)
+    return fail(ctx, SMB_ERR_ARG, "raw is pageable host memory, not device memory (host samples go through smb_map_reads)");
+  if (a.type == cudaMemoryTypeHost)
+    return fail(ctx, SMB_ERR_ARG, "raw is pinned host memory, not device memory (host samples go through smb_map_reads)");
+  if (a.device != ctx->device)
+    return fail(ctx, SMB_ERR_ARG, "raw is memory of device " + std::to_string(a.device) + ", this context runs on device " +
+                                      std::to_string(ctx->device));
+  return SMB_OK;
+}
+
+static int map_device_impl(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_start, const uint32_t *read_len,
+                           const float *dig, const float *range, const float *offset, size_t n_reads,
+                           const smb_params *params, smb_mapping *out, cudaStream_t caller) {
+  CK(cudaSetDevice(ctx->device));
+  // pack: the reads laid end to end (the kept layout); span: K1's start table, then its end table
+  std::vector<uint64_t> pack(n_reads + 1, 0), span(2 * n_reads);
+  for (size_t r = 0; r < n_reads; ++r) {
+    pack[r + 1] = pack[r] + read_len[r];
+    span[r] = read_start[r];
+    span[n_reads + r] = read_start[r] + read_len[r];
+  }
+  if (pack[n_reads]) {  // raw is not read when every read is empty
+    const int rc = check_device_input(ctx, raw);
+    if (rc) return rc;
+  }
+  // the context's streams do not synchronise with the legacy default stream (NULL): it is waited
+  // for like any other
+  cudaStream_t s = ctx->stream;
+  CK(cudaEventRecord(ctx->ev_input, caller));
+  CK(cudaStreamWaitEvent(s, ctx->ev_input, 0));
+  ctx->device_input = true;
+  int rc = reads_prepare(ctx, pack.data(), dig, range, offset, n_reads, s);
+  if (rc) return rc;
+  if (n_reads) {
+    CK(ctx->d_read_off.ensure(2 * n_reads));
+    CK(cudaMemcpyAsync(ctx->d_read_off.p, span.data(), 2 * n_reads * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    ctx->stats.h2d_bytes += n_reads * 16;
+    // K1 also runs on the copy stream when option pipeline=on cuts the reads into filter-only slices
+    CK(cudaEventRecord(ctx->ev_input, s));
+    CK(cudaStreamWaitEvent(ctx->stream_cp, ctx->ev_input, 0));
+  }
+  return map_uploaded_impl(ctx, params, out, nullptr, {raw, ctx->d_read_off.p, ctx->d_read_off.p + n_reads});
+}
+
+extern "C" {
+
+int smb_map_reads_device(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_start, const uint32_t *read_len,
+                         const float *digitisation, const float *range, const float *offset, size_t n_reads,
+                         const smb_params *params, smb_mapping *out, void *stream) {
+  const int rc = map_device_impl(ctx, raw, read_start, read_len, digitisation, range, offset, n_reads, params, out,
+                                 (cudaStream_t)stream);
+  if (rc) {
+    // the caller may free raw once the call returns: no K1 of a failed call may still be queued
+    cudaStreamSynchronize(ctx->stream);
+    cudaStreamSynchronize(ctx->stream_cp);
     // a failed member must not leave its in-process peers waiting at a rendezvous
     if (ctx->local_group) ctx->local_group->abort_all();
   }
@@ -1881,7 +1985,7 @@ int smb_stage_raw_to_pa(smb_ctx *ctx, const int16_t *raw, size_t n, float dig, f
   uint64_t off[2] = {0, n};
   int rc = smb_reads_upload(ctx, raw, off, &dig, &range, &offset, 1);
   if (rc) return rc;
-  rc = filter_reads(ctx);
+  rc = filter_reads(ctx, uploaded_source(ctx));
   if (rc) return rc;
   const uint32_t kept = ctx->h_kept_len[0];
   *n_out = kept;

@@ -74,6 +74,7 @@ class Mapper:
             msg = F.lib.smb_last_error(None).decode()
             self._ctx = None
             raise SigmapError(f"smb_create failed ({rc}): {msg}")
+        self.device = device
         self.contig_lengths = None
 
     def close(self):
@@ -244,6 +245,58 @@ class Mapper:
         return Rows(out, reads.n)
 
     StreamingMap = map_reads
+
+    def map_device(self, raw, read_start, read_len, digitisation, range_, offset, params=None,
+                   stream=None):
+        """Map reads whose samples are already in device memory (smb_map_reads_device): raw is a
+        contiguous torch.int16 CUDA tensor on this mapper's device, of any shape, read as flat
+        elements; read r is raw.view(-1)[read_start[r] : read_start[r] + read_len[r]].  The samples
+        are not copied, and raw is not written.  The per-read tables are host arrays (or tensors).
+        The call's device work is ordered after what is queued on `stream` (a torch.cuda.Stream or
+        a cudaStream_t handle; default: the device's current torch stream).  Returns the rows
+        map_reads returns for the same samples."""
+        import torch
+        if not isinstance(raw, torch.Tensor):
+            raise SigmapError(f"map_device: raw must be a torch tensor, not {type(raw).__name__}")
+        if raw.dtype != torch.int16:
+            raise SigmapError(f"map_device: raw must be torch.int16, not {raw.dtype}")
+        if raw.device != torch.device("cuda", self.device):
+            raise SigmapError(f"map_device: raw is on {raw.device}, this mapper runs on cuda:{self.device}")
+        if not raw.is_contiguous():
+            raise SigmapError("map_device: raw must be contiguous")
+
+        def table(x, dtype):
+            if isinstance(x, torch.Tensor):
+                x = x.cpu().numpy()
+            return np.ascontiguousarray(x, dtype).reshape(-1)
+
+        start, length = table(read_start, np.uint64), table(read_len, np.uint32)
+        dig, rng, off = table(digitisation, np.float32), table(range_, np.float32), table(offset, np.float32)
+        n = len(start)
+        if not len(length) == len(dig) == len(rng) == len(off) == n:
+            raise SigmapError("map_device: read_start, read_len, digitisation, range_ and offset "
+                              "must have one entry per read")
+        if n and int((start + length).max()) > raw.numel():
+            raise SigmapError(f"map_device: a read ends past the {raw.numel()} elements of raw")
+        if stream is None:
+            stream = torch.cuda.current_stream(raw.device)
+        handle = stream.cuda_stream if isinstance(stream, torch.cuda.Stream) else int(stream)
+        params = params or default_params()
+        out = (F.Mapping * max(n, 1))()
+        self._check(F.lib.smb_map_reads_device(self._ctx, raw.data_ptr(), F.ptr(start, F.u64p),
+                                               F.ptr(length, F.u32p), F.ptr(dig, F.f32p), F.ptr(rng, F.f32p),
+                                               F.ptr(off, F.f32p), n, C.byref(params), out, handle),
+                    "smb_map_reads_device")
+        return Rows(out, n)
+
+    def map_device_padded(self, batch, lengths, digitisation, range_, offset, params=None,
+                          stream=None):
+        """map_device over the rows of a padded [n, stride] batch: read r is batch[r, :lengths[r]]."""
+        if batch.dim() != 2:
+            raise SigmapError(f"map_device_padded: batch must be [n, stride], not {list(batch.shape)}")
+        n, stride = batch.shape
+        read_start = np.arange(n, dtype=np.uint64) * np.uint64(stride)
+        return self.map_device(batch, read_start, lengths, digitisation, range_, offset, params, stream)
 
     def paf_lines(self, reads, rows, contig_names, mt_ms=0.0):
         out = []
