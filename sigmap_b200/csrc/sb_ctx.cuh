@@ -111,7 +111,7 @@ struct smb_ctx {
   int prep_rounds = 0;            // SMB_PREP_ROUNDS=n: settle rounds inside k_chain_prep (0 = none; smb_create: kPrepRounds)
   uint32_t dp_pass_max_entries = 0;  // SMB_DP_TILES=n: per-tile DP pass up to n chunks per step (0 = never;
                                      // smb_create: kDpPassMaxEntries)
-  int pipeline_mode = 0;          // SMB_PIPELINE=auto|on|off: wave-pipelined ticks (see map_uploaded_impl)
+  int pipeline_mode = 0;          // SMB_PIPELINE=auto|on|off: wave-pipelined ticks (see map_read_set)
   uint32_t cloud_tile = 16384;    // SMB_CLOUD_TILE=n: window starts per tile of the device cloud's point selection
   smb_build_stats build_stats{};  // the last device cloud build (smb_index_build_stats)
   PinnedBuf<unsigned char> h_cloud_stage;  // two upload slices of the device cloud build
@@ -119,13 +119,13 @@ struct smb_ctx {
   unsigned dp_grid = 148 * 8;     // persistent DP grid: every block that fits on the device
   bool part_sort = true;          // SMB_SORT=entry: always the one-CTA-per-entry sort (k_seg_sort)
   bool seg_sort = true;           // per-entry shared-memory sort; SMB_SORT=global forces the radix sort
-  Stream stream_cp;  // smb_map_reads: upload slices (copy + K1 filter) run here, under the mapping
+  Stream stream_cp;  // the slices of every mapping call (host input: copy + K1; otherwise K1) run here
   std::vector<Event> slice_events;
   size_t upload_slice_bytes = 64u << 20;  // SMB_UPLOAD_SLICE_MB=n
   PinnedBuf<uint32_t> h_kept_pinned;  // kept length of every read, written by the device
   Stream stream_ev;  // lookahead event blocks run here, next to the mapping rounds
   Event ev_blk_t0[2], ev_blk_t1[2];
-  Event ev_cp[2];  // first / last filter-only slice of a wave-pipelined call (copy stream)
+  Event ev_cp[2];  // around a mapping call's slices on the copy stream (K1 time of resident / device input)
   bool ev_overlap = true;            // SMB_EVENTS_OVERLAP=0: compute every block when it is needed
   double ev_survival_hint = 0.0;     // share of reads that went past their first chunk in the last call
   uint32_t ev_warp_max = 2048;    // event batches up to this many chunks run warp-per-chunk in shared memory

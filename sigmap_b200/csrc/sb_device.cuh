@@ -30,9 +30,10 @@ constexpr int kFan = 8;                 // children per node; a warp tests 4 nod
 constexpr int kMaxLevels = 12;          // 8^12 leaves: never reached below 2^32 points
 
 // cudaFree waits for the whole device -- including an upload still queued on the copy stream,
-// which would serialise the upload and the mapping it is supposed to hide behind.  While
-// defer_frees() is on (smb_map_reads), buffers that have to grow park their old allocation here;
-// it is released when the call is over and every stream is idle.
+// which would serialise the upload and the mapping it is supposed to hide behind.  While a
+// mapping call's DeferFrees (sb_engine.cu) is alive, buffers that have to grow park their old
+// allocation here; it is released when the call's mapping is over (after a failure, cudaFree then
+// waits for whatever the call left queued).
 struct FreeLater {
   static inline thread_local bool on = false;
   static inline thread_local std::vector<void *> parked;

@@ -20,6 +20,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <memory>
+#include <optional>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 #include <string>
@@ -1382,10 +1383,13 @@ int smb_reads_upload(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off,
 
 }  // extern "C"
 
-// K1's input: read r is raw[beg[r] .. end[r])
+// K1's input: read r is raw[beg[r] .. end[r]).  host != nullptr (smb_map_reads): the call first
+// copies the samples from host, packed as host_off says, into raw, slice by slice.
 struct ReadSource {
   const int16_t *raw;
   const uint64_t *beg, *end;
+  const int16_t *host = nullptr;
+  const uint64_t *host_off = nullptr;
 };
 
 // the samples of smb_reads_upload / smb_map_reads, packed in `raw` as read_off says
@@ -1407,33 +1411,14 @@ static int filter_slice(smb_ctx *ctx, const ReadSource &src, size_t r0, size_t r
   return SMB_OK;
 }
 
-// K1 over all reads of the read set, then kept lengths to the host
-static int filter_reads(smb_ctx *ctx, const ReadSource &src) {
-  const size_t n_reads = ctx->n_reads;
-  ctx->h_kept_len.resize(n_reads);
-  if (!n_reads) return SMB_OK;
-  cudaStream_t s = ctx->stream;
-  CK(cudaEventRecord(ctx->ev[5], s));
-  int rc = filter_slice(ctx, src, 0, n_reads, s);
-  if (rc) return rc;
-  CK(cudaEventRecord(ctx->ev[4], s));
-  rc = host_sync(ctx);
-  if (rc) return rc;
-  memcpy(ctx->h_kept_len.data(), ctx->h_kept_pinned.p, n_reads * sizeof(uint32_t));
-  float ms = 0;
-  cudaEventElapsedTime(&ms, ctx->ev[5], ctx->ev[4]);
-  ctx->stats.ms_filter += ms;
-  return SMB_OK;
-}
-
-// smb_map_reads: the samples arrive in slices on the copy stream while earlier slices are being
-// mapped.  Slice k = reads [first_read[k], first_read[k+1]); done[k] fires once the slice has been
-// copied, filtered, and its kept lengths are in the pinned host mirror.
+// The read set as the copy stream delivers it to the mapping loop.  Slice k = reads
+// [first_read[k], first_read[k+1]); done[k] fires once the slice's samples are on the device, have
+// been filtered, and its kept lengths are in the pinned host mirror.
 struct UploadPlan {
   std::vector<size_t> first_read;
   std::vector<cudaEvent_t> done;
   size_t admitted = 0;  // slices handed to the mapping loop so far
-  size_t n_slices() const { return done.size(); }
+  bool pending() const { return admitted < done.size(); }
 };
 
 // from construction to destruction no cudaFree (it waits for the whole device, i.e. for the queued
@@ -1457,145 +1442,134 @@ static int slice_event(smb_ctx *ctx, size_t k, cudaEvent_t *out) {
   return SMB_OK;
 }
 
-extern "C" {
-
-static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out, UploadPlan *plan,
-                             const ReadSource &src);
-
-int smb_map_uploaded(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out) {
-  if (ctx->device_input)
-    return fail(ctx, SMB_ERR_STATE, "no uploaded reads: the last read set was mapped from device memory "
-                                    "(smb_map_reads_device); upload one with smb_reads_upload or smb_map_reads");
-  const int rc = map_uploaded_impl(ctx, prm_in, out, nullptr, uploaded_source(ctx));
-  if (rc) cudaStreamSynchronize(ctx->stream_cp);  // filter-only slices of a failed wave-pipelined call
-  // a failed member must not leave its in-process peers waiting at a rendezvous
-  if (rc && ctx->local_group) ctx->local_group->abort_all();
-  return rc;
+// Enqueues the read set on the copy stream in slices of consecutive reads, each: [its samples
+// copied from src.host] -> K1 over its reads -> kept lengths to the host -> its done event, with
+// ev_cp[0] / ev_cp[1] around all of them.  A slice takes one read, then more while they fit in
+// slice_samples (host input: as read_off packs them; otherwise in the kept layout);
+// slice_samples = 0: one slice of every read.
+static int plan_slices(smb_ctx *ctx, const ReadSource &src, uint64_t slice_samples, UploadPlan &plan) {
+  const size_t R = ctx->n_reads;
+  cudaStream_t cs = ctx->stream_cp;
+  CK(cudaEventRecord(ctx->ev_cp[0], cs));
+  for (size_t r0 = 0, r1; r0 < R; r0 = r1) {
+    r1 = slice_samples ? r0 + 1 : R;
+    if (src.host)
+      while (r1 < R && src.host_off[r1 + 1] - src.host_off[r0] <= slice_samples) ++r1;
+    else
+      while (r1 < R && ctx->h_kept_off[r1] - ctx->h_kept_off[r0] <= slice_samples) ++r1;
+    cudaEvent_t done;
+    int rc = slice_event(ctx, plan.done.size(), &done);
+    if (rc) return rc;
+    if (src.host) {
+      const uint64_t a = src.host_off[r0], b = src.host_off[r1];
+      const cudaError_t ce =
+          cudaMemcpyAsync(ctx->raw.p + a, src.host + a, (b - a) * sizeof(int16_t), cudaMemcpyHostToDevice, cs);
+      if (ce != cudaSuccess) return fail(ctx, SMB_ERR_CUDA, std::string("upload slice: ") + cudaGetErrorString(ce));
+      ctx->stats.h2d_bytes += (b - a) * 2;
+    }
+    rc = filter_slice(ctx, src, r0, r1, cs);
+    if (rc) return rc;
+    CK(cudaEventRecord(done, cs));
+    plan.first_read.push_back(r0);
+    plan.done.push_back(done);
+  }
+  plan.first_read.push_back(R);
+  CK(cudaEventRecord(ctx->ev_cp[1], cs));
+  return SMB_OK;
 }
 
-}  // extern "C"
+// K1 time of a read set filtered on the copy stream (not for host input, whose slices also copy)
+static int add_filter_time(smb_ctx *ctx) {
+  CK(cudaEventSynchronize(ctx->ev_cp[1]));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, ctx->ev_cp[0], ctx->ev_cp[1]));
+  ctx->stats.ms_filter += ms;
+  return SMB_OK;
+}
 
-// plan == nullptr: K1 runs here over the samples `src` names; otherwise the caller's upload slices
-// have filtered them
-static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out, UploadPlan *plan,
-                             const ReadSource &src) {
-  CK(cudaSetDevice(ctx->device));
-  if (!ctx->has_index) return fail(ctx, SMB_ERR_STATE, "no index loaded");
-  smb_params prm = *prm_in;
-  if (prm.step_size < 1) return fail(ctx, SMB_ERR_ARG, "step_size must be >= 1");
-  const size_t R = ctx->n_reads;
-  SlotSpace &sp = ctx->map_slots;
-  int rc = slots_init(ctx, sp, (uint32_t)R);
-  if (rc) return rc;
-  // The loop below advances in TICKS: tick t maps the next chunk of every active read.  Reads join
-  // ("are admitted") at a tick boundary -- all of them at tick 0 when the samples are already on
-  // the device, slice by slice as the copy stream delivers them otherwise -- so read r is at chunk
-  // t - t_admit[r]; which reads share a tick changes the composition of the batches, never a row.
-  std::vector<uint32_t> n_chunks(R, 0), chunks_used(R, 1), t_admit(R, 0);
-  std::vector<uint32_t> active;
-  uint32_t round = 0;  // the tick
-  ctx->h_kept_len.resize(R);
-  auto chunk_limit = [&](uint32_t r) { return std::min<uint32_t>(n_chunks[r], (uint32_t)prm.max_num_chunks); };
-  auto admit = [&](size_t r0, size_t r1) {
-    for (size_t r = r0; r < r1; ++r) {
+// Event detection does not depend on the mapping state, only on the raw signal, and its kernels
+// are one-thread-per-chunk sequential scans that want as many chunks per launch as possible.  So
+// events run in LOOKAHEAD BLOCKS: the next `depth` chunks of every read active at tick r0 in one
+// launch, cached as feature rows (two feature caches, so that the next block can be computed on
+// the event stream while the ticks of the current one are being mapped; a block is handed over
+// with a host wait on its event).
+struct EvBlock {
+  uint32_t r0 = 0, r1 = 0;            // ticks covered
+  bool ready = false;                 // launched, not yet consumed
+  std::vector<uint32_t> row_base;     // per read: first row of the read in the block's cache
+  std::vector<uint64_t> cs;           // host chunk table (kept alive until the block is consumed)
+  std::vector<float> co, csc;
+};
+constexpr uint32_t kEvRowCap = 96u << 10;
+
+// The read scheduler of a mapping call, which advances in TICKS: tick t maps the next chunk of
+// every active read.  Reads join ("are admitted") at a tick boundary, slice by slice as the copy
+// stream delivers them, so read r is at chunk t - t_admit[r]; which reads share a tick changes the
+// composition of the batches, never a row.  The two tick policies, run_blocks and run_waves, work
+// on this state.
+struct Sched {
+  smb_ctx *ctx;
+  SlotSpace &sp;
+  const smb_params &prm;
+  const size_t R;
+  UploadPlan plan;
+  std::vector<uint32_t> n_chunks, chunks_used, t_admit;
+  uint32_t round = 0;                          // the tick
+  std::vector<RoundInfo> info;                 // of the reads of the last tick
+  uint64_t first_active = 0, after_first = 0;  // reads that had a first chunk / went past it
+  EvBlock blk[2];
+  int cur = 0;  // the block the ticks read
+
+  Sched(smb_ctx *c, SlotSpace &s, const smb_params &p)
+      : ctx(c), sp(s), prm(p), R(c->n_reads), n_chunks(R, 0), chunks_used(R, 1), t_admit(R, 0) {}
+
+  uint32_t chunk_limit(uint32_t r) const { return std::min<uint32_t>(n_chunks[r], (uint32_t)prm.max_num_chunks); }
+
+  // Takes the plan's next slice if it has arrived (wait: once it has).  Its kept lengths go to
+  // h_kept_len and n_chunks, and its reads that have a whole chunk to map to `into`.  *took =
+  // false: no slice is left, or the next one has not arrived.
+  int take_slice(bool wait, std::vector<uint32_t> &into, bool *took) {
+    *took = false;
+    if (!plan.pending()) return SMB_OK;
+    const size_t k = plan.admitted;
+    const cudaError_t q = cudaEventQuery(plan.done[k]);
+    if (q == cudaErrorNotReady) {
+      if (!wait) return SMB_OK;
+      ctx->stats.sync_points++;
+      CK(cudaEventSynchronize(plan.done[k]));
+    } else if (q != cudaSuccess) {
+      return fail(ctx, SMB_ERR_CUDA, std::string("upload slice: ") + cudaGetErrorString(q));
+    }
+    for (size_t r = plan.first_read[k]; r < plan.first_read[k + 1]; ++r) {
       ctx->h_kept_len[r] = ctx->h_kept_pinned.p[r];
       n_chunks[r] = ctx->h_kept_len[r] / kChunk;  // tail dropped, sigmap.cc:643
-      t_admit[r] = round;
-      if (n_chunks[r] > 0 && prm.max_num_chunks > 0) active.push_back((uint32_t)r);
+      if (n_chunks[r] > 0 && prm.max_num_chunks > 0) into.push_back((uint32_t)r);
     }
-  };
-  // slices the copy stream has finished (wait = true: block for the next one)
-  auto admit_ready = [&](bool wait) -> int {
-    while (plan && plan->admitted < plan->n_slices()) {
-      const size_t k = plan->admitted;
-      cudaError_t q = cudaEventQuery(plan->done[k]);
-      if (q == cudaErrorNotReady) {
-        if (!wait) break;
-        ctx->stats.sync_points++;
-        CK(cudaEventSynchronize(plan->done[k]));
-      } else if (q != cudaSuccess) {
-        return fail(ctx, SMB_ERR_CUDA, std::string("upload slice: ") + cudaGetErrorString(q));
-      }
-      admit(plan->first_read[k], plan->first_read[k + 1]);
-      plan->admitted++;
-      wait = false;  // one is enough to go on; take whatever else is ready
-    }
+    plan.admitted++;
+    *took = true;
     return SMB_OK;
-  };
-  auto uploads_pending = [&]() { return plan && plan->admitted < plan->n_slices(); };
-  // Wave-pipelined ticks (below) when the stop rules retire most reads after their first chunk
-  // (known from the previous call; a fresh context starts this way): K1 and the events of the next
-  // wave run while the current one is being mapped (option pipeline=on: also with resident samples,
-  // which then join in waves of filter-only slices).  Contig shards must run identical ticks on every
-  // rank: no timing-dependent admission there.
-  const bool sharded_index = ctx->ex && ctx->index.sharded;
-  // auto: only when the samples arrive from the host during the call.  With resident samples the
-  // GPU is busy mapping from the first tick on and the overlap only adds contention and steps
-  // (measured on config 3: 437 ms pipelined against 403 ms; with host buffers on two GPUs e2e
-  // 1.65 against 1.58 G samples/s).
-  const bool pipeline = !sharded_index && R > 0 && prm.max_num_chunks > 0 &&
-                        (ctx->pipeline_mode == 1 ||
-                         (ctx->pipeline_mode == 0 && plan != nullptr && ctx->ev_survival_hint <= 0.5));
-  UploadPlan local_plan;
-  std::unique_ptr<DeferFrees> local_defer;
-  if (!plan && pipeline) {
-    // samples resident: slices that only filter (K1 on the copy stream, kept lengths to the host)
-    local_defer.reset(new DeferFrees());
-    const uint64_t slice_samples = std::max<uint64_t>(ctx->upload_slice_bytes / sizeof(int16_t), 1);
-    CK(cudaEventRecord(ctx->ev_cp[0], ctx->stream_cp));
-    size_t r0 = 0;
-    while (r0 < R) {
-      size_t r1 = r0 + 1;
-      while (r1 < R && ctx->h_kept_off[r1] - ctx->h_kept_off[r0] <= slice_samples) ++r1;
-      cudaEvent_t done_ev;
-      rc = slice_event(ctx, local_plan.done.size(), &done_ev);
-      if (rc) return rc;
-      rc = filter_slice(ctx, src, r0, r1, ctx->stream_cp);
-      if (rc) return rc;
-      CK(cudaEventRecord(done_ev, ctx->stream_cp));
-      local_plan.first_read.push_back(r0);
-      local_plan.done.push_back(done_ev);
-      r0 = r1;
-    }
-    CK(cudaEventRecord(ctx->ev_cp[1], ctx->stream_cp));
-    local_plan.first_read.push_back(R);
-    plan = &local_plan;
   }
-  if (!plan) {
-    rc = filter_reads(ctx, src);  // K1: part of the mapped path, redone on every call
-    if (rc) return rc;
-    admit(0, R);
-  } else if (sharded_index) {
-    // contig shards must run identical ticks on every rank: no timing-dependent admission
-    while (uploads_pending()) {
-      rc = admit_ready(true);
-      if (rc) return rc;
+
+  // the end of a tick that mapped `act` (info[i] is act[i]'s): chunks used, the survival counts,
+  // and the reads that go on to another chunk appended to `next`
+  void end_tick(const std::vector<uint32_t> &act, std::vector<uint32_t> &next) {
+    ctx->stats.samples += (uint64_t)act.size() * kChunk;
+    for (size_t i = 0; i < act.size(); ++i) {
+      const uint32_t r = act[i];
+      const uint32_t done = round + 1 - t_admit[r];
+      chunks_used[r] = done;
+      const bool more = !info[i].stop && done < n_chunks[r] && done < (uint32_t)prm.max_num_chunks;
+      if (done == 1) {
+        ++first_active;
+        if (more) ++after_first;
+      }
+      if (more) next.push_back(r);
     }
+    ++round;
   }
-  std::vector<RoundInfo> info;
-  const std::vector<uint32_t> none;
-  // Event detection does not depend on the mapping state, only on the raw signal, and its
-  // kernels are one-thread-per-chunk sequential scans that want as many chunks per launch as
-  // possible.  So events run in LOOKAHEAD BLOCKS: the next `depth` chunks of every read active at
-  // tick r0 in one launch, cached as feature rows; the block is several ticks deep only while most
-  // reads survive from tick to tick (full-read mapping), one tick deep when the stop rules retire
-  // most reads after their first chunk or while reads are still being admitted.  The kernels are
-  // latency-bound and leave the SMs almost idle, so the NEXT block is computed on the event stream
-  // while the ticks of the current one are being mapped (two feature caches); a block is handed
-  // over with a host wait on its event.
-  const uint32_t kEvRowCap = 96u << 10;
-  struct EvBlock {
-    uint32_t r0 = 0, r1 = 0;            // ticks covered
-    bool ready = false;                 // launched, not yet consumed
-    std::vector<uint32_t> row_base;     // per read: first row of the read in the block's cache
-    std::vector<uint64_t> cs;           // host chunk table (kept alive until the block is consumed)
-    std::vector<float> co, csc;
-  } blk[2];
-  int cur = 0;            // block being mapped (blk[cur].r0 <= round < blk[cur].r1 once consumed)
-  bool have_next = false; // blk[1 - cur] holds a launched block for round == blk[cur].r1
-  size_t prev_active = 0;
+
   // enqueue the events of ticks [r0, r0 + depth) of `who` on the event stream, into cache `c`
-  auto launch_block = [&](int c, uint32_t r0, uint32_t depth, const std::vector<uint32_t> &who) -> int {
+  int launch_block(int c, uint32_t r0, uint32_t depth, const std::vector<uint32_t> &who) {
     EvBlock &b = blk[c];
     Workspace &w = ctx->ws;
     cudaStream_t s = ctx->stream_ev;
@@ -1629,16 +1603,17 @@ static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping
       CK(cudaMemcpyAsync(w.blk_chunk_scale.p, b.csc.data(), rows * sizeof(float), cudaMemcpyHostToDevice, s));
       ctx->stats.h2d_bytes += rows * 16ull;
       const ChunkTable ct{w.blk_chunk_start.p, w.blk_chunk_offset.p, w.blk_chunk_scale.p};
-      int rc2 = run_events(ctx, SRC_RAW_KEPT, ctx->kept.p, rows, nullptr, w.feat_cache[c].p, w.nf_cache[c].p,
-                           w.nraw_cache[c].p, s, &ct);
-      if (rc2) return rc2;
+      int rc = run_events(ctx, SRC_RAW_KEPT, ctx->kept.p, rows, nullptr, w.feat_cache[c].p, w.nf_cache[c].p,
+                          w.nraw_cache[c].p, s, &ct);
+      if (rc) return rc;
     }
     CK(cudaEventRecord(ctx->ev_blk_t1[c], s));
     b.ready = true;
     return SMB_OK;
-  };
+  }
+
   // wait for block `c` and make it the one the ticks read
-  auto consume_block = [&](int c) -> int {
+  int consume_block(int c) {
     ctx->stats.sync_points++;
     CK(cudaEventSynchronize(ctx->ev_blk_t1[c]));
     float ms = 0;
@@ -1648,147 +1623,55 @@ static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping
     cur = c;
     ctx->ws.cache_cur = c;
     return SMB_OK;
-  };
-  uint64_t first_active = 0, after_first = 0;  // reads that had a first chunk / went past it
-  if (pipeline) {
-    // ---- wave-pipelined ticks.  Every tick maps the reads of ONE event block (one tick deep); while
-    // it is being mapped, the block of the next tick is computed on the event stream for the reads
-    // that are known by then: the survivors of the PREVIOUS tick (they wait one tick, carried forward
-    // as absent slots) and the reads whose slices have arrived since -- at most one step's worth.  So
-    // neither K1 nor event detection is ever waited for after the first wave, however the reads
-    // arrive.  A read's chunk at tick T is T - t_admit[r]; t_admit is (re)set whenever the read is
-    // put into a block, which is all that "waiting a tick" takes.  Which reads share a tick changes
-    // the composition of batches, never a row.
-    std::vector<uint32_t> done_chunks(R, 0), members[2], waiting, absent;
-    auto want_reads = [&]() -> size_t {
-      const uint64_t by_anchors = (uint64_t)(0.6 * (double)ctx->max_batch_anchors / std::max(ctx->est_anchors_per_chunk, 1.0));
-      return (size_t)std::max<uint64_t>(1, std::min<uint64_t>(by_anchors, ctx->max_batch_chunks));
-    };
-    // reads of the slices that have arrived, in order, at most `cap` of them; wait = true: block
-    // until at least `min_new` reads have joined or no slice is left
-    auto gather_new = [&](std::vector<uint32_t> &into, size_t min_new, size_t cap, bool wait) -> int {
-      size_t got = 0;
-      while (plan->admitted < plan->n_slices() && got < cap) {
-        const size_t k = plan->admitted;
-        cudaError_t q = cudaEventQuery(plan->done[k]);
-        if (q == cudaErrorNotReady) {
-          if (!wait || got >= min_new) break;
-          ctx->stats.sync_points++;
-          CK(cudaEventSynchronize(plan->done[k]));
-        } else if (q != cudaSuccess) {
-          return fail(ctx, SMB_ERR_CUDA, std::string("upload slice: ") + cudaGetErrorString(q));
-        }
-        for (size_t r = plan->first_read[k]; r < plan->first_read[k + 1]; ++r) {
-          ctx->h_kept_len[r] = ctx->h_kept_pinned.p[r];
-          n_chunks[r] = ctx->h_kept_len[r] / kChunk;  // tail dropped, sigmap.cc:643
-          if (n_chunks[r] > 0) {
-            into.push_back((uint32_t)r);
-            ++got;
-          }
-        }
-        plan->admitted++;
-      }
-      return SMB_OK;
-    };
-    auto launch_for = [&](int c, uint32_t tick) -> int {
-      for (uint32_t r : members[c]) t_admit[r] = tick - done_chunks[r];
-      return launch_block(c, tick, 1, members[c]);
-    };
-    int c = 0;
-    bool have_blk = false;  // blk[c] has been launched for tick `round` with members[c]
-    for (;;) {
-      if (!have_blk) {
-        // nothing was prefetched for this tick: whoever is waiting, plus new reads (a batch, or
-        // what is left of the input)
-        members[c].swap(waiting);
-        waiting.clear();
-        const size_t want = want_reads();
-        if (members[c].size() < want && uploads_pending()) {
-          const size_t room = want - members[c].size();
-          rc = gather_new(members[c], (room + 1) / 2, room, true);
-          if (rc) return rc;
-        }
-        if (members[c].empty()) {
-          if (!uploads_pending()) break;
-          continue;  // slices without a single whole chunk
-        }
-        rc = launch_for(c, round);
-        if (rc) return rc;
-      }
-      rc = consume_block(c);
-      if (rc) return rc;
-      have_blk = false;
-      const std::vector<uint32_t> &act = members[c];
-      // the next tick's block while this one is mapped
-      absent.clear();
-      for (uint32_t r : waiting)
-        if (sp.h_nchains[r] > 0) absent.push_back(r);
-      if (ctx->ev_overlap) {
-        std::vector<uint32_t> &nx = members[1 - c];
-        nx.swap(waiting);
-        waiting.clear();
-        const size_t want = want_reads();
-        if (nx.size() < want && uploads_pending()) {
-          rc = gather_new(nx, 0, want - nx.size(), false);
-          if (rc) return rc;
-        }
-        if (!nx.empty()) {
-          rc = launch_for(1 - c, round + 1);
-          if (rc) return rc;
-          have_blk = true;
-        }
-      }
-      const std::vector<uint32_t> &row_base = blk[c].row_base;
-      auto fill = [&](StepEntries &en, size_t first, uint32_t count) {
-        en.feat_row.resize(count);
-        for (uint32_t i = 0; i < count; ++i) en.feat_row[i] = row_base[act[first + i]];
-      };
-      RoundOut rout;
-      rout.ids = &act;
-      rout.info = &info;
-      rc = run_round(ctx, sp, act, absent, SRC_CACHED, prm, fill, &rout);
-      if (rc) return rc;
-      ctx->stats.samples += (uint64_t)act.size() * kChunk;
-      for (size_t i = 0; i < act.size(); ++i) {
-        const uint32_t r = act[i];
-        const uint32_t dc = round + 1 - t_admit[r];
-        chunks_used[r] = dc;
-        done_chunks[r] = dc;
-        const bool more = dc < n_chunks[r] && dc < (uint32_t)prm.max_num_chunks;
-        if (dc == 1) {
-          ++first_active;
-          if (!info[i].stop && more) ++after_first;
-        }
-        if (!info[i].stop && more) waiting.push_back(r);
-      }
-      ++round;
-      if (have_blk) c = 1 - c;
-    }
-    if (plan == &local_plan) {  // K1 time of the call: first to last filter-only slice on the copy stream
-      float ms = 0;
-      if (cudaEventElapsedTime(&ms, ctx->ev_cp[0], ctx->ev_cp[1]) == cudaSuccess) ctx->stats.ms_filter += ms;
-    }
   }
-  while (!pipeline && (!active.empty() || uploads_pending())) {
-    if (round >= blk[cur].r1) {
-      // a block boundary: the only place reads are admitted (every row of a block then belongs
-      // to a read that was there when the block was launched)
-      rc = admit_ready(active.empty());
+};
+
+// Ticks in lookahead event blocks.  A block is several ticks deep only while most reads survive
+// from tick to tick (full-read mapping), one tick deep when the stop rules retire most reads after
+// their first chunk or while reads are still being admitted.  The kernels are latency-bound and
+// leave the SMs almost idle, so the NEXT block is computed while the current one is being mapped.
+static int run_blocks(Sched &S) {
+  smb_ctx *ctx = S.ctx;
+  std::vector<uint32_t> active;
+  const std::vector<uint32_t> none;
+  bool have_next = false;  // blk[1 - cur] holds a launched block for round == blk[cur].r1
+  size_t prev_active = 0;
+  int rc;
+  bool took;
+  // contig shards must run identical ticks on every rank: no timing-dependent admission
+  if (ctx->ex && ctx->index.sharded)
+    while (S.plan.pending()) {
+      rc = S.take_slice(true, active, &took);
       if (rc) return rc;
+    }
+  while (!active.empty() || S.plan.pending()) {
+    const uint32_t round = S.round;
+    if (round >= S.blk[S.cur].r1) {
+      // a block boundary: the only place reads are admitted (every row of a block then belongs
+      // to a read that was there when the block was launched).  Wait for a slice only when no
+      // read is active.
+      const size_t n0 = active.size();
+      bool wait = active.empty();
+      do {
+        rc = S.take_slice(wait, active, &took);
+        if (rc) return rc;
+        wait = false;  // one is enough to go on; take whatever else is ready
+      } while (took);
+      for (size_t i = n0; i < active.size(); ++i) S.t_admit[active[i]] = round;
       if (active.empty()) continue;  // that slice held no read with a whole chunk
       // (a prefetched block is only ever launched once every slice has been admitted, so it
       // covers every read that is active now)
-      if (have_next && blk[1 - cur].r0 == round) {
-        rc = consume_block(1 - cur);
+      if (have_next && S.blk[1 - S.cur].r0 == round) {
+        rc = S.consume_block(1 - S.cur);
         if (rc) return rc;
       } else {
         uint32_t depth = 1;
-        if (round > 0 && !uploads_pending() && active.size() * 2 > prev_active)
+        if (round > 0 && !S.plan.pending() && active.size() * 2 > prev_active)
           depth = (uint32_t)std::min<size_t>(8, std::max<size_t>(1, kEvRowCap / active.size()));
-        const int c = round == 0 ? 0 : 1 - cur;
-        rc = launch_block(c, round, depth, active);
+        const int c = round == 0 ? 0 : 1 - S.cur;
+        rc = S.launch_block(c, round, depth, active);
         if (rc) return rc;
-        rc = consume_block(c);
+        rc = S.consume_block(c);
         if (rc) return rc;
       }
       have_next = false;
@@ -1796,118 +1679,204 @@ static int map_uploaded_impl(smb_ctx *ctx, const smb_params *prm_in, smb_mapping
     // the block after this one, while this one is being mapped: worth it only while most reads
     // go on from tick to tick (known from the previous tick; for tick 0 from the last call) and
     // nobody is waiting to be admitted
-    if (ctx->ev_overlap && !have_next && !uploads_pending()) {
+    if (ctx->ev_overlap && !have_next && !S.plan.pending()) {
       const bool surviving = round > 0 ? active.size() * 2 > prev_active : ctx->ev_survival_hint > 0.5;
       if (surviving) {
-        const uint32_t r0n = blk[cur].r1;
+        const uint32_t r0n = S.blk[S.cur].r1;
         std::vector<uint32_t> who;
         who.reserve(active.size());
         for (uint32_t r : active)
-          if (chunk_limit(r) > r0n - t_admit[r]) who.push_back(r);
+          if (S.chunk_limit(r) > r0n - S.t_admit[r]) who.push_back(r);
         if (!who.empty()) {
           const uint32_t depth = (uint32_t)std::min<size_t>(8, std::max<size_t>(1, kEvRowCap / who.size()));
-          rc = launch_block(1 - cur, r0n, depth, who);
+          rc = S.launch_block(1 - S.cur, r0n, depth, who);
           if (rc) return rc;
           have_next = true;
         }
       }
     }
     prev_active = active.size();
-    const std::vector<uint32_t> &row_base = blk[cur].row_base;
-    const uint32_t ev_r0 = blk[cur].r0;
+    const std::vector<uint32_t> &row_base = S.blk[S.cur].row_base;
+    const uint32_t ev_r0 = S.blk[S.cur].r0;
     auto fill = [&](StepEntries &en, size_t first, uint32_t count) {
       en.feat_row.resize(count);
       for (uint32_t i = 0; i < count; ++i) en.feat_row[i] = row_base[active[first + i]] + (round - ev_r0);
     };
     RoundOut rout;
     rout.ids = &active;
-    rout.info = &info;
-    rc = run_round(ctx, sp, active, none, SRC_CACHED, prm, fill, &rout);
+    rout.info = &S.info;
+    rc = run_round(ctx, S.sp, active, none, SRC_CACHED, S.prm, fill, &rout);
     if (rc) return rc;
-    ctx->stats.samples += (uint64_t)active.size() * kChunk;
     std::vector<uint32_t> next;
     next.reserve(active.size());
-    for (size_t i = 0; i < active.size(); ++i) {
-      const uint32_t r = active[i];
-      const uint32_t done_chunks = round + 1 - t_admit[r];
-      chunks_used[r] = done_chunks;
-      const bool more = done_chunks < n_chunks[r] && done_chunks < (uint32_t)prm.max_num_chunks;
-      if (done_chunks == 1) {
-        ++first_active;
-        if (!info[i].stop && more) ++after_first;
-      }
-      if (!info[i].stop && more) next.push_back(r);
-    }
+    S.end_tick(active, next);
     active.swap(next);
-    ++round;
   }
+  return SMB_OK;
+}
+
+// Wave-pipelined ticks.  Every tick maps the reads of ONE event block (one tick deep); while it is
+// being mapped, the block of the next tick is computed on the event stream for the reads that are
+// known by then: the survivors of the PREVIOUS tick (they wait one tick, carried forward as absent
+// slots) and the reads whose slices have arrived since -- at most one step's worth.  So neither K1
+// nor event detection is ever waited for after the first wave, however the reads arrive.  A read's
+// chunk at tick T is T - t_admit[r]; t_admit is (re)set whenever the read is put into a block, which
+// is all that "waiting a tick" takes.
+static int run_waves(Sched &S) {
+  smb_ctx *ctx = S.ctx;
+  std::vector<uint32_t> done_chunks(S.R, 0), members[2], waiting, absent;
+  auto want_reads = [&]() -> size_t {
+    const uint64_t by_anchors = (uint64_t)(0.6 * (double)ctx->max_batch_anchors / std::max(ctx->est_anchors_per_chunk, 1.0));
+    return (size_t)std::max<uint64_t>(1, std::min<uint64_t>(by_anchors, ctx->max_batch_chunks));
+  };
+  // reads of the slices that have arrived, in order, until `cap` have joined; wait: block until at
+  // least `min_new` have joined or no slice is left
+  auto join = [&](std::vector<uint32_t> &into, size_t min_new, size_t cap, bool wait) -> int {
+    const size_t n0 = into.size();
+    for (bool took = true; took && into.size() - n0 < cap;) {
+      const int rc = S.take_slice(wait && into.size() - n0 < min_new, into, &took);
+      if (rc) return rc;
+    }
+    return SMB_OK;
+  };
+  auto launch_for = [&](int c, uint32_t tick) -> int {
+    for (uint32_t r : members[c]) S.t_admit[r] = tick - done_chunks[r];
+    return S.launch_block(c, tick, 1, members[c]);
+  };
+  int c = 0, rc;
+  bool have_blk = false;  // blk[c] has been launched for tick `round` with members[c]
+  for (;;) {
+    if (!have_blk) {
+      // nothing was prefetched for this tick: whoever is waiting, plus new reads (a batch, or
+      // what is left of the input)
+      members[c].swap(waiting);
+      waiting.clear();
+      const size_t want = want_reads();
+      if (members[c].size() < want && S.plan.pending()) {
+        const size_t room = want - members[c].size();
+        rc = join(members[c], (room + 1) / 2, room, true);
+        if (rc) return rc;
+      }
+      if (members[c].empty()) {
+        if (!S.plan.pending()) break;
+        continue;  // slices without a single whole chunk
+      }
+      rc = launch_for(c, S.round);
+      if (rc) return rc;
+    }
+    rc = S.consume_block(c);
+    if (rc) return rc;
+    have_blk = false;
+    const std::vector<uint32_t> &act = members[c];
+    // the next tick's block while this one is mapped
+    absent.clear();
+    for (uint32_t r : waiting)
+      if (S.sp.h_nchains[r] > 0) absent.push_back(r);
+    if (ctx->ev_overlap) {
+      std::vector<uint32_t> &nx = members[1 - c];
+      nx.swap(waiting);
+      waiting.clear();
+      const size_t want = want_reads();
+      if (nx.size() < want && S.plan.pending()) {
+        rc = join(nx, 0, want - nx.size(), false);
+        if (rc) return rc;
+      }
+      if (!nx.empty()) {
+        rc = launch_for(1 - c, S.round + 1);
+        if (rc) return rc;
+        have_blk = true;
+      }
+    }
+    const std::vector<uint32_t> &row_base = S.blk[c].row_base;
+    auto fill = [&](StepEntries &en, size_t first, uint32_t count) {
+      en.feat_row.resize(count);
+      for (uint32_t i = 0; i < count; ++i) en.feat_row[i] = row_base[act[first + i]];
+    };
+    RoundOut rout;
+    rout.ids = &act;
+    rout.info = &S.info;
+    rc = run_round(ctx, S.sp, act, absent, SRC_CACHED, S.prm, fill, &rout);
+    if (rc) return rc;
+    S.end_tick(act, waiting);
+    for (uint32_t r : waiting) done_chunks[r] = S.chunks_used[r];
+    if (have_blk) c = 1 - c;
+  }
+  return SMB_OK;
+}
+
+// what every mapping entry point checks before it does any work
+static int map_check(smb_ctx *ctx, const smb_params *prm) {
+  if (!ctx->has_index) return fail(ctx, SMB_ERR_STATE, "no index loaded");
+  if (prm->step_size < 1) return fail(ctx, SMB_ERR_ARG, "step_size must be >= 1");
+  return SMB_OK;
+}
+
+// Maps the read set (ctx->n_reads reads, their samples where `src` says): every mapping entry
+// point ends here, after map_check.
+static int map_read_set(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out, const ReadSource &src) {
+  CK(cudaSetDevice(ctx->device));
+  const smb_params prm = *prm_in;
+  const size_t R = ctx->n_reads;
+  // Wave-pipelined ticks when the stop rules retire most reads after their first chunk (known from
+  // the previous call; a fresh context starts this way): K1 and the events of the next wave run
+  // while the current one is being mapped (option pipeline=on: also with resident samples, which
+  // then join in waves of filter-only slices).  Contig shards must run identical ticks on every
+  // rank: no timing-dependent admission there.
+  // auto: only when the samples arrive from the host during the call.  With resident samples the
+  // GPU is busy mapping from the first tick on and the overlap only adds contention and steps
+  // (measured on config 3: 437 ms pipelined against 403 ms; with host buffers on two GPUs e2e
+  // 1.65 against 1.58 G samples/s).
+  const bool sharded_index = ctx->ex && ctx->index.sharded;
+  const bool pipeline = !sharded_index && R > 0 && prm.max_num_chunks > 0 &&
+                        (ctx->pipeline_mode == 1 ||
+                         (ctx->pipeline_mode == 0 && src.host && ctx->ev_survival_hint <= 0.5));
+  Sched S(ctx, ctx->map_slots, prm);
+  int rc = slots_init(ctx, S.sp, (uint32_t)R);
+  if (rc) return rc;
+  // Slices still queued when the mapping starts (host input, or wave-pipelined): frees wait for
+  // the end of the mapping.  The one slice of any other call is waited for before the first tick.
+  const bool sliced = src.host || pipeline;
+  std::optional<DeferFrees> defer;
+  if (sliced) defer.emplace();
+  rc = plan_slices(ctx, src, sliced ? ctx->upload_slice_bytes / sizeof(int16_t) : 0, S.plan);
+  if (rc) return rc;
+  ctx->h_kept_len.resize(R);
+  rc = pipeline ? run_waves(S) : run_blocks(S);
+  if (rc) return rc;
   // a block launched for ticks that never came (every read stopped) must not outlive the call
-  if (blk[0].ready || blk[1].ready) CK(cudaStreamSynchronize(ctx->stream_ev));
-  if (first_active) ctx->ev_survival_hint = (double)after_first / (double)first_active;
+  if (S.blk[0].ready || S.blk[1].ready) CK(cudaStreamSynchronize(ctx->stream_ev));
+  if (S.first_active) ctx->ev_survival_hint = (double)S.after_first / (double)S.first_active;
+  if (!src.host && R) {
+    rc = add_filter_time(ctx);
+    if (rc) return rc;
+  }
   // final rows
   std::vector<SlotState> st(std::max<size_t>(R, 1));
   if (R) {
-    CK(cudaMemcpyAsync(st.data(), sp.slots.p, R * sizeof(SlotState), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(st.data(), S.sp.slots.p, R * sizeof(SlotState), cudaMemcpyDeviceToHost, ctx->stream));
     rc = host_sync(ctx);
     if (rc) return rc;
     ctx->stats.d2h_bytes += R * sizeof(SlotState);
     rc = merge_owner_tags(ctx, st, R);
     if (rc) return rc;
   }
-  for (size_t r = 0; r < R; ++r) make_row(ctx, st[r], ctx->h_kept_len[r], chunks_used[r], &out[r]);
+  for (size_t r = 0; r < R; ++r) make_row(ctx, st[r], ctx->h_kept_len[r], S.chunks_used[r], &out[r]);
   return SMB_OK;
 }
 
-extern "C" {
-
-int smb_map_reads(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off, const float *dig,
-                  const float *range, const float *offset, size_t n_reads, const smb_params *params,
-                  smb_mapping *out) {
-  CK(cudaSetDevice(ctx->device));
-  cudaStream_t cs = ctx->stream_cp;
-  // the small per-read tables first, then the samples in slices of ~64 MB on the copy stream:
-  // copy -> K1 filter of the slice's reads -> kept lengths to the host -> event.  The mapping loop
-  // admits a slice's reads once its event has fired, so the rest of the upload hides behind the
-  // mapping of the reads that are already there (raw should be pinned host memory for that).
-  int rc = reads_prepare_host(ctx, read_off, dig, range, offset, n_reads, cs);
-  DeferFrees defer_frees;
-  UploadPlan plan;
-  const ReadSource src = uploaded_source(ctx);
-  if (!rc && n_reads) {
-    const uint64_t slice_samples = ctx->upload_slice_bytes / sizeof(int16_t);
-    size_t r0 = 0;
-    while (r0 < n_reads && !rc) {
-      size_t r1 = r0 + 1;
-      while (r1 < n_reads && read_off[r1 + 1] - read_off[r0] <= slice_samples) ++r1;
-      cudaEvent_t done_ev;
-      rc = slice_event(ctx, plan.done.size(), &done_ev);
-      if (rc) break;
-      const uint64_t a = read_off[r0], b = read_off[r1];
-      cudaError_t ce = cudaMemcpyAsync(ctx->raw.p + a, raw + a, (b - a) * sizeof(int16_t), cudaMemcpyHostToDevice, cs);
-      if (ce != cudaSuccess) {
-        rc = fail(ctx, SMB_ERR_CUDA, std::string("upload slice: ") + cudaGetErrorString(ce));
-        break;
-      }
-      ctx->stats.h2d_bytes += (b - a) * 2;
-      rc = filter_slice(ctx, src, r0, r1, cs);
-      if (rc) break;
-      cudaEventRecord(done_ev, cs);
-      plan.first_read.push_back(r0);
-      plan.done.push_back(done_ev);
-      r0 = r1;
-    }
-    plan.first_read.push_back(n_reads);
-  }
-  if (!rc) rc = map_uploaded_impl(ctx, params, out, n_reads ? &plan : nullptr, src);
-  cudaStreamSynchronize(cs);  // nothing of this call may still be in flight when it returns (or when buffers are freed)
+// The end of every mapping call: nothing of it stays queued on the copy stream.  Nothing of a
+// failed call stays queued on the other two streams either (the caller of smb_map_reads_device may
+// free raw once the call returns), and a failed member must not leave its in-process peers waiting
+// at a rendezvous.
+static int map_done(smb_ctx *ctx, int rc) {
+  cudaStreamSynchronize(ctx->stream_cp);
   if (rc) {
-    // a failed member must not leave its in-process peers waiting at a rendezvous
+    cudaStreamSynchronize(ctx->stream);
+    cudaStreamSynchronize(ctx->stream_ev);
     if (ctx->local_group) ctx->local_group->abort_all();
   }
   return rc;
 }
-
-}  // extern "C"
 
 // raw must be device (or managed) memory of this context's device
 static int check_device_input(smb_ctx *ctx, const void *raw) {
@@ -1931,6 +1900,8 @@ static int map_device_impl(smb_ctx *ctx, const int16_t *raw, const uint64_t *rea
                            const float *dig, const float *range, const float *offset, size_t n_reads,
                            const smb_params *params, smb_mapping *out, cudaStream_t caller) {
   CK(cudaSetDevice(ctx->device));
+  int rc = map_check(ctx, params);
+  if (rc) return rc;
   // pack: the reads laid end to end (the kept layout); span: K1's start table, then its end table
   std::vector<uint64_t> pack(n_reads + 1, 0), span(2 * n_reads);
   for (size_t r = 0; r < n_reads; ++r) {
@@ -1939,7 +1910,7 @@ static int map_device_impl(smb_ctx *ctx, const int16_t *raw, const uint64_t *rea
     span[n_reads + r] = read_start[r] + read_len[r];
   }
   if (pack[n_reads]) {  // raw is not read when every read is empty
-    const int rc = check_device_input(ctx, raw);
+    rc = check_device_input(ctx, raw);
     if (rc) return rc;
   }
   // the context's streams do not synchronise with the legacy default stream (NULL): it is waited
@@ -1948,34 +1919,55 @@ static int map_device_impl(smb_ctx *ctx, const int16_t *raw, const uint64_t *rea
   CK(cudaEventRecord(ctx->ev_input, caller));
   CK(cudaStreamWaitEvent(s, ctx->ev_input, 0));
   ctx->device_input = true;
-  int rc = reads_prepare(ctx, pack.data(), dig, range, offset, n_reads, s);
+  rc = reads_prepare(ctx, pack.data(), dig, range, offset, n_reads, s);
   if (rc) return rc;
   if (n_reads) {
     CK(ctx->d_read_off.ensure(2 * n_reads));
     CK(cudaMemcpyAsync(ctx->d_read_off.p, span.data(), 2 * n_reads * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
     ctx->stats.h2d_bytes += n_reads * 16;
-    // K1 also runs on the copy stream when option pipeline=on cuts the reads into filter-only slices
+    // K1 runs on the copy stream, after the tables
     CK(cudaEventRecord(ctx->ev_input, s));
     CK(cudaStreamWaitEvent(ctx->stream_cp, ctx->ev_input, 0));
   }
-  return map_uploaded_impl(ctx, params, out, nullptr, {raw, ctx->d_read_off.p, ctx->d_read_off.p + n_reads});
+  return map_read_set(ctx, params, out, {raw, ctx->d_read_off.p, ctx->d_read_off.p + n_reads});
 }
 
 extern "C" {
 
+int smb_map_uploaded(smb_ctx *ctx, const smb_params *prm_in, smb_mapping *out) {
+  if (ctx->device_input)
+    return fail(ctx, SMB_ERR_STATE, "no uploaded reads: the last read set was mapped from device memory "
+                                    "(smb_map_reads_device); upload one with smb_reads_upload or smb_map_reads");
+  const int rc = map_check(ctx, prm_in);
+  if (rc) return rc;
+  return map_done(ctx, map_read_set(ctx, prm_in, out, uploaded_source(ctx)));
+}
+
+int smb_map_reads(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_off, const float *dig,
+                  const float *range, const float *offset, size_t n_reads, const smb_params *params,
+                  smb_mapping *out) {
+  CK(cudaSetDevice(ctx->device));
+  // the small per-read tables first, then the samples in slices of ~64 MB on the copy stream:
+  // copy -> K1 filter of the slice's reads -> kept lengths to the host -> event.  The mapping loop
+  // admits a slice's reads once its event has fired, so the rest of the upload hides behind the
+  // mapping of the reads that are already there (raw should be pinned host memory for that).
+  int rc = map_check(ctx, params);
+  if (rc) return rc;
+  rc = reads_prepare_host(ctx, read_off, dig, range, offset, n_reads, ctx->stream_cp);
+  if (!rc) {
+    ReadSource src = uploaded_source(ctx);
+    src.host = raw;
+    src.host_off = read_off;
+    rc = map_read_set(ctx, params, out, src);
+  }
+  return map_done(ctx, rc);
+}
+
 int smb_map_reads_device(smb_ctx *ctx, const int16_t *raw, const uint64_t *read_start, const uint32_t *read_len,
                          const float *digitisation, const float *range, const float *offset, size_t n_reads,
                          const smb_params *params, smb_mapping *out, void *stream) {
-  const int rc = map_device_impl(ctx, raw, read_start, read_len, digitisation, range, offset, n_reads, params, out,
-                                 (cudaStream_t)stream);
-  if (rc) {
-    // the caller may free raw once the call returns: no K1 of a failed call may still be queued
-    cudaStreamSynchronize(ctx->stream);
-    cudaStreamSynchronize(ctx->stream_cp);
-    // a failed member must not leave its in-process peers waiting at a rendezvous
-    if (ctx->local_group) ctx->local_group->abort_all();
-  }
-  return rc;
+  return map_done(ctx, map_device_impl(ctx, raw, read_start, read_len, digitisation, range, offset, n_reads,
+                                       params, out, (cudaStream_t)stream));
 }
 
 // ------------------------------------------------------------- stage hooks
@@ -1985,9 +1977,14 @@ int smb_stage_raw_to_pa(smb_ctx *ctx, const int16_t *raw, size_t n, float dig, f
   uint64_t off[2] = {0, n};
   int rc = smb_reads_upload(ctx, raw, off, &dig, &range, &offset, 1);
   if (rc) return rc;
-  rc = filter_reads(ctx, uploaded_source(ctx));
+  UploadPlan plan;  // K1 in one slice
+  rc = plan_slices(ctx, uploaded_source(ctx), 0, plan);
   if (rc) return rc;
-  const uint32_t kept = ctx->h_kept_len[0];
+  ctx->stats.sync_points++;
+  CK(cudaEventSynchronize(plan.done[0]));
+  rc = add_filter_time(ctx);
+  if (rc) return rc;
+  const uint32_t kept = ctx->h_kept_pinned.p[0];
   *n_out = kept;
   if (!kept) return SMB_OK;
   DevBuf<float> d;

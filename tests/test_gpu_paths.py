@@ -76,14 +76,25 @@ def test_every_shipped_path_gives_the_default_rows(mapper, small):
     assert _lines(mapper, small) == base["default"]
 
 
+def _device_input(reads):
+    """a CUDA tensor of the reads' samples and the per-read tables Mapper.map_device takes"""
+    import torch
+    off = reads.read_off
+    raw = torch.from_numpy(reads.raw).to("cuda:0")
+    return raw, off[:-1].copy(), np.diff(off).astype(np.uint32)
+
+
 def test_wave_pipelined_ticks_give_identical_rows(mapper, small):
     """Reads joining in waves (1 MB slices, seven reads per tick: survivors wait a tick and are carried
     forward as absent slots while the next wave's events run) give the rows of the one-batch run, with
-    host buffers and with resident samples, default and full-read rules, with and without event overlap."""
+    host buffers, with resident samples and with device input (filter-only slices over a CUDA tensor),
+    default and full-read rules, with and without event overlap."""
     from sigmap_b200.mapper import full_read_params
     modes = (("default", None), ("full", full_read_params()))
     base = {mode: _lines(mapper, small, prm) for mode, prm in modes}
     names = small.ref.names
+    reads = small.reads
+    raw, start, length = _device_input(reads)
     try:
         mapper.set_option("upload_slice_mb", "1")
         mapper.set_limits(max_batch_chunks=7)
@@ -99,12 +110,57 @@ def test_wave_pipelined_ticks_give_identical_rows(mapper, small):
                 rows = mapper.map_uploaded(prm)
                 got = [paf_cols(l) for l in mapper.paf_lines(small.reads, rows, names)]
                 assert got == base[mode], f"pipeline={pipe} overlap={overlap} {mode}: resident samples"
+                rows = mapper.map_device(raw, start, length, reads.digitisation, reads.range, reads.offset, prm)
+                got = [paf_cols(l) for l in mapper.paf_lines(reads, rows, names)]
+                assert got == base[mode], f"pipeline={pipe} overlap={overlap} {mode}: device input"
     finally:
         mapper.set_option("pipeline", "auto")
         mapper.set_option("events_overlap", "1")
         mapper.set_option("upload_slice_mb", "64")
         mapper.set_limits(max_batch_chunks=32768)
     assert _lines(mapper, small) == base["default"]
+
+
+def test_failed_mapping_call_leaves_the_context_usable(mapper, small):
+    """A call of each entry point that fails mid-call (an anchor limit that one chunk overflows), with
+    and without wave-pipelined ticks, reports the error; the next call on the same context, with a
+    working limit, returns the rows of the default run."""
+    from sigmap_b200.mapper import Mapper, SigmapError
+    base = _lines(mapper, small)
+    reads, names = small.reads, small.ref.names
+    raw, start, length = _device_input(reads)
+
+    # a mapper of its own: a failed call inflates the context's anchor estimate, so the working
+    # limit is a moderate one (the default would size buffers for that estimate).  1 MB slices and
+    # seven reads per tick: calls in several slices, which may still be queued when a call fails.
+    m = Mapper(0)
+
+    def host():
+        return m.map_reads(reads)
+
+    def resident():
+        m.upload_reads(reads)
+        return m.map_uploaded()
+
+    def device():
+        return m.map_device(raw, start, length, reads.digitisation, reads.range, reads.offset)
+
+    try:
+        m.set_index(small.pos, small.val)
+        m.set_contigs(small.ref.lengths)
+        m.set_option("upload_slice_mb", "1")
+        m.set_limits(max_batch_chunks=7)
+        for pipe in ("on", "off"):
+            m.set_option("pipeline", pipe)
+            for name, call in (("host", host), ("resident", resident), ("device", device)):
+                m.set_limits(max_batch_anchors=16)
+                with pytest.raises(SigmapError, match="one chunk overflows max_batch_anchors"):
+                    call()
+                m.set_limits(max_batch_anchors=1 << 24)
+                got = [paf_cols(l) for l in m.paf_lines(reads, call(), names)]
+                assert got == base, f"pipeline={pipe} {name}: rows after a failed call"
+    finally:
+        m.close()
 
 
 def test_radius_search_paths_agree_with_the_oracle(mapper, port, small):
