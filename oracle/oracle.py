@@ -62,6 +62,22 @@ class Mapping(C.Structure):
                 ("at", C.c_float), ("aq", C.c_float), ("num_events", C.c_uint32)]
 
 
+class ChainCounters(C.Structure):
+    """orc_chain_counters: what the chaining met (sigmap_oracle.h)."""
+    _fields_ = [(n, C.c_uint64) for n in (
+        "max_query_hits", "max_bucket_anchors", "walks_band", "walks_skips", "walks_target_gap", "longest_walk",
+        "deep_link_ranges", "traceback_hit_used", "end_ties", "primary_ties")]
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
+
+    def add(self, other):
+        """fold another read's counters into these (sums; the maxima keep the larger)"""
+        for n, _ in self._fields_:
+            a, b = getattr(self, n), getattr(other, n)
+            setattr(self, n, max(a, b) if n in ("max_query_hits", "max_bucket_anchors", "longest_walk") else a + b)
+
+
 def chains_to_py(n, get_chain, get_anchors):
     out = []
     for i in range(n):
@@ -90,6 +106,8 @@ class Port:
         L.orc_generate_chains.restype = None
         L.orc_generate_chains.argtypes = [u64p, f32p, C.c_size_t, f32p, C.c_size_t, C.c_uint32,
                                           C.c_int, C.c_float, C.c_size_t, C.POINTER(ChainList)]
+        L.orc_generate_chains_counted.restype = None
+        L.orc_generate_chains_counted.argtypes = L.orc_generate_chains.argtypes + [C.POINTER(ChainCounters)]
         L.orc_chain_from_hits.restype = None
         L.orc_chain_from_hits.argtypes = [u64p, u32p, C.c_size_t, u64p, u64p, f32p, C.c_float,
                                           C.c_size_t, C.POINTER(ChainList)]
@@ -98,6 +116,8 @@ class Port:
         L.orc_streaming_map.restype = None
         L.orc_streaming_map.argtypes = [u64p, f32p, C.c_size_t, C.c_size_t, u32p, f32p, C.c_size_t,
                                         C.POINTER(Params), C.POINTER(Mapping)]
+        L.orc_streaming_map_counted.restype = None
+        L.orc_streaming_map_counted.argtypes = L.orc_streaming_map.argtypes + [C.POINTER(ChainCounters)]
         L.orc_format_paf.restype = C.c_int
         L.orc_format_paf.argtypes = [C.POINTER(Mapping), C.c_char_p, C.c_char_p, C.c_uint32,
                                      C.c_double, C.c_char_p, C.c_size_t]
@@ -148,13 +168,15 @@ class Port:
         return ChainList(None, 0, 0)
 
     def generate_chains(self, pos, vals, features, query_offset, chain_list, step=2, radius=0.08,
-                        n_targets=1):
+                        n_targets=1, counters=None):
+        """`counters`: a ChainCounters to add this chunk's counts to"""
         pos = np.ascontiguousarray(pos, np.uint64)
         vals = np.ascontiguousarray(vals, np.float32)
         features = np.ascontiguousarray(features, np.float32)
-        self.lib.orc_generate_chains(_p(pos, u64p), _p(vals, f32p), len(pos), _p(features, f32p),
-                                     len(features), query_offset, step, radius, n_targets,
-                                     C.byref(chain_list))
+        self.lib.orc_generate_chains_counted(_p(pos, u64p), _p(vals, f32p), len(pos),
+                                             _p(features, f32p), len(features), query_offset, step,
+                                             radius, n_targets, C.byref(chain_list),
+                                             None if counters is None else C.byref(counters))
         return self.chains_py(chain_list)
 
     def chain_from_hits(self, pos, query_pos, hit_off, hit_idx, hit_d2, chain_list, radius=0.08,
@@ -183,16 +205,17 @@ class Port:
     def free_chain_list(self, cl):
         self.lib.orc_chain_list_free(C.byref(cl))
 
-    def streaming_map(self, pos, vals, n_targets, contig_len, pa, params=None):
+    def streaming_map(self, pos, vals, n_targets, contig_len, pa, params=None, counters=None):
+        """`counters`: a ChainCounters to add the read's counts to"""
         pos = np.ascontiguousarray(pos, np.uint64)
         vals = np.ascontiguousarray(vals, np.float32)
         contig_len = np.ascontiguousarray(contig_len, np.uint32)
         pa = np.ascontiguousarray(pa, np.float32)
         p = params or self.default_params()
         m = Mapping()
-        self.lib.orc_streaming_map(_p(pos, u64p), _p(vals, f32p), len(pos), n_targets,
-                                   _p(contig_len, u32p), _p(pa, f32p), len(pa), C.byref(p),
-                                   C.byref(m))
+        self.lib.orc_streaming_map_counted(_p(pos, u64p), _p(vals, f32p), len(pos), n_targets,
+                                           _p(contig_len, u32p), _p(pa, f32p), len(pa), C.byref(p),
+                                           C.byref(m), None if counters is None else C.byref(counters))
         return m
 
     def format_paf(self, m, read_name, contig_name, contig_len, mt_ms=0.0):

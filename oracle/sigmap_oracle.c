@@ -305,7 +305,7 @@ static int chain_greater(const orc_chain *a, const orc_chain *b) {
 /* spatial_index.cc:165-220 */
 static void traceback(uint32_t dir, size_t end_i, uint32_t contig, const float *score,
                       const size_t *pred, const orc_anchor *A, unsigned char *used,
-                      orc_chain_list *out) {
+                      orc_chain_list *out, orc_chain_counters *ctr) {
   if (used[end_i]) return;
   size_t cap = 128, n = 0;
   orc_anchor *list = (orc_anchor *)malloc(cap * sizeof(orc_anchor));
@@ -326,7 +326,10 @@ static void traceback(uint32_t dir, size_t end_i, uint32_t contig, const float *
   }
   if (n >= 2) { /* min_num_anchors = 2, spatial_index.cc:288 */
     float sc = score[end_i];
-    if (hit_used) sc -= score[pred[s]];
+    if (hit_used) {
+      sc -= score[pred[s]];
+      if (ctr) ctr->traceback_hit_used++;
+    }
     orc_chain c;
     c.score = sc;
     c.contig = contig;
@@ -342,8 +345,27 @@ static void traceback(uint32_t dir, size_t end_i, uint32_t contig, const float *
   }
 }
 
-/* spatial_index.cc:411-576 given filled buckets [strand][contig] */
-static void chain_buckets(bucket *bk[2], size_t n_targets, float radius, orc_chain_list *chains) {
+/* Counters only: the position-only lookback range of anchor i (the range the CUDA chain
+ * preparation tests for a gap-compatible predecessor): 1 when it holds more than 1 152
+ * predecessors and none of them is gap-compatible. */
+static int deep_link_range(const orc_anchor *A, size_t i, int band, int max_target_gap,
+                           int max_gap, uint32_t qmin) {
+  int32_t ct = (int32_t)A[i].target, cq = (int32_t)A[i].query;
+  int64_t qlim = 4 * ((int64_t)cq - (int64_t)qmin);
+  size_t depth = i < (size_t)band ? i : (size_t)band, d;
+  for (d = 1; d <= depth; ++d) {
+    int32_t pt = (int32_t)A[i - d].target, pq = (int32_t)A[i - d].query;
+    if (pt + max_target_gap < ct || 3 * (int64_t)(ct - pt) >= qlim) break;
+    int32_t dt = ct - pt, dq = cq - pq;
+    if (abs(dt - dq) < max_gap && dq < 5 * dt && 4 * dq > 3 * dt) return 0;
+  }
+  return d - 1 > 1152;
+}
+
+/* spatial_index.cc:411-576 given filled buckets [strand][contig]; query_offset is the
+ * chunk's first query position (for the counters only) */
+static void chain_buckets(bucket *bk[2], size_t n_targets, float radius, uint32_t query_offset,
+                          orc_chain_list *chains, orc_chain_counters *ctr) {
   const int max_gap_length = 2000, max_target_gap_length = 5000, band = 5000, max_skips = 25;
   const int num_best = 3;
   const float min_score = 10;
@@ -356,6 +378,12 @@ static void chain_buckets(bucket *bk[2], size_t n_targets, float radius, orc_cha
       const orc_anchor *A = bk[s][t].a;
       size_t n = bk[s][t].n;
       if (n == 0) continue; /* nothing observable happens for an empty bucket */
+      uint32_t qmin = query_offset;
+      if (ctr) {
+        if (n > ctr->max_bucket_anchors) ctr->max_bucket_anchors = n;
+        for (size_t i = 0; i < n; ++i)
+          if (A[i].query < qmin) qmin = A[i].query;
+      }
       float *score = (float *)malloc(n * sizeof(float));
       size_t *pred = (size_t *)malloc(n * sizeof(size_t));
       unsigned char *used = (unsigned char *)calloc(n, 1);
@@ -370,12 +398,16 @@ static void chain_buckets(bucket *bk[2], size_t n_targets, float radius, orc_cha
         int32_t ct = (int32_t)A[i].target, cq = (int32_t)A[i].query;
         int32_t start = 0;
         if (i > (size_t)band) start = (int32_t)i - band;
-        int32_t skips = 0;
-        for (int32_t j = (int32_t)i - 1; j >= start; --j) {
+        int32_t skips = 0, j;
+        int stop = 0; /* counters: 1 target gap, 2 skips */
+        for (j = (int32_t)i - 1; j >= start; --j) {
           int32_t pt = (int32_t)A[j].target, pq = (int32_t)A[j].query;
           if (pq == cq) continue;
           if (pt == ct) continue;
-          if (pt + max_target_gap_length < ct) break;
+          if (pt + max_target_gap_length < ct) {
+            stop = 1;
+            break;
+          }
           int32_t dt = ct - pt, dq = cq - pq;
           float cur = 0;
           if (dq < 0) continue;
@@ -391,8 +423,20 @@ static void chain_buckets(bucket *bk[2], size_t n_targets, float radius, orc_cha
             --skips;
           } else {
             ++skips;
-            if (skips > max_skips) break;
+            if (skips > max_skips) {
+              stop = 2;
+              break;
+            }
           }
+        }
+        if (ctr) {
+          uint64_t walked = (uint64_t)((int32_t)i - j - (stop ? 0 : 1));
+          if (walked > ctr->longest_walk) ctr->longest_walk = walked;
+          if (stop == 1) ctr->walks_target_gap++;
+          if (stop == 2) ctr->walks_skips++;
+          if (stop == 0 && start > 0) ctr->walks_band++;
+          ctr->deep_link_ranges +=
+              deep_link_range(A, i, band, max_target_gap_length, max_gap_length, qmin);
         }
         if (score[i] > gmax) gmax = score[i];
         if (score[i] >= min_score && score[i] > gmax / 2) {
@@ -416,8 +460,14 @@ static void chain_buckets(bucket *bk[2], size_t n_targets, float radius, orc_cha
             best = e;
         }
         taken[best] = 1;
+        if (ctr)
+          for (size_t e = 0; e < n_ends; ++e)
+            if (!taken[e] && end_score[e] == end_score[best]) {
+              ctr->end_ties++;
+              break;
+            }
         /* direction_i == 0 -> Positive (dir 1) */
-        traceback(s == 0 ? 1u : 0u, end_idx[best], (uint32_t)t, score, pred, A, used, chains);
+        traceback(s == 0 ? 1u : 0u, end_idx[best], (uint32_t)t, score, pred, A, used, chains, ctr);
         if (score[end_idx[best]] < gmax / 2) break;
       }
       free(taken);
@@ -439,6 +489,9 @@ static void chain_buckets(bucket *bk[2], size_t n_targets, float radius, orc_cha
       }
       chains->chains[j] = c;
     }
+    if (ctr)
+      for (size_t i = 1; i < chains->n; ++i)
+        ctr->primary_ties += chains->chains[i].score == chains->chains[i - 1].score;
     size_t np = 1;
     unsigned char *is_primary = (unsigned char *)calloc(chains->n, 1);
     size_t *prim = (size_t *)malloc(chains->n * sizeof(size_t));
@@ -515,6 +568,14 @@ static void emit_hit(bucket *bk[2], uint64_t P, uint32_t qpos, float d2) {
 void orc_generate_chains(const uint64_t *pos, const float *vals, size_t n_points,
                          const float *features, size_t n_features, uint32_t query_offset,
                          int step, float radius, size_t n_targets, orc_chain_list *chains) {
+  orc_generate_chains_counted(pos, vals, n_points, features, n_features, query_offset, step,
+                              radius, n_targets, chains, NULL);
+}
+
+void orc_generate_chains_counted(const uint64_t *pos, const float *vals, size_t n_points,
+                                 const float *features, size_t n_features, uint32_t query_offset,
+                                 int step, float radius, size_t n_targets, orc_chain_list *chains,
+                                 orc_chain_counters *ctr) {
   const size_t num_nearest = 5000;
   bucket *bk[2];
   seed_buckets(bk, n_targets, chains);
@@ -526,6 +587,7 @@ void orc_generate_chains(const uint64_t *pos, const float *vals, size_t n_points
   for (uint32_t p = 0; p < np; ++p) {
     if (p < prev + (uint32_t)step && p + (uint32_t)step > prev) continue;
     size_t nh = orc_radius_search(vals, n_points, features + p, radius, hi, hd, num_nearest);
+    if (ctr && nh > ctr->max_query_hits) ctr->max_query_hits = nh;
     for (size_t a = 0; a < nh && a < num_nearest; ++a)
       emit_hit(bk, pos[hi[a]], p + query_offset, hd[a]);
     ++count;
@@ -534,7 +596,7 @@ void orc_generate_chains(const uint64_t *pos, const float *vals, size_t n_points
   }
   free(hi);
   free(hd);
-  chain_buckets(bk, n_targets, radius, chains);
+  chain_buckets(bk, n_targets, radius, query_offset, chains, ctr);
   free_buckets(bk, n_targets);
 }
 
@@ -548,7 +610,7 @@ void orc_chain_from_hits(const uint64_t *pos, const uint32_t *query_pos, size_t 
     for (uint64_t a = 0; a < n && a < 5000; ++a)
       emit_hit(bk, pos[hit_idx[hit_off[k] + a]], query_pos[k], hit_d2[hit_off[k] + a]);
   }
-  chain_buckets(bk, n_targets, radius, chains);
+  chain_buckets(bk, n_targets, radius, 0, chains, NULL);
   free_buckets(bk, n_targets);
 }
 
@@ -556,6 +618,13 @@ void orc_chain_from_hits(const uint64_t *pos, const uint32_t *query_pos, size_t 
 void orc_streaming_map(const uint64_t *pos, const float *vals, size_t n_points,
                        size_t n_targets, const uint32_t *contig_len, const float *pa,
                        size_t n_pa, const orc_params *p, orc_mapping *out) {
+  orc_streaming_map_counted(pos, vals, n_points, n_targets, contig_len, pa, n_pa, p, out, NULL);
+}
+
+void orc_streaming_map_counted(const uint64_t *pos, const float *vals, size_t n_points,
+                               size_t n_targets, const uint32_t *contig_len, const float *pa,
+                               size_t n_pa, const orc_params *p, orc_mapping *out,
+                               orc_chain_counters *ctr) {
   const uint32_t bp_per_sec = 450, sample_rate = 4000, chunk_size = 4000;
   memset(out, 0, sizeof(*out));
   size_t num_chunks = n_pa / chunk_size;
@@ -565,8 +634,8 @@ void orc_streaming_map(const uint64_t *pos, const float *vals, size_t n_points,
   for (ci = 0; ci < num_chunks && ci < (uint32_t)p->max_num_chunks; ++ci) {
     size_t nf = orc_generate_events(pa + (size_t)chunk_size * ci, chunk_size, feat);
     if (nf > 50) {
-      orc_generate_chains(pos, vals, n_points, feat, nf, num_events, p->step, p->search_radius,
-                          n_targets, &chains);
+      orc_generate_chains_counted(pos, vals, n_points, feat, nf, num_events, p->step,
+                                  p->search_radius, n_targets, &chains, ctr);
       num_events += (uint32_t)nf;
       if (chains.n >= 2) {
         if (chains.chains[0].score / chains.chains[1].score >= p->stop_ratio) break;

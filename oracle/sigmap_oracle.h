@@ -64,6 +64,26 @@ typedef struct {
   uint32_t num_events;        /* kept events consumed (query offset at the end) */
 } orc_mapping;
 
+/* What the chaining of spatial_index.cc:411-576 met, for tests that must show their data
+ * reaches the rare branches of the CUDA chaining.  Filled by the *_counted entry points when
+ * given a non-NULL pointer: counts add up over calls, the maxima keep the largest value. */
+typedef struct {
+  uint64_t max_query_hits;     /* most hits one query found (the reference keeps 5 000: :371-372) */
+  uint64_t max_bucket_anchors; /* largest (contig, strand) bucket of a chunk, carried anchors included */
+  /* the lookback of :434-540 */
+  uint64_t walks_band;         /* lookbacks that ran to start = i - band > 0 */
+  uint64_t walks_skips;        /* lookbacks ended by skips > max_skips */
+  uint64_t walks_target_gap;   /* lookbacks ended by a target gap > 5 000 */
+  uint64_t longest_walk;       /* most predecessors one lookback visited */
+  /* anchors whose position-only lookback range (same bucket, band, target gap, and
+   * 3 dt < 4 (q_i - qmin) with qmin the chunk's query offset lowered by the bucket's carried
+   * anchors) holds more than 1 152 predecessors and no gap-compatible one */
+  uint64_t deep_link_ranges;
+  uint64_t traceback_hit_used; /* chains emitted with score[end] - score[pred] (:165-220) */
+  uint64_t end_ties;           /* top-3 end picks decided by index between equal scores (:552-568) */
+  uint64_t primary_ties;       /* adjacent equal scores after the primary sort (:222-253) */
+} orc_chain_counters;
+
 void orc_default_params(orc_params *p);
 
 /* A.0  signal_batch.cc:182-210 */
@@ -82,6 +102,10 @@ size_t orc_radius_search(const float *vals, size_t n_points, const float *q, flo
 void orc_generate_chains(const uint64_t *pos, const float *vals, size_t n_points,
                          const float *features, size_t n_features, uint32_t query_offset,
                          int step, float radius, size_t n_targets, orc_chain_list *chains);
+void orc_generate_chains_counted(const uint64_t *pos, const float *vals, size_t n_points,
+                                 const float *features, size_t n_features, uint32_t query_offset,
+                                 int step, float radius, size_t n_targets, orc_chain_list *chains,
+                                 orc_chain_counters *ctr);
 /* same but with the hit lists supplied by the caller (per query: first hit index into
  * hit_idx/hit_d2 = hit_off[k], count = hit_off[k+1]-hit_off[k]); lets tests drive A.3
  * with the reference's own KD-tree hit order */
@@ -93,6 +117,10 @@ void orc_chain_list_free(orc_chain_list *l);
 void orc_streaming_map(const uint64_t *pos, const float *vals, size_t n_points,
                        size_t n_targets, const uint32_t *contig_len, const float *pa,
                        size_t n_pa, const orc_params *p, orc_mapping *out);
+void orc_streaming_map_counted(const uint64_t *pos, const float *vals, size_t n_points,
+                               size_t n_targets, const uint32_t *contig_len, const float *pa,
+                               size_t n_pa, const orc_params *p, orc_mapping *out,
+                               orc_chain_counters *ctr);
 /* A.4  output_tools.h:200-210,336-354 + sigmap.cc:731-745 ; mt tag printed as given */
 int orc_format_paf(const orc_mapping *m, const char *read_name, const char *contig_name,
                    uint32_t contig_len, double mt_ms, char *buf, size_t cap);

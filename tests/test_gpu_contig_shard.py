@@ -37,8 +37,20 @@ def row_bytes(rows):
     return [bytes(r) for r in rows]
 
 
+@pytest.fixture(scope="module")
+def repeats(host, model):
+    from repeat_genome import RepeatGenome
+    from sigmap_b200.mapper import Mapper
+    g = RepeatGenome(host, model)
+    m = Mapper(0)
+    m.set_index(g.pos, g.val)
+    m.set_contigs(g.ref.lengths)
+    yield g, m
+    m.close()
+
+
 @pytest.mark.parametrize("world", [2, 3])
-def test_sharded_rows_equal_unsharded(multi, whole, world):
+def test_sharded_rows_equal_unsharded(multi, whole, repeats, world):
     from sigmap_b200 import shard
     from sigmap_b200.mapper import default_params, full_read_params
     g = shard.ContigShardGroup([0] * world)
@@ -60,6 +72,15 @@ def test_sharded_rows_equal_unsharded(multi, whole, world):
         whole.map_reads(multi.reads, default_params())
         g.map_reads(multi.reads, default_params())
         assert sum(m.stats()["hits"] for m in g.mappers) == whole.stats()["hits"]
+        # the repeat genome with B, C and D (exact copies: tied chains) on different ranks, so the
+        # tied candidates meet in the exchange and every rank must pick the unsharded winner
+        rep, rep_whole = repeats
+        owner = [world - 1, 0, 1 % world, 2 % world, 0, 1 % world, 0, world - 1]  # A B C D S t5 t11 t12
+        g.set_index(rep.pos, rep.val, rep.ref.lengths, owner=owner)
+        for prm in (default_params(), full_read_params()):
+            exp = rep_whole.map_reads(rep.reads, prm)
+            for rank_rows in g.map_reads(rep.reads, prm):
+                assert row_bytes(rank_rows) == row_bytes(exp), "repeats"
     finally:
         g.close()
 
